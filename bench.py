@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- OFDM symbols/s through the full Task-5 RX chain (SURVEY 8d, workload M1).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--streams B]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--streams B] [--dump-outputs DIR]
 
 One "step" = one pass of the fused RX chain (OFDM_demodulator -> LS_CE -> equalize_signal ->
 get_payload -> demapping -> DeScrambler -> BER count) over a batch of B synthetic streams of 14 OFDM
@@ -10,6 +10,11 @@ that is already resident in HBM.  `value` is device-timed whole-job throughput; 
 chain through the host-buffer C-ABI entry (pinned host memory, H2D + D2H inside the timed region).
 `--impl reference` times the CPU restatement of the reference (oracle/, NumPy float64 -- MATLAB and
 Octave do not exist on the box) on all host cores.  Prints ONE JSON line on rank 0.
+
+`--dump-outputs DIR` writes, after the timed steps, what the last timed step returned to its caller (rank 0's):
+DIR/bits.npy (decided bits, 0/1), DIR/H.npy (LS channel estimate, real and imaginary parts) and DIR/counts.npy (errors,
+bits, near-boundary decisions of one step).  The inputs are seeded, so two builds run with the same arguments can be
+compared output for output.
 """
 import argparse
 import json
@@ -129,6 +134,25 @@ def load_traffic():
     return None
 
 
+DUMP_STREAMS = 128      # --dump-outputs sample: 128 x 43,008 bits as float32 + 128 x 1,024 complex carriers = 23.1 MB
+
+
+def dump_outputs(out_dir, B, words, out_bits, H, counts, steps):
+    """Write what the last timed step returned: decided bits and channel estimate of a fixed, seeded sample of streams,
+    and one step's counters (every timed step decodes the same input, so the accumulated counters are `steps` times one
+    step's).  Runs after the last timed event, so the copies are not timed."""
+    import torch
+    from ofdm_b200 import unpack_bits
+    idx = np.sort(np.random.default_rng(0).choice(B, min(B, DUMP_STREAMS), replace=False))
+    sel = torch.from_numpy(idx).to(H.device)
+    w = out_bits.view(B, words).index_select(0, sel).cpu().numpy()
+    bits = unpack_bits(w.view(np.uint32), w.size * 32).reshape(len(idx), words * 32).astype(np.float32)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "bits.npy"), bits)
+    np.save(os.path.join(out_dir, "H.npy"), torch.view_as_real(H.index_select(0, sel)).cpu().numpy())
+    np.save(os.path.join(out_dir, "counts.npy"), counts.cpu().numpy().astype(np.float64) / steps)
+
+
 # --------------------------------------------------------------------------------------------
 def run_reference(args, rank, world):
     if rank != 0:
@@ -138,7 +162,7 @@ def run_reference(args, rank, world):
     vals = []
     for _ in range(args.warmup):
         pass  # the oracle has no warm-up state worth timing; keep the run short
-    for _ in range(max(1, min(args.steps, 3))):
+    for _ in range(args.steps):
         v, syms, wall, _ = cpu_baseline(n_proc, per_proc, target_s=args.cpu_seconds)
         vals.append((v, syms, wall))
     v = float(np.median([x[0] for x in vals]))
@@ -261,6 +285,8 @@ def run_gpu(args, rank, world, local_rank):
     for i in range(args.steps):
         step()
         ev[i + 1].record()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, B, words, out_bits, H, counts, args.steps)
     if world > 1:
         dist.all_reduce(counts)             # the chain's only collective: int64 error / bit counters
     barrier()
@@ -435,7 +461,12 @@ def main():
     ap.add_argument("--near-eps", type=float, default=1e-4,
                     help="squared-distance margin below which a decision counts as 'within epsilon of a boundary' (0 = counter off)")
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as DIR/<name>.npy (GPU path)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path; the reference arm has none to write")
     args.warmup = max(args.warmup, 3) if args.impl != "reference" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -2,10 +2,10 @@
 
 `file_reader('eagle.tiff', n)` (`Task 5/file_reader.m:2-12`: imread -> imbinarize -> first n entries, column-major)
 restated by `oracle.chains.read_payload_bits`; 129,600 bits packed MSB-first (numpy.packbits) = 16,200 bytes.  Needs
-/root/reference (authoring container only); the GPU box reads the committed file.  `eagle_bits_digest.json` holds the
-SHA-256 of exactly these bytes.
+the image from a checkout of the reference (it is not copied into this repository); the tests read the committed file.
+`eagle_bits_digest.json` holds the SHA-256 of exactly these bytes.
 
-    python tests/golden/make_eagle_bits.py
+    python tests/golden/make_eagle_bits.py "<reference checkout>/Task 5/eagle.tiff"
 """
 import hashlib
 import json
@@ -19,7 +19,7 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
 from oracle import chains as OC  # noqa: E402
 
 if __name__ == "__main__":
-    b = OC.read_payload_bits("/root/reference/Task 5/eagle.tiff", 129600)
+    b = OC.read_payload_bits(sys.argv[1], 129600)
     raw = np.packbits(b).tobytes()
     want = json.load(open(os.path.join(HERE, "eagle_bits_digest.json")))["sha256_of_packbits"]
     assert hashlib.sha256(raw).hexdigest() == want

@@ -25,6 +25,7 @@ P4  `Task 2/README.md:54`, figure `Task 2/graphs/PAPR1.png`: PAPR 23 dB unscramb
     pin is +-1.5 dB.
 """
 import os
+import struct
 
 import numpy as np
 
@@ -60,6 +61,23 @@ def eagle_bits(n):
     """First n payload bits of `file_reader('eagle.tiff', n)` from the committed golden input vector."""
     raw = np.frombuffer(open(os.path.join(HERE, "golden", "eagle_bits.bin"), "rb").read(), dtype=np.uint8)
     return np.unpackbits(raw)[:n].copy()
+
+
+def write_eagle_tiff(path, side=360):
+    """Write an 8-bit grey-level baseline TIFF (side x side, one uncompressed strip) whose Otsu binarisation, read
+    column-major, is the golden payload.  The reference image is not part of this repository: each pixel's grey level is
+    drawn (seeded) from a dark band for a 0 and a bright band for a 1, so every threshold in the gap between the bands
+    gives back `eagle_bits(side * side)`."""
+    bits = eagle_bits(side * side)
+    rng = np.random.default_rng(360)
+    grey = np.where(bits == 1, rng.integers(150, 256, bits.size), rng.integers(0, 100, bits.size)).astype(np.uint8)
+    data = grey.reshape((side, side), order="F").tobytes()
+    entries = [(256, 4, 1, side), (257, 4, 1, side), (258, 3, 1, 8), (259, 3, 1, 1), (262, 3, 1, 1), (273, 4, 1, 8),
+               (277, 3, 1, 1), (278, 4, 1, side), (279, 4, 1, len(data))]
+    ifd = struct.pack("<H", len(entries)) + b"".join(struct.pack("<HHII", *e) for e in entries) + struct.pack("<I", 0)
+    with open(path, "wb") as fh:
+        fh.write(b"II*\0" + struct.pack("<I", 8 + len(data)) + data + ifd)
+    return str(path)
 
 
 def keys_cubic(x, y, xq):

@@ -257,13 +257,12 @@ def test_equalize_zero_rows_and_ber():
     assert O.BER_func([0, 1, 1, 0], [0, 1, 0, 1]) == 0.5
 
 
-def test_payload_reader_matches_survey_stats():
-    import os
-    path = "/root/reference/Task 5/eagle.tiff"
-    if not os.path.exists(path):
-        pytest.skip("reference fixture only exists in the build container")
+def test_payload_reader_matches_survey_stats(tmp_path):
+    import reference_pins as RP
+    path = RP.write_eagle_tiff(tmp_path / "eagle.tiff")
     bits = C.read_payload_bits(path, 129600)
     assert bits.size == 129600 and abs(bits.mean() - 0.337) < 0.005
+    assert np.array_equal(bits, RP.eagle_bits(129600))
 
 
 @pytest.mark.parametrize("L", [1, 5, 13, 14, 15, 16, 100, 6640])

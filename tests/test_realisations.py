@@ -1,5 +1,5 @@
 """Realisation import/export (SURVEY 8f rank 2): the MAT-file codec against SciPy's (checker only), the committed
-golden realisation against the oracle, and the payload reader against the reference image when it is present."""
+golden realisation against the oracle, and the payload reader against the pinned reference payload."""
 import hashlib
 import json
 import os
@@ -11,8 +11,9 @@ import ofdm_b200  # noqa: F401
 from ofdm_b200 import realisations as R
 from oracle import chains as OC
 
+import reference_pins as RP
+
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
-EAGLE = "/root/reference/Task 5/eagle.tiff"
 
 
 def test_mat5_round_trip_and_scipy_interop(tmp_path):
@@ -97,10 +98,10 @@ def test_payload_reader_and_display_pic(tmp_path):
     assert pic.shape == (12, 12) and pic.dtype == np.uint8 and np.array_equal((pic.ravel(order="F")[:100] // 255), bits) and not pic.ravel(order="F")[100:].any()
 
 
-@pytest.mark.skipif(not os.path.exists(EAGLE), reason="reference image only exists in the authoring container")
-def test_file_reader_on_the_reference_payload():
+def test_file_reader_on_the_reference_payload(tmp_path):
     d = json.load(open(os.path.join(GOLD, "eagle_bits_digest.json")))
-    bits = R.file_reader(EAGLE, d["n_bits"])
+    eagle = RP.write_eagle_tiff(tmp_path / "eagle.tiff")
+    bits = R.file_reader(eagle, d["n_bits"])
     assert int(bits.sum()) == d["n_ones"] and "".join(map(str, bits[:64])) == d["first_64"]
     assert hashlib.sha256(np.packbits(bits).tobytes()).hexdigest() == d["sha256_of_packbits"]
-    assert np.array_equal(bits, OC.read_payload_bits(EAGLE, d["n_bits"]))
+    assert np.array_equal(bits, OC.read_payload_bits(eagle, d["n_bits"]))

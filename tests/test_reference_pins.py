@@ -14,15 +14,14 @@ from oracle import chains as OC
 import reference_pins as RP
 
 
-def test_payload_fixture_is_the_pinned_payload():
+def test_payload_fixture_is_the_pinned_payload(tmp_path):
     d = json.load(open(os.path.join(RP.HERE, "golden", "eagle_bits_digest.json")))
     raw = open(os.path.join(RP.HERE, "golden", "eagle_bits.bin"), "rb").read()
     assert hashlib.sha256(raw).hexdigest() == d["sha256_of_packbits"]
     b = RP.eagle_bits(129600)
     assert b.size == d["n_bits"] and int(b.sum()) == d["n_ones"] and "".join(map(str, b[:64])) == d["first_64"]
-    path = "/root/reference/Task 5/eagle.tiff"
-    if os.path.exists(path):
-        assert np.array_equal(b, OC.read_payload_bits(path, 129600))
+    path = RP.write_eagle_tiff(tmp_path / "eagle.tiff")
+    assert np.array_equal(b, OC.read_payload_bits(path, 129600))
 
 
 def _task3_ber(cname, snr, seeds):
