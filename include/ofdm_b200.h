@@ -313,7 +313,8 @@ OFDM_API int ofdm_rx_chain_t4_ex(ofdm_ctx*, const ofdm_link_params*, const void*
 
 /* ---- Monte-Carlo BER-vs-SNR sweep (the script loops) ------------------------------------------ */
 /* Replaces the SNR loops `Task 3/Main_model_Task_3.m:192-268` / `Task 5/Main_model_Task_5.m:303-346` (chain
- * OFDM_SWEEP_TASK5: TX chain -> Noise -> multipath -> M1 RX chain) and the impaired channel of
+ * OFDM_SWEEP_TASK5: TX chain -> Noise -> multipath -> M1 RX chain; the BER half of the Task-5 loop, ofdm_sweep_mse below
+ * runs its channel-estimation half) and the impaired channel of
  * `Task 4/Main_model_Task_4.m:95-110,252-264,277-366` swept over SNR (chain OFDM_SWEEP_TASK4: TX chain -> Noise ->
  * add_STO -> add_CFO -> multipath -> M2 RX chain with AutoCorrFunction / remove_IFO / fine_sync / estimate_channel).
  * Streams are numbered globally, g = snr_index * streams_per_point + j; payload bits, noise, STO and CFO draws are
@@ -341,6 +342,19 @@ typedef struct ofdm_sweep_params {
     int32_t cfo_int_max;         /* Task-4 chain: Freq_Shift = U{0..cfo_int_max} + U(-0.5, 0.5) (`:108`: 30) */
 } ofdm_sweep_params;
 OFDM_API int ofdm_sweep_ber(ofdm_ctx*, const ofdm_link_params*, const ofdm_sweep_params*, int64_t* counts_dev);
+/* Task-5 channel-estimation study over SNR (`Task 5/Main_model_Task_5.m:303-346`, MSE as `:195-205`): per stream Noise ->
+ * multipath -> OFDM_demodulator -> LS_CE / MMSE_CE (h = ifft(H_LS), `:179`) / MP_estimate / OMP_estimate on the partial-DFT
+ * dictionary of Ldict columns (`:182-190`, Ldict >= Np), and (H - Hest)(H - Hest)'/N_carrier against the true response
+ * fft(h, Nfft)(1:N_carrier).  Uses chain (must be OFDM_SWEEP_TASK5), n_snr, snr_db_host, streams_per_point, tile_streams,
+ * rank, world, seed, taps_host / n_taps (required, n_taps <= 32; K = n_taps dominant taps) and near_eps (OMP's tie_eps);
+ * sto_max and cfo_int_max are ignored.  Share rule and stream numbering are those of ofdm_sweep_ber.  Nd == 0 transmits the
+ * pilot-only stream (`:24-33`, the same for every g); Nd >= 1 the stream ofdm_sweep_ber transmits for g.  N_carrier must
+ * be a power of two and the pilots lie in 1..N_carrier.
+ * mse_dev: n_snr x 4 x streams_per_point doubles, [i][e][j] with e = LS, MMSE, MP, OMP; only this call's share is written.
+ * counts_dev: n_snr x 2 int64 += {streams processed, OMP frames with a near-tie}.  The per-stream values do not depend on
+ * the rank count or the tile size; the caller sums the arrays of all ranks (each cell is written by one rank). */
+OFDM_API int ofdm_sweep_mse(ofdm_ctx*, const ofdm_link_params*, const ofdm_sweep_params*, int Ldict, double* mse_dev,
+                            int64_t* counts_dev);
 /* first / count of the contiguous share of `total_streams` that (rank, world) processes */
 OFDM_API int ofdm_sweep_share(int64_t total_streams, int rank, int world, int64_t* first, int64_t* count);
 /* The sweep's synthetic inputs, also usable on their own: payload words of streams first_stream_id .. +n_streams-1

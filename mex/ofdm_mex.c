@@ -642,6 +642,57 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
         mxArray* cm = mxCreateDoubleMatrix(n, 4, mxREAL);
         for (i = 0; i < n; ++i) { int j; for (j = 0; j < 4; ++j) real_data(cm)[(size_t)j * n + i] = (double)ch[4 * i + j]; }
         OUT(0, cm);
+    } else if (!strcmp(op, "sweep_mse")) {   /* [MSE (n_snr x 4), per_stream (spp x 4*n_snr), counts (n_snr x 2)] =
+                                                 sweep_mse(LINK..., snrs, streams_per_point, taps (K x 2), seed, tie_eps [, Ldict]);
+                                                 dataCarriers may be [] (the pilot-only comb-1 layout) */
+        NEED(N_LINK + 5);
+        ofdm_link_params lp;
+        ofdm_sweep_params sp;
+        parse_link(&A(0), &lp);
+        memset(&sp, 0, sizeof sp);
+        size_t n = mxGetNumberOfElements(A(N_LINK)), i;
+        int K = (int)mxGetM(A(N_LINK + 2)), k2, e;
+        if (!n) fail("ofdm:sweep_mse:snr", "need at least one SNR point");
+        if (!K || mxGetN(A(N_LINK + 2)) != 2) fail("ofdm:sweep_mse:taps", "channel_taps must be K x 2 (delay, amplitude)");
+        if (lp.Np < 2) fail("ofdm:sweep_mse:pilots", "need at least two pilots");
+        sp.chain = OFDM_SWEEP_TASK5;
+        sp.n_snr = (int32_t)n;
+        sp.snr_db_host = real_data(A(N_LINK));
+        sp.streams_per_point = (int64_t)mxGetScalar(A(N_LINK + 1));
+        sp.rank = 0; sp.world = 1;
+        sp.seed = (uint64_t)mxGetScalar(A(N_LINK + 3));
+        sp.near_eps = mxGetScalar(A(N_LINK + 4));
+        double* tp = real_data(A(N_LINK + 2));
+        double* taps = (double*)hostbuf((size_t)K * 16);
+        for (k2 = 0; k2 < K; ++k2) { taps[2 * k2] = tp[k2]; taps[2 * k2 + 1] = tp[K + k2]; }
+        sp.taps_host = taps; sp.n_taps = K;
+        /* Ldict: the script's ceil(N_carrier / comb) (`Main_model_Task_5.m:182-190`) unless given */
+        int comb = lp.pilot_carriers_host[1] - lp.pilot_carriers_host[0];
+        int Ldict = nrhs > N_LINK + 6 ? (int)mxGetScalar(A(N_LINK + 5)) : (comb > 0 ? (lp.N_carrier + comb - 1) / comb : 0);
+        size_t spp = (size_t)(sp.streams_per_point > 0 ? sp.streams_per_point : 0), cells = n * 4 * spp;
+        double* md = (double*)devbuf(cells * 8 + 8);
+        int64_t* cd = (int64_t*)devbuf(n * 16);
+        double* mh = (double*)hostbuf(cells * 8 + 8);
+        int64_t* ch = (int64_t*)hostbuf(n * 16);
+        chk(ofdm_memset(g_ctx, md, 0, cells * 8), "memset");
+        chk(ofdm_memset(g_ctx, cd, 0, n * 16), "memset");
+        chk(ofdm_sweep_mse(g_ctx, &lp, &sp, Ldict, md, cd), op);
+        chk(ofdm_d2h(g_ctx, mh, md, cells * 8), "d2h");
+        chk(ofdm_d2h(g_ctx, ch, cd, n * 16), "d2h");
+        mxArray* mm = mxCreateDoubleMatrix(n, 4, mxREAL);           /* mean over the streams of each point */
+        for (i = 0; i < n; ++i)
+            for (e = 0; e < 4; ++e) {
+                double s = 0; size_t j;
+                for (j = 0; j < spp; ++j) s += mh[(i * 4 + e) * spp + j];
+                real_data(mm)[(size_t)e * n + i] = s / (double)spp;
+            }
+        OUT(0, mm);
+        mxArray* pm = mxCreateDoubleMatrix(spp, 4 * n, mxREAL);     /* reshape(per_stream, spp, 4, n_snr) in MATLAB */
+        memcpy(real_data(pm), mh, cells * 8);
+        OUT(1, pm);
+        mxArray* cm = mxCreateDoubleMatrix(n, 2, mxREAL);
+        for (i = 0; i < n; ++i) { real_data(cm)[i] = (double)ch[2 * i]; real_data(cm)[n + i] = (double)ch[2 * i + 1]; }
+        OUT(2, cm);
     } else {
         fail("ofdm:arg:op", "unknown operation");
     }

@@ -95,6 +95,7 @@ SIGNATURES = {
     "ofdm_rx_chain_t5_host_eps": (i32, [vp, C.POINTER(LinkParams), vp, i64, vp, vp, vp, vp, i64, dbl]),
     "ofdm_rx_chain_t4": (i32, [vp, C.POINTER(LinkParams), vp, i64, i32, i32, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, dbl]),
     "ofdm_sweep_ber": (i32, [vp, C.POINTER(LinkParams), C.POINTER(SweepParams), vp]),
+    "ofdm_sweep_mse": (i32, [vp, C.POINTER(LinkParams), C.POINTER(SweepParams), i32, vp, vp]),
     "ofdm_sweep_share": (i32, [i64, i32, i32, C.POINTER(i64), C.POINTER(i64)]),
     "ofdm_payload_bits": (i32, [vp, vp, i64, i64, u64, i64]),
     "ofdm_draw_sto_cfo": (i32, [vp, i64, u64, i64, i32, i32, vp, vp]),

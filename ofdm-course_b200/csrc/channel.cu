@@ -591,3 +591,12 @@ extern "C" int ofdm_mse(ofdm_ctx* ctx, const void* a_dev, int64_t a_stride, cons
     LAUNCH_CHECK(ctx);
     return OFDM_OK;
 }
+// Same kernel against ONE reference row shared by the batch (a_stride 0; not exported): ofdm_sweep_mse compares every estimate
+// with the single true response.  Per stream the sums are those of ofdm_mse on a replicated reference, bit for bit.
+int ofdm_mse_shared_ref(ofdm_ctx* ctx, const void* ref_dev, const void* b_dev, int64_t b_stride, int64_t B, int n, double* out_dev) {
+    REQUIRE(ctx, ref_dev && b_dev && out_dev && B >= 0 && n > 0 && b_stride >= n, "bad argument");
+    if (B == 0) return OFDM_OK;
+    DISPATCH_T(ctx, { mse_kernel<T><<<(unsigned)B, 256, 0, ctx->stream>>>((const cx<T>*)ref_dev, 0, (const cx<T>*)b_dev, b_stride, n, out_dev); });
+    LAUNCH_CHECK(ctx);
+    return OFDM_OK;
+}

@@ -67,6 +67,7 @@ __global__ void __launch_bounds__(CE_THREADS) estimate_channel_kernel(const cx<T
 // ---- MMSE_CE (`Task 5/MMSE_CE.m:13-38`).  Rows 1:Np of Rhp equal Rpp - I/snr, and only those rows
 // survive line 38, so H(1:Np) = Ht - Rpp^{-1} Ht / snr: one Hermitian-Toeplitz solve per stream,
 // done with Levinson's recursion in double (cond(Rpp) ~ snr*lambda_max is too much for FP32).
+// MEAS = true reads the measurement vectors Y = RX(pilot_loc,1)./Xp (B x Np, as ofdm_pilot_ls writes them) instead of grids.
 #define MM_THREADS 128
 __device__ __forceinline__ void block_sum4(double v[4], double (*red)[4]) {
     const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
@@ -79,7 +80,7 @@ __device__ __forceinline__ void block_sum4(double v[4], double (*red)[4]) {
     for (int q = 0; q < 4; ++q) { double s = 0; for (int k = 0; k < MM_THREADS / 32; ++k) s += red[k][q]; v[q] = s; }
 }
 
-template <typename T>
+template <typename T, bool MEAS = false>
 __global__ void __launch_bounds__(MM_THREADS) mmse_kernel(const cx<T>* __restrict__ grid, int64_t stream_stride, const int32_t* __restrict__ loc0,
                                                           const cx<T>* __restrict__ Xp, int Np, double Nps, int N_carrier, const cx<T>* __restrict__ h,
                                                           int h_len, const double* __restrict__ snr_db, PlanDev<T> p, cx<T>* __restrict__ H) {
@@ -110,7 +111,7 @@ __global__ void __launch_bounds__(MM_THREADS) mmse_kernel(const cx<T>* __restric
     for (int m = tid; m < Np; m += MM_THREADS) {
         double den = 1.0 + c * c * (double)m * (double)m;    // 1/(1+j c m) = (1 - j c m)/den
         t[m] = make_double2(1.0 / den + (m == 0 ? 1.0 / snr : 0.0), -c * (double)m / den);
-        Ht[m] = to_d(cdiv(Y[loc0[m]], Xp[m]));                // :17 computed in T like LS_CE, promoted
+        Ht[m] = MEAS ? to_d(Y[m]) : to_d(cdiv(Y[loc0[m]], Xp[m]));   // :17 computed in T like LS_CE, promoted
     }
     __syncthreads();
     // Levinson: T[i][j] = t[i-j] (i>=j), conj(t[j-i]) otherwise.  f solves T_m f = e_1; the backward
@@ -259,6 +260,28 @@ extern "C" int ofdm_mmse_ce(ofdm_ctx* ctx, const void* grid, int64_t B, int S, i
         auto k = mmse_kernel<T>;
         if (smem > 48 * 1024) CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         k<<<(unsigned)B, MM_THREADS, smem, ctx->stream>>>((const cx<T>*)grid, (int64_t)S * Nfft, l0, (const cx<T>*)xp, Np, (double)(loc[1] - loc[0]), Nc,
+                                                           (const cx<T>*)h, h_len, snr_db, plan_dev<T>(pl), (cx<T>*)H);
+    });
+    LAUNCH_CHECK(ctx);
+    return OFDM_OK;
+}
+
+// MMSE_CE from measurement vectors (not exported): y_dev B x Np = RX(pilot_loc,1)./Xp, h_dev B x h_len, snr_db_dev B doubles.
+// The same kernel as ofdm_mmse_ce with the quotient already taken, so the result is bit-identical to ofdm_mmse_ce on the grid
+// that ofdm_pilot_ls read y from.  Used by ofdm_sweep_mse, whose front end hands out y only.
+int ofdm_mmse_ce_meas(ofdm_ctx* ctx, const void* y, int64_t B, const int32_t* loc, int Np, int Nc, const void* h, int h_len, const double* snr_db,
+                      void* H) {
+    REQUIRE(ctx, y && H && loc && h && snr_db && Np >= 2 && Nc >= Np && h_len >= 1 && B >= 0, "bad argument");
+    const int32_t* l0; int rc = pilots0(ctx, loc, Np, Nc, &l0); if (rc) return rc;
+    if (B == 0) return OFDM_OK;
+    const InterpPlan* pl = ctx_plan(ctx, loc, Np, Nc, nullptr, Nc, OFDM_INTERP_SPLINE);
+    REQUIRE(ctx, pl != nullptr, "plan construction failed");
+    DISPATCH_T(ctx, {
+        size_t smem = 5 * sizeof(double2) * Np + 2 * sizeof(cx<T>) * pl->n_knots;
+        REQUIRE(ctx, smem <= 220 * 1024, "too many pilots for the in-SMEM Levinson solver");
+        auto k = mmse_kernel<T, true>;
+        if (smem > 48 * 1024) CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        k<<<(unsigned)B, MM_THREADS, smem, ctx->stream>>>((const cx<T>*)y, (int64_t)Np, l0, nullptr, Np, (double)(loc[1] - loc[0]), Nc,
                                                            (const cx<T>*)h, h_len, snr_db, plan_dev<T>(pl), (cx<T>*)H);
     });
     LAUNCH_CHECK(ctx);

@@ -1,4 +1,4 @@
-"""Monte-Carlo BER-vs-SNR sweep sharded over ranks (SURVEY 8e; loop shape of
+"""Monte-Carlo BER-vs-SNR and channel-estimation MSE-vs-SNR sweeps sharded over ranks (SURVEY 8e; loop shape of
 `Task 3/Main_model_Task_3.m:192-268`, `Task 5/Main_model_Task_5.m:303-346`, and the Task-4 impaired channel
 `Task 4/Main_model_Task_4.m:95-110,277-366` swept over SNR).
 
@@ -8,6 +8,10 @@ streams (equal to within one stream for any R) -- **no data-path collective**; t
 ``all_reduce(SUM)`` of the int64 counters at the end (NCCL on GPUs; the same host logic runs over ``gloo`` in the CPU
 tests with a stand-in compute function).  Payload bits, noise, STO and CFO draws are Philox streams keyed by g, so the
 counters do not depend on the number of ranks.
+
+``mse_sweep`` is the channel-estimation half of `Task 5/Main_model_Task_5.m:303-346` (LS / MMSE / MP / OMP MSE per stream,
+``ofdm_sweep_mse`` in csrc/sweep_mse.cu) on the same share rule; its per-stream float64 array is summed over the ranks,
+which is exact because every cell is written by exactly one rank.
 """
 from __future__ import annotations
 
@@ -18,6 +22,7 @@ import torch
 import torch.distributed as dist
 
 from . import _cabi
+from .part2 import ESTIMATORS  # noqa: F401  (order of the estimator axis: LS, MMSE, MP, OMP)
 
 CHAINS = {"task5": 0, "task4": 1}
 
@@ -96,3 +101,66 @@ def ber_sweep(ctx, lp, snrs_db, streams_per_point, taps=None, chain="task5", see
         reduce_counts(acc)                      # NCCL all-reduce on the device tensor, ordered after the sweep's stream work
     ctx.sync()
     return acc.cpu().numpy()
+
+
+def reduce_mse(per_stream, counts):
+    """Sum the per-stream MSE array (n_snr, 4, streams_per_point) float64 and the counters (n_snr, 2) int64 over all ranks
+    (no-op without an initialised process group) and take the mean over the streams of each point on the host.
+    Returns (mean[n_snr, 4], per_stream, counts) as NumPy arrays, identical on every rank."""
+    if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
+        dist.all_reduce(per_stream, op=dist.ReduceOp.SUM)     # exact: every cell is non-zero on one rank only
+        dist.all_reduce(counts, op=dist.ReduceOp.SUM)
+    per = per_stream.cpu().numpy()
+    return per.mean(axis=2), per, counts.cpu().numpy()
+
+
+def run_mse_sweep(snrs_db, streams_per_point, tile, compute, rank=0, world=1):
+    """Generic host driver of the MSE sweep (used with a stand-in ``compute`` in the gloo tests).
+    ``compute(snr_index, snr_db, first_stream, n_streams) -> (mse[4, n_streams], (streams, near_ties))`` processes one tile
+    on this rank; the result is that of :func:`reduce_mse`."""
+    snrs_db = list(snrs_db)
+    per = torch.zeros((len(snrs_db), 4, int(streams_per_point)), dtype=torch.float64)
+    counts = torch.zeros((len(snrs_db), 2), dtype=torch.int64)
+    for (i, s0, n) in tiles(len(snrs_db), streams_per_point, tile, rank, world):
+        m, c = compute(i, snrs_db[i], s0, n)
+        per[i, :, s0:s0 + n] = torch.as_tensor(np.asarray(m, dtype=np.float64))
+        counts[i] += torch.as_tensor(np.asarray(c, dtype=np.int64))
+    return reduce_mse(per, counts)
+
+
+def mse_sweep_local(ctx, lp, snrs_db, streams_per_point, taps, Ldict=None, seed=1, rank=0, world=1, tile=0, tie_eps=0.0, per_stream=None, counts=None):
+    """This rank's share of the MSE sweep through ``ofdm_sweep_mse``, WITHOUT synchronising: writes its cells of
+    ``per_stream`` (n_snr, 4, streams_per_point) float64 and adds to ``counts`` (n_snr, 2) int64 {streams, OMP frames with a
+    near-tie}; both are zero-initialised device tensors when not given.  ``Ldict`` defaults to the script's
+    ceil(N_carrier / comb) (`Main_model_Task_5.m:182-190`)."""
+    snr = np.ascontiguousarray(np.asarray(snrs_db, dtype=np.float64))
+    pc = np.asarray(lp.pilotCarriers)
+    if Ldict is None:
+        Ldict = -(-int(lp.N_carrier) // int(pc[1] - pc[0]))
+    sp = _cabi.SweepParams()
+    sp.chain = CHAINS["task5"]
+    sp.n_snr = snr.size
+    sp.snr_db_host = snr.ctypes.data_as(_cabi.pdbl)
+    sp.streams_per_point = int(streams_per_point)
+    sp.tile_streams = int(tile)
+    sp.rank, sp.world = int(rank), int(world)
+    sp.seed = int(seed)
+    t = np.ascontiguousarray(np.asarray(taps, dtype=np.float64).reshape(-1, 2))
+    sp.taps_host = t.ctypes.data_as(_cabi.pdbl)
+    sp.n_taps = t.shape[0]
+    sp.near_eps = float(tie_eps)
+    if per_stream is None:
+        per_stream = torch.zeros((snr.size, 4, int(streams_per_point)), dtype=torch.float64, device=ctx.device)
+    if counts is None:
+        counts = torch.zeros((snr.size, 2), dtype=torch.int64, device=ctx.device)
+    ctx._chk(ctx.lib.ofdm_sweep_mse(ctx.h, C.byref(lp), C.byref(sp), int(Ldict), ctx.p(per_stream), ctx.p(counts)))
+    return per_stream, counts
+
+
+def mse_sweep(ctx, lp, snrs_db, streams_per_point, taps, Ldict=None, seed=1, rank=0, world=1, tile=0, tie_eps=0.0):
+    """Whole MSE-vs-SNR sweep: this rank's call, then one all-reduce each of the per-stream array and the counters.
+    Returns (mean[n_snr, 4], per_stream[n_snr, 4, streams_per_point], counts[n_snr, 2]) on the host, estimators in the
+    order LS, MMSE, MP, OMP; identical on every rank and for every world size and tile."""
+    per, cnt = mse_sweep_local(ctx, lp, snrs_db, streams_per_point, taps, Ldict, seed, rank, world, tile, tie_eps)
+    ctx.sync()
+    return reduce_mse(per, cnt)                 # NCCL all-reduce on the device tensors when world > 1
