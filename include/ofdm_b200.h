@@ -355,6 +355,39 @@ OFDM_API int ofdm_sweep_ber(ofdm_ctx*, const ofdm_link_params*, const ofdm_sweep
  * the rank count or the tile size; the caller sums the arrays of all ranks (each cell is written by one rank). */
 OFDM_API int ofdm_sweep_mse(ofdm_ctx*, const ofdm_link_params*, const ofdm_sweep_params*, int Ldict, double* mse_dev,
                             int64_t* counts_dev);
+/* Task-5 part-2 pilot-density study (`Task 5/Task5_part2.m:46-321`): n_points pilot layouts x mc_runs static fading runs x
+ * the LS / MMSE / MP / OMP estimators; for every cell the NMSE of the estimate (`:200-203`) and the bit errors after equalising
+ * with it (`:269-303`).  From `base` the call reads Nfft, Tg, N_carrier, S, SpF and the constellation only; the data carriers
+ * of a point are the complement of its pilots in 1..N_carrier, scrambling is off (`:99-115`).  Keys, those of the composed
+ * Python driver part2.run_point: point k transmits the first S * Nd_k * bps payload bits through ofdm_tx_chain, gets AWGN
+ * once (ofdm_add_noise, first_stream_id k), run r fades with ofdm_tdl_channel(first_stream_id k * 1,000,003 + r); MMSE gets
+ * the true impulse response zero-padded to N_carrier, MP / OMP the partial-DFT dictionary of ldict_host[k] columns with
+ * K = n_paths of the profile.  Work item g = k * mc_runs + r; the call processes the share ofdm_sweep_share(n_points *
+ * mc_runs, rank, world) gives, in tiles of tile_runs runs (0 = 4096) that never straddle a point. */
+typedef struct ofdm_part2_params {
+    int32_t n_points;
+    const int32_t* pilot_offsets_host;  /* n_points + 1, from 0: point k's pilots are pilot_carriers_host[off[k] .. off[k+1]) */
+    const int32_t* pilot_carriers_host; /* 1-based, strictly increasing within 1..N_carrier per point, >= 2 per point */
+    const int32_t* ldict_host;          /* n_points: MP/OMP dictionary columns, Np <= Ldict <= Nfft */
+    const double* pilot_pattern_host;   /* 2 complex doubles: pilot q (0-based) carries pattern[q % 2] in every symbol */
+    const uint32_t* payload_host;       /* packed payload bits; point k transmits the first S * Nd_k * bps of them */
+    int64_t payload_bits;
+    int32_t profile;                    /* as ofdm_tdl_channel: 0 EPA, 1 EVA, 2 ETU */
+    double fs_hz;
+    double snr_db;
+    int64_t mc_runs;                    /* 1 .. 1,000,003 */
+    int64_t tile_runs;                  /* runs per work item; 0 = 4096 (per run about 4 Nfft + 3 N_carrier complex of temporaries) */
+    int32_t rank, world;
+    uint64_t seed;
+    double near_eps;                    /* symbols whose two smallest squared distances differ by less are counted */
+    double tie_eps;                     /* OMP near-tie threshold, as ofdm_omp_ex */
+} ofdm_part2_params;
+/* nmse_dev: n_points x 4 x mc_runs doubles, [k][e][r] with e = LS, MMSE, MP, OMP; only this call's share is written.
+ * counts_dev: n_points x 4 x 3 int64 += {bit errors, bits, symbols within near_eps of a decision boundary}.
+ * runs_dev: n_points x 2 int64 += {runs processed, OMP runs with a near-tie}.  The values do not depend on the rank count
+ * or the tile size; the caller sums the arrays of all ranks (each NMSE cell is written by one rank). */
+OFDM_API int ofdm_sweep_part2(ofdm_ctx*, const ofdm_link_params* base, const ofdm_part2_params*, double* nmse_dev,
+                              int64_t* counts_dev, int64_t* runs_dev);
 /* first / count of the contiguous share of `total_streams` that (rank, world) processes */
 OFDM_API int ofdm_sweep_share(int64_t total_streams, int rank, int world, int64_t* first, int64_t* count);
 /* The sweep's synthetic inputs, also usable on their own: payload words of streams first_stream_id .. +n_streams-1

@@ -693,6 +693,107 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
         mxArray* cm = mxCreateDoubleMatrix(n, 2, mxREAL);
         for (i = 0; i < n; ++i) { real_data(cm)[i] = (double)ch[2 * i]; real_data(cm)[n + i] = (double)ch[2 * i + 1]; }
         OUT(2, cm);
+    } else if (!strcmp(op, "sweep_part2")) {   /* [NMSE (4 x n_points), BER (4 x n_points), per_run (mc_runs x 4*n_points), counts (12 x n_points),
+                                                   runs (2 x n_points)] = sweep_part2(Nfft, T_Guard, N_carrier, N_symb, SpF, Constellation,
+                                                   pilots, offsets, Ldict, pattern, bits, profile, fs, SNR, monteCarloRuns, seed, near_eps, tie_eps):
+                                                   offsets = [] -> pilots is a vector of combs (pilots 1:comb:N_carrier, Ldict ceil(Nfft/comb));
+                                                   else pilots are the concatenated 1-based pilot vectors of the points, offsets (n_points + 1,
+                                                   from 0) delimit them and Ldict defaults to Nfft.  Ldict = [] takes the defaults.  pattern: the
+                                                   two pilot values (pilot q carries pattern(mod(q-1,2)+1)).  bits: 0/1 payload.  Single GPU. */
+        NEED(18);
+        ofdm_link_params lp;
+        ofdm_part2_params pp;
+        char prof[8];
+        size_t i, P, n_comb = mxGetNumberOfElements(A(6)), n_off = mxGetNumberOfElements(A(7));
+        int e;
+        memset(&lp, 0, sizeof lp);
+        memset(&pp, 0, sizeof pp);
+        lp.Nfft = (int32_t)mxGetScalar(A(0)); lp.Tg = (int32_t)mxGetScalar(A(1)); lp.N_carrier = (int32_t)mxGetScalar(A(2));
+        lp.S = (int32_t)mxGetScalar(A(3)); lp.SpF = (int32_t)mxGetScalar(A(4));
+        lp.constellation = constellation_id(A(5));
+        const double* pil = real_data(A(6));
+        int32_t* off; int32_t* car; int32_t* ld;
+        if (n_off == 0) {                                               /* combs (`Task5_part2.m:50-55`) */
+            size_t tot = 0;
+            P = n_comb;
+            if (!P) fail("ofdm:sweep_part2:pilots", "need at least one comb");
+            for (i = 0; i < P; ++i) {
+                if (pil[i] < 1) fail("ofdm:sweep_part2:pilots", "combs must be >= 1");
+                tot += (size_t)((lp.N_carrier + (int)pil[i] - 1) / (int)pil[i]);
+            }
+            off = (int32_t*)hostbuf((P + 1) * 4); car = (int32_t*)hostbuf(tot * 4 + 4); ld = (int32_t*)hostbuf(P * 4);
+            for (i = 0; i < P; ++i) {
+                int comb = (int)pil[i], c;
+                off[i + 1] = off[i];
+                for (c = 1; c <= lp.N_carrier; c += comb) car[off[i + 1]++] = c;
+                ld[i] = (lp.Nfft + comb - 1) / comb;                    /* F(:,1:ceil(Nfft/comb)), `:183-185` */
+            }
+        } else {                                                        /* explicit pilot vectors (random masks, `:57-65`) */
+            const double* po = real_data(A(7));
+            P = n_off - 1;
+            if (!P) fail("ofdm:sweep_part2:pilots", "offsets must have n_points + 1 entries");
+            off = (int32_t*)hostbuf((P + 1) * 4); car = (int32_t*)hostbuf(n_comb * 4 + 4); ld = (int32_t*)hostbuf(P * 4);
+            for (i = 0; i <= P; ++i) {
+                off[i] = (int32_t)llround(po[i]);
+                if (off[i] < 0 || (size_t)off[i] > n_comb) fail("ofdm:sweep_part2:pilots", "offsets must lie in 0..numel(pilots)");
+            }
+            for (i = 0; i < n_comb; ++i) car[i] = (int32_t)llround(pil[i]);
+            for (i = 0; i < P; ++i) ld[i] = lp.Nfft;
+        }
+        if (mxGetNumberOfElements(A(8))) {
+            if (mxGetNumberOfElements(A(8)) != P) fail("ofdm:sweep_part2:ldict", "Ldict must have one entry per point");
+            for (i = 0; i < P; ++i) ld[i] = (int32_t)llround(real_data(A(8))[i]);
+        }
+        if (mxGetNumberOfElements(A(9)) != 2) fail("ofdm:sweep_part2:pattern", "the pilot pattern must have two values");
+        size_t nbits = mxGetNumberOfElements(A(10));
+        uint32_t* words = (uint32_t*)hostbuf(OFDM_BIT_WORDS(nbits) * 4 + 4);
+        for (i = 0; i < nbits; ++i) if (real_data(A(10))[i] != 0.0) words[i >> 5] |= 1u << (i & 31);
+        if (!mxIsChar(A(11)) || mxGetString(A(11), prof, sizeof prof)) fail("ofdm:sweep_part2:profile", "profile must be 'EPA', 'EVA' or 'ETU'");
+        pp.profile = !strcmp(prof, "EPA") ? 0 : !strcmp(prof, "EVA") ? 1 : !strcmp(prof, "ETU") ? 2 : -1;
+        if (pp.profile < 0) fail("ofdm:sweep_part2:profile", "profile must be 'EPA', 'EVA' or 'ETU'");
+        pp.n_points = (int32_t)P;
+        pp.pilot_offsets_host = off; pp.pilot_carriers_host = car; pp.ldict_host = ld;
+        pp.pilot_pattern_host = to_cdoubles(A(9), 2);
+        pp.payload_host = words; pp.payload_bits = (int64_t)nbits;
+        pp.fs_hz = mxGetScalar(A(12)); pp.snr_db = mxGetScalar(A(13));
+        pp.mc_runs = (int64_t)mxGetScalar(A(14));
+        pp.rank = 0; pp.world = 1;
+        pp.seed = (uint64_t)mxGetScalar(A(15));
+        pp.near_eps = mxGetScalar(A(16)); pp.tie_eps = mxGetScalar(A(17));
+        size_t R = (size_t)(pp.mc_runs > 0 ? pp.mc_runs : 0), cells = P * 4 * R;
+        double* md = (double*)devbuf(cells * 8 + 8);
+        int64_t* cd = (int64_t*)devbuf(P * 96);
+        int64_t* rd = (int64_t*)devbuf(P * 16);
+        double* mh = (double*)hostbuf(cells * 8 + 8);
+        int64_t* ch = (int64_t*)hostbuf(P * 96);
+        int64_t* rh = (int64_t*)hostbuf(P * 16);
+        chk(ofdm_memset(g_ctx, md, 0, cells * 8), "memset");
+        chk(ofdm_memset(g_ctx, cd, 0, P * 96), "memset");
+        chk(ofdm_memset(g_ctx, rd, 0, P * 16), "memset");
+        chk(ofdm_sweep_part2(g_ctx, &lp, &pp, md, cd, rd), op);
+        chk(ofdm_d2h(g_ctx, mh, md, cells * 8), "d2h");
+        chk(ofdm_d2h(g_ctx, ch, cd, P * 96), "d2h");
+        chk(ofdm_d2h(g_ctx, rh, rd, P * 16), "d2h");
+        mxArray* nm = mxCreateDoubleMatrix(4, P, mxREAL);              /* `Task5_part2.m:305-314`: estimators x points */
+        mxArray* bm = mxCreateDoubleMatrix(4, P, mxREAL);
+        for (i = 0; i < P; ++i)
+            for (e = 0; e < 4; ++e) {
+                double s = 0; size_t r;
+                for (r = 0; r < R; ++r) s += mh[(i * 4 + e) * R + r];
+                real_data(nm)[i * 4 + e] = s / (double)R;
+                real_data(bm)[i * 4 + e] = (double)ch[i * 12 + 3 * e] / (double)ch[i * 12 + 3 * e + 1];
+            }
+        OUT(0, nm);
+        OUT(1, bm);
+        mxArray* pm = mxCreateDoubleMatrix(R, 4 * P, mxREAL);          /* reshape(per_run, mc_runs, 4, n_points) in MATLAB */
+        memcpy(real_data(pm), mh, cells * 8);
+        OUT(2, pm);
+        mxArray* cm = mxCreateDoubleMatrix(12, P, mxREAL);             /* reshape(counts, 3, 4, n_points): {errors, bits, near} */
+        for (i = 0; i < 12 * P; ++i) real_data(cm)[i] = (double)ch[i];
+        OUT(3, cm);
+        mxArray* rm = mxCreateDoubleMatrix(2, P, mxREAL);              /* {runs, OMP runs with a near-tie} */
+        for (i = 0; i < 2 * P; ++i) real_data(rm)[i] = (double)rh[i];
+        OUT(4, rm);
     } else {
         fail("ofdm:arg:op", "unknown operation");
     }

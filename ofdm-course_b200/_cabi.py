@@ -32,6 +32,15 @@ class SweepParams(C.Structure):
                 ("cfo_int_max", C.c_int32)]
 
 
+class Part2Params(C.Structure):
+    """``ofdm_part2_params`` of include/ofdm_b200.h."""
+    _fields_ = [("n_points", C.c_int32), ("pilot_offsets_host", pi32), ("pilot_carriers_host", pi32), ("ldict_host", pi32),
+                ("pilot_pattern_host", pdbl), ("payload_host", C.POINTER(C.c_uint32)), ("payload_bits", C.c_int64),
+                ("profile", C.c_int32), ("fs_hz", C.c_double), ("snr_db", C.c_double), ("mc_runs", C.c_int64),
+                ("tile_runs", C.c_int64), ("rank", C.c_int32), ("world", C.c_int32), ("seed", C.c_uint64),
+                ("near_eps", C.c_double), ("tie_eps", C.c_double)]
+
+
 # name -> (restype, argtypes); every symbol declared in include/ofdm_b200.h
 SIGNATURES = {
     "ofdm_ctx_create": (i32, [C.POINTER(vp), i32, i32]),
@@ -96,6 +105,7 @@ SIGNATURES = {
     "ofdm_rx_chain_t4": (i32, [vp, C.POINTER(LinkParams), vp, i64, i32, i32, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, dbl]),
     "ofdm_sweep_ber": (i32, [vp, C.POINTER(LinkParams), C.POINTER(SweepParams), vp]),
     "ofdm_sweep_mse": (i32, [vp, C.POINTER(LinkParams), C.POINTER(SweepParams), i32, vp, vp]),
+    "ofdm_sweep_part2": (i32, [vp, C.POINTER(LinkParams), C.POINTER(Part2Params), vp, vp, vp]),
     "ofdm_sweep_share": (i32, [i64, i32, i32, C.POINTER(i64), C.POINTER(i64)]),
     "ofdm_payload_bits": (i32, [vp, vp, i64, i64, u64, i64]),
     "ofdm_draw_sto_cfo": (i32, [vp, i64, u64, i64, i32, i32, vp, vp]),

@@ -8,8 +8,14 @@ ofdm_tdl_channel (stand-in for lteFadingChannel), ofdm_apply_fir, ofdm_demodulat
 ofdm_pilot_ls, ofdm_mp, ofdm_omp, ofdm_fft, ofdm_mse, ofdm_equalize, ofdm_get_payload, ofdm_demap,
 ofdm_ber_count.  Points x run-blocks are dealt round-robin to the ranks; every (point, run, estimator) cell is
 written by exactly one rank, so the closing all_reduce(SUM) is exact and independent of the rank count.
+
+``sweep_lib`` runs the same experiment as ONE C-ABI call per rank, ``ofdm_sweep_part2`` (csrc/sweep_part2.cu), with the keys
+of ``run_point``: its per-run NMSE and per-point error counts equal those of ``sweep`` bit for bit.  Ranks take the contiguous
+share of the (point, run) items that ``ofdm_sweep_share`` gives, as the other library sweeps do.
 """
 from __future__ import annotations
+
+import ctypes as C
 
 import numpy as np
 import torch
@@ -122,3 +128,94 @@ def sweep(ctx, combs, mc_runs, payload, *, block=None, rank=0, world=1, reg_pilo
     NMSE = nm.mean(dim=1).numpy().T                               # mean over the Monte-Carlo runs, :311-314
     BER = (er.double() / nb.double()[:, None]).numpy().T          # equal run sizes: mean of per-run BERs, :305-308
     return NMSE, BER
+
+
+def lib_layout(combs, N_carrier=1024, Nfft=4096, reg_pilot=True, random_masks=None):
+    """The pilot layouts of ``sweep`` in the form ``ofdm_sweep_part2`` takes: (offsets int32[n_points + 1], 1-based pilot
+    carriers int32 concatenated over the points, Ldict int32[n_points]) with the layout and Ldict rules of ``sweep``."""
+    n_pts = len(combs)
+    pcs, ldict = [], []
+    for k in range(n_pts):
+        if reg_pilot:
+            comb = int(combs[k])
+            pc, _ = layout(N_carrier, comb=comb)
+            ldict.append(-(-Nfft // comb))
+        else:
+            pc, _ = layout(N_carrier, pilotCarriers=random_masks[k])
+            ldict.append(Nfft)
+        pcs.append(pc)
+    offsets = np.concatenate([[0], np.cumsum([len(pc) for pc in pcs])]).astype(np.int32)
+    return offsets, np.concatenate(pcs).astype(np.int32), np.asarray(ldict, dtype=np.int32)
+
+
+def pilot_pattern(amp):
+    """The two pilot values of ``pilot_values`` (pilot q carries pattern[q % 2] in every symbol), as the exact doubles."""
+    return pilot_values(2, 1, amp)[:, 0]
+
+
+def reduce_part2(per_run, counts, runs):
+    """Sum the per-run NMSE (n_points, 4, mc_runs) float64, the counts (n_points, 4, 3) and the runs (n_points, 2) int64 over
+    all ranks (no-op without an initialised process group), then form ``sweep``'s results with its own arithmetic.
+    Returns (NMSE[4, n_points], BER[4, n_points], per_run, counts, runs) as NumPy arrays, identical on every rank."""
+    if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
+        for t in (per_run, counts, runs):
+            dist.all_reduce(t, op=dist.ReduceOp.SUM)         # exact: every NMSE cell is non-zero on one rank only
+    per, cnt, rn = per_run.cpu().numpy(), counts.cpu().numpy(), runs.cpu().numpy()
+    nm = torch.from_numpy(np.ascontiguousarray(per.transpose(0, 2, 1)))      # the (point, run, estimator) layout of sweep
+    er = torch.from_numpy(np.ascontiguousarray(cnt[:, :, 0]))
+    nb = torch.from_numpy(np.ascontiguousarray(cnt[:, 0, 1]))
+    NMSE = nm.mean(dim=1).numpy().T
+    BER = (er.double() / nb.double()[:, None]).numpy().T
+    return NMSE, BER, per, cnt, rn
+
+
+def sweep_lib_local(ctx, combs, mc_runs, payload_bits, *, tile=0, rank=0, world=1, reg_pilot=True, random_masks=None, profile="EPA",
+                    fs_hz=4e7, snr_db=20.0, seed=1, near_eps=0.0, tie_eps=0.0, Nfft=4096, N_carrier=1024, frames=2, spf=7,
+                    constellation="16QAM", per_run=None, counts=None, runs=None):
+    """This rank's share of the experiment through ``ofdm_sweep_part2``, WITHOUT synchronising: writes its cells of ``per_run``
+    (n_points, 4, mc_runs) float64 and adds to ``counts`` (n_points, 4, 3) and ``runs`` (n_points, 2) int64; all three are
+    zero-initialised device tensors when not given.  ``payload_bits``: uint8 0/1, at least the longest stream of any point."""
+    from . import _cabi
+    from . import link as G
+    offsets, carriers, ldict = lib_layout(combs, N_carrier, Nfft, reg_pilot, random_masks)
+    n_pts = ldict.size
+    d, _ = G.constellation_func(constellation)
+    pattern = np.ascontiguousarray(pilot_pattern(2.0 * float(np.max(np.abs(d)))))
+    bits = np.asarray(payload_bits, dtype=np.uint8).ravel()
+    words = G.pack_bits(bits)
+    lp = _cabi.LinkParams()
+    lp.Nfft, lp.Tg, lp.N_carrier, lp.S, lp.SpF = int(Nfft), int(Nfft) // 8, int(N_carrier), int(frames * spf), int(spf)
+    lp.constellation = G.CONSTELLATIONS[str(constellation)]
+    pp = _cabi.Part2Params()
+    pp.n_points = n_pts
+    pp.pilot_offsets_host = offsets.ctypes.data_as(_cabi.pi32)
+    pp.pilot_carriers_host = carriers.ctypes.data_as(_cabi.pi32)
+    pp.ldict_host = ldict.ctypes.data_as(_cabi.pi32)
+    pp.pilot_pattern_host = pattern.ctypes.data_as(_cabi.pdbl)
+    pp.payload_host = words.ctypes.data_as(C.POINTER(C.c_uint32))
+    pp.payload_bits = bits.size
+    pp.profile = G.TDL_PROFILES[str(profile).upper()]
+    pp.fs_hz, pp.snr_db = float(fs_hz), float(snr_db)
+    pp.mc_runs, pp.tile_runs = int(mc_runs), int(tile)
+    pp.rank, pp.world, pp.seed = int(rank), int(world), int(seed)
+    pp.near_eps, pp.tie_eps = float(near_eps), float(tie_eps)
+    if per_run is None:
+        per_run = torch.zeros((n_pts, 4, int(mc_runs)), dtype=torch.float64, device=ctx.device)
+    if counts is None:
+        counts = torch.zeros((n_pts, 4, 3), dtype=torch.int64, device=ctx.device)
+    if runs is None:
+        runs = torch.zeros((n_pts, 2), dtype=torch.int64, device=ctx.device)
+    ctx._chk(ctx.lib.ofdm_sweep_part2(ctx.h, C.byref(lp), C.byref(pp), ctx.p(per_run), ctx.p(counts), ctx.p(runs)))
+    return per_run, counts, runs
+
+
+def sweep_lib(ctx, combs, mc_runs, payload_bits, *, tile=0, rank=0, world=1, reg_pilot=True, random_masks=None, **kw):
+    """The whole experiment as one library call per rank, then one all-reduce each of the per-run array, the counts and the
+    runs.  Takes ``sweep``'s layout arguments; ``payload_bits`` are the bits ``sweep``'s ``payload`` would return (point k sends
+    the first S * Nd_k * bps of them).  Returns (NMSE[4, n_points], BER[4, n_points], per_run[n_points, 4, mc_runs],
+    counts[n_points, 4, 3] {errors, bits, near-boundary symbols}, runs[n_points, 2] {runs, OMP runs with a near-tie}),
+    estimators in the order LS, MMSE, MP, OMP; identical on every rank and for every world size and tile."""
+    per, cnt, rn = sweep_lib_local(ctx, combs, mc_runs, payload_bits, tile=tile, rank=rank, world=world, reg_pilot=reg_pilot,
+                                   random_masks=random_masks, **kw)
+    ctx.sync()
+    return reduce_part2(per, cnt, rn)             # NCCL all-reduce on the device tensors when world > 1
