@@ -388,6 +388,40 @@ typedef struct ofdm_part2_params {
  * or the tile size; the caller sums the arrays of all ranks (each NMSE cell is written by one rank). */
 OFDM_API int ofdm_sweep_part2(ofdm_ctx*, const ofdm_link_params* base, const ofdm_part2_params*, double* nmse_dev,
                               int64_t* counts_dev, int64_t* runs_dev);
+/* Task-4 synchroniser and channel-estimate accuracy study over SNR (`Task 4/Main_model_Task_4.m:95-110,277-374`,
+ * `Task 4/README.md:111-121,189-193`): per stream TX -> Noise -> add_STO -> add_CFO -> multipath -> the M2 RX chain of
+ * ofdm_rx_chain_t4_ex (its split form, for any tile size), reporting the estimates, the channel-estimate error and the MER.
+ * Share rule, stream numbering g = snr_index * streams_per_point + j, tiles and the Philox keys of the payload, noise and
+ * STO / CFO draws are those of ofdm_sweep_ber's Task-4 chain: with sto_mode 0 and all three desync flags on, the same seed
+ * transmits the same streams.  FP32 contexts and Nfft = 1024 only (OFDM_ERR_UNSUPPORTED otherwise); word-aligned streams.
+ * rec_dev: n_snr x 9 x streams_per_point doubles, [i][f][j]; only this call's share is written.  Fields f:
+ *   0 TgPosition (1-based, 65 on detector failure; 0 when time_desync = 0, the offset the chain then applies)
+ *   1 FreqOffset (0 when freq_desync = 0)
+ *   2 IFO (-1: no bin above 0.77, the chain then removes none; 0 when freq_desync = 0)
+ *   3 tau, 4 phase_shift of fine_sync (0 when time_desync = freq_desync = 0)
+ *   5 mean over k = 1..N_carrier of |H_est(k) - H(k)|^2, H = fft(h, Nfft)(1:N_carrier) of the taps in double (H = 1 without
+ *     multipath); NaN when mp_desync = 0, or where the estimate itself is NaN (a failed synchronisation)
+ *   6 MER_func of the stream's equalised data carriers in dB (`MER_func.m:7-25`)
+ *   7 the true STO (nsto), 8 the true CFO
+ * counts_dev: n_snr x 4 int64 += {bit errors, bits, guard-interval detector failures, streams with IFO = -1}.  The values
+ * do not depend on the rank count or the tile size; the caller sums the arrays of all ranks (each record cell is written by
+ * one rank). */
+typedef struct ofdm_sync_params {
+    int32_t n_snr;
+    const double* snr_db_host;   /* n_snr SNR points in dB */
+    int64_t streams_per_point;
+    int64_t tile_streams;        /* streams per work item; 0 = 8192 (two signal buffers of tile x stream bytes are allocated) */
+    int32_t rank, world;
+    uint64_t seed;
+    const double* taps_host;     /* n_taps x 2 doubles (delay, amplitude), delays integers in [0, Nfft); n_taps = 0: no multipath */
+    int32_t n_taps;
+    int32_t sto_mode;            /* 0: drawn as ofdm_sweep_ber (sto_max, cfo_int_max); 1: sto_fixed / cfo_fixed for every stream */
+    int32_t sto_max, cfo_int_max;
+    int32_t sto_fixed;
+    double cfo_fixed;
+    int32_t time_desync, freq_desync, mp_desync;   /* receiver stages, as ofdm_rx_chain_t4_ex */
+} ofdm_sync_params;
+OFDM_API int ofdm_sweep_sync(ofdm_ctx*, const ofdm_link_params*, const ofdm_sync_params*, double* rec_dev, int64_t* counts_dev);
 /* first / count of the contiguous share of `total_streams` that (rank, world) processes */
 OFDM_API int ofdm_sweep_share(int64_t total_streams, int rank, int world, int64_t* first, int64_t* count);
 /* The sweep's synthetic inputs, also usable on their own: payload words of streams first_stream_id .. +n_streams-1

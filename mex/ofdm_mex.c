@@ -693,6 +693,54 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
         mxArray* cm = mxCreateDoubleMatrix(n, 2, mxREAL);
         for (i = 0; i < n; ++i) { real_data(cm)[i] = (double)ch[2 * i]; real_data(cm)[n + i] = (double)ch[2 * i + 1]; }
         OUT(2, cm);
+    } else if (!strcmp(op, "sweep_sync")) {   /* [rec (spp x 9*n_snr), counts (n_snr x 4)] =
+                                                 sweep_sync(LINK..., snrs, streams_per_point, taps (K x 2, [] = none), seed, sto, cfo,
+                                                 [time_desync freq_desync mp_desync] [, sto_max, cfo_int_max]);
+                                                 sto < 0: STO / CFO drawn as sweep_ber (sto_max defaults to Nfft + T_Guard, cfo_int_max
+                                                 to 30); else every stream gets sto and cfo */
+        NEED(N_LINK + 7);
+        ofdm_link_params lp;
+        ofdm_sync_params sp;
+        parse_link(&A(0), &lp);
+        memset(&sp, 0, sizeof sp);
+        size_t n = mxGetNumberOfElements(A(N_LINK)), i;
+        int K = (int)mxGetM(A(N_LINK + 2)), k2;
+        if (!n) fail("ofdm:sweep_sync:snr", "need at least one SNR point");
+        if (K && mxGetN(A(N_LINK + 2)) != 2) fail("ofdm:sweep_sync:taps", "channel_taps must be K x 2 (delay, amplitude) or []");
+        if (mxGetNumberOfElements(A(N_LINK + 6)) != 3) fail("ofdm:sweep_sync:flags", "flags must be [time_desync freq_desync mp_desync]");
+        sp.n_snr = (int32_t)n;
+        sp.snr_db_host = real_data(A(N_LINK));
+        sp.streams_per_point = (int64_t)mxGetScalar(A(N_LINK + 1));
+        sp.rank = 0; sp.world = 1;
+        sp.seed = (uint64_t)mxGetScalar(A(N_LINK + 3));
+        if (K) {
+            double* tp = real_data(A(N_LINK + 2));
+            double* taps = (double*)hostbuf((size_t)K * 16);
+            for (k2 = 0; k2 < K; ++k2) { taps[2 * k2] = tp[k2]; taps[2 * k2 + 1] = tp[K + k2]; }
+            sp.taps_host = taps; sp.n_taps = K;
+        }
+        const double sto = mxGetScalar(A(N_LINK + 4));
+        sp.sto_mode = sto < 0 ? 0 : 1;
+        sp.sto_fixed = sto < 0 ? 0 : (int32_t)sto;
+        sp.cfo_fixed = mxGetScalar(A(N_LINK + 5));
+        sp.sto_max = nrhs > N_LINK + 8 ? (int32_t)mxGetScalar(A(N_LINK + 7)) : lp.Nfft + lp.Tg;
+        sp.cfo_int_max = nrhs > N_LINK + 9 ? (int32_t)mxGetScalar(A(N_LINK + 8)) : 30;
+        const double* fl = real_data(A(N_LINK + 6));
+        sp.time_desync = fl[0] != 0; sp.freq_desync = fl[1] != 0; sp.mp_desync = fl[2] != 0;
+        size_t spp = (size_t)(sp.streams_per_point > 0 ? sp.streams_per_point : 0), cells = n * 9 * spp;
+        double* rd = (double*)devbuf(cells * 8 + 8);
+        int64_t* cd = (int64_t*)devbuf(n * 32);
+        int64_t* ch = (int64_t*)hostbuf(n * 32);
+        chk(ofdm_memset(g_ctx, rd, 0, cells * 8), "memset");
+        chk(ofdm_memset(g_ctx, cd, 0, n * 32), "memset");
+        chk(ofdm_sweep_sync(g_ctx, &lp, &sp, rd, cd), op);
+        mxArray* rm = mxCreateDoubleMatrix(spp, 9 * n, mxREAL);     /* reshape(rec, spp, 9, n_snr) in MATLAB */
+        chk(ofdm_d2h(g_ctx, real_data(rm), rd, cells * 8), "d2h");
+        chk(ofdm_d2h(g_ctx, ch, cd, n * 32), "d2h");
+        OUT(0, rm);
+        mxArray* cm = mxCreateDoubleMatrix(n, 4, mxREAL);
+        for (i = 0; i < n; ++i) { int j; for (j = 0; j < 4; ++j) real_data(cm)[(size_t)j * n + i] = (double)ch[4 * i + j]; }
+        OUT(1, cm);
     } else if (!strcmp(op, "sweep_part2")) {   /* [NMSE (4 x n_points), BER (4 x n_points), per_run (mc_runs x 4*n_points), counts (12 x n_points),
                                                    runs (2 x n_points)] = sweep_part2(Nfft, T_Guard, N_carrier, N_symb, SpF, Constellation,
                                                    pilots, offsets, Ldict, pattern, bits, profile, fs, SNR, monteCarloRuns, seed, near_eps, tie_eps):

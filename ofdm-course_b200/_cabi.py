@@ -41,6 +41,14 @@ class Part2Params(C.Structure):
                 ("near_eps", C.c_double), ("tie_eps", C.c_double)]
 
 
+class SyncParams(C.Structure):
+    """``ofdm_sync_params`` of include/ofdm_b200.h."""
+    _fields_ = [("n_snr", C.c_int32), ("snr_db_host", pdbl), ("streams_per_point", C.c_int64), ("tile_streams", C.c_int64),
+                ("rank", C.c_int32), ("world", C.c_int32), ("seed", C.c_uint64), ("taps_host", pdbl), ("n_taps", C.c_int32),
+                ("sto_mode", C.c_int32), ("sto_max", C.c_int32), ("cfo_int_max", C.c_int32), ("sto_fixed", C.c_int32),
+                ("cfo_fixed", C.c_double), ("time_desync", C.c_int32), ("freq_desync", C.c_int32), ("mp_desync", C.c_int32)]
+
+
 # name -> (restype, argtypes); every symbol declared in include/ofdm_b200.h
 SIGNATURES = {
     "ofdm_ctx_create": (i32, [C.POINTER(vp), i32, i32]),
@@ -106,6 +114,7 @@ SIGNATURES = {
     "ofdm_sweep_ber": (i32, [vp, C.POINTER(LinkParams), C.POINTER(SweepParams), vp]),
     "ofdm_sweep_mse": (i32, [vp, C.POINTER(LinkParams), C.POINTER(SweepParams), i32, vp, vp]),
     "ofdm_sweep_part2": (i32, [vp, C.POINTER(LinkParams), C.POINTER(Part2Params), vp, vp, vp]),
+    "ofdm_sweep_sync": (i32, [vp, C.POINTER(LinkParams), C.POINTER(SyncParams), vp, vp]),
     "ofdm_sweep_share": (i32, [i64, i32, i32, C.POINTER(i64), C.POINTER(i64)]),
     "ofdm_payload_bits": (i32, [vp, vp, i64, i64, u64, i64]),
     "ofdm_draw_sto_cfo": (i32, [vp, i64, u64, i64, i32, i32, vp, vp]),

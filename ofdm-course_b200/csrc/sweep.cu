@@ -238,3 +238,18 @@ extern "C" int ofdm_sweep_ber(ofdm_ctx* ctx, const ofdm_link_params* lp, const o
     cudaFreeAsync(pool, ctx->stream);
     return rc;
 }
+
+// The payload of streams g .. g + n - 1 exactly as ofdm_sweep_ber draws it (not exported; ofdm_sweep_sync uses it): Philox
+// words s into sbits, and p = DeScrambler(s) into bits when the chain scrambles (otherwise p = s and bits is not written).
+int ofdm_sweep_tile_payload(ofdm_ctx* ctx, const ofdm_link_params* lp, uint32_t* sbits, uint32_t* bits, int64_t n, int64_t words, uint64_t seed, int64_t g) {
+    int rc = ofdm_payload_bits(ctx, sbits, n, words, seed, g);
+    if (rc != OFDM_OK || !lp->scramble) return rc;
+    const int64_t frames = lp->S / lp->SpF, frame_bits = 32 * words / frames;
+    if (frame_bits >= 64) {
+        descramble_streams_kernel<<<(unsigned)cdiv64(n * words, 256), 256, 0, ctx->stream>>>(sbits, bits, n * words, (int)words, (int)frame_bits,
+                                                                                             ofdm_reg_to_prev(lp->reg0_host));
+        ctx->launches++;
+        return OFDM_OK;
+    }
+    return ofdm_descramble(ctx, sbits, bits, n * frames, frame_bits, lp->reg0_host, nullptr);
+}

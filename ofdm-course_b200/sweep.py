@@ -12,6 +12,9 @@ counters do not depend on the number of ranks.
 ``mse_sweep`` is the channel-estimation half of `Task 5/Main_model_Task_5.m:303-346` (LS / MMSE / MP / OMP MSE per stream,
 ``ofdm_sweep_mse`` in csrc/sweep_mse.cu) on the same share rule; its per-stream float64 array is summed over the ranks,
 which is exact because every cell is written by exactly one rank.
+
+``sync_sweep`` is Task 4's own study (``ofdm_sweep_sync`` in csrc/sweep_sync.cu): the synchroniser's estimates, the
+channel-estimate error and the MER of every stream of the Task-4 chain, one record per stream, reduced the same way.
 """
 from __future__ import annotations
 
@@ -164,3 +167,112 @@ def mse_sweep(ctx, lp, snrs_db, streams_per_point, taps, Ldict=None, seed=1, ran
     per, cnt = mse_sweep_local(ctx, lp, snrs_db, streams_per_point, taps, Ldict, seed, rank, world, tile, tie_eps)
     ctx.sync()
     return reduce_mse(per, cnt)                 # NCCL all-reduce on the device tensors when world > 1
+
+
+SYNC_FIELDS = ("TgPosition", "FreqOffset", "IFO", "tau", "phase_shift", "h_err", "mer_db", "nsto", "cfo")
+
+
+def channel_power(taps, Nfft, N_carrier):
+    """mean |H(k)|^2 over k = 1..N_carrier of H = fft(h, Nfft) (`get_MP_channel_resp.m:2-19`, later rows overwrite); 1 without
+    multipath.  The denominator of the NMSE that :func:`reduce_sync` reports."""
+    if taps is None or len(taps) == 0:
+        return 1.0
+    t = np.asarray(taps, dtype=np.float64).reshape(-1, 2)
+    h = np.zeros(int(t[:, 0].max()) + 1)
+    for d, a in t:
+        h[int(d)] = a
+    H = np.fft.fft(h, int(Nfft))[:int(N_carrier)]
+    return float(np.mean(np.abs(H) ** 2))
+
+
+def reduce_sync(rec, counts, h_power=1.0, sym_len=1152, cfo_tol=0.02):
+    """Sum the per-stream records (n_snr, 9, streams_per_point) float64 and the counters (n_snr, 4) int64 over all ranks -- one
+    all-reduce each, exact because every record cell is written by one rank (no-op without an initialised process group) --
+    then form the per-point statistics on the host.  Returns a dict of NumPy arrays over the SNR points, identical on every
+    rank:
+      ber, fail_rate (guard-interval detector fell back to TgPosition 65), ifo_miss_rate (IFO = -1);
+      cfo_err_mean / cfo_err_rms / cfo_within: the CFO error FreqOffset + max(IFO, 0) - cfo, and the fraction of streams with
+      |error| <= cfo_tol;
+      timing_mean / timing_std / timing_min / timing_max: the residual (nsto + TgPosition) mod sym_len;
+      h_err_mean over the non-NaN cells, h_err_nan (NaN cells), nmse = h_err_mean / h_power;
+      mer_db: mean of the finite per-stream MER values in dB;
+    plus ``rec`` and ``counts`` themselves."""
+    if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
+        dist.all_reduce(rec, op=dist.ReduceOp.SUM)
+        dist.all_reduce(counts, op=dist.ReduceOp.SUM)
+    r = rec.cpu().numpy()
+    c = counts.cpu().numpy()
+    n = r.shape[2]
+    tg, fo, ifo, herr, mer, nsto, cfo = (r[:, SYNC_FIELDS.index(f), :] for f in ("TgPosition", "FreqOffset", "IFO", "h_err", "mer_db", "nsto", "cfo"))
+    e = fo + np.maximum(ifo, 0) - cfo
+    t = np.mod(nsto + tg, sym_len)
+    ok = ~np.isnan(herr)
+    n_ok = ok.sum(axis=1)
+    h_mean = np.where(n_ok > 0, np.where(ok, herr, 0.0).sum(axis=1) / np.maximum(n_ok, 1), np.nan)
+    fin = np.isfinite(mer)
+    mer_db = np.where(fin.sum(axis=1) > 0, np.where(fin, mer, 0.0).sum(axis=1) / np.maximum(fin.sum(axis=1), 1), np.nan)
+    return {
+        "ber": c[:, 0] / np.maximum(c[:, 1], 1), "fail_rate": c[:, 2] / n, "ifo_miss_rate": c[:, 3] / n,
+        "cfo_err_mean": e.mean(axis=1), "cfo_err_rms": np.sqrt(np.mean(e ** 2, axis=1)), "cfo_within": np.mean(np.abs(e) <= cfo_tol, axis=1),
+        "timing_mean": t.mean(axis=1), "timing_std": t.std(axis=1), "timing_min": t.min(axis=1), "timing_max": t.max(axis=1),
+        "h_err_mean": h_mean, "h_err_nan": (~ok).sum(axis=1), "nmse": h_mean / h_power, "mer_db": mer_db,
+        "rec": r, "counts": c,
+    }
+
+
+def run_sync_sweep(snrs_db, streams_per_point, tile, compute, rank=0, world=1, **reduce_kw):
+    """Generic host driver of the sync sweep (used with a stand-in ``compute`` in the gloo tests).
+    ``compute(snr_index, snr_db, first_stream, n_streams) -> (rec[9, n_streams], counts[4])`` processes one tile on this rank;
+    the result is that of :func:`reduce_sync`."""
+    snrs_db = list(snrs_db)
+    rec = torch.zeros((len(snrs_db), 9, int(streams_per_point)), dtype=torch.float64)
+    counts = torch.zeros((len(snrs_db), 4), dtype=torch.int64)
+    for (i, s0, n) in tiles(len(snrs_db), streams_per_point, tile, rank, world):
+        r, c = compute(i, snrs_db[i], s0, n)
+        rec[i, :, s0:s0 + n] = torch.as_tensor(np.asarray(r, dtype=np.float64))
+        counts[i] += torch.as_tensor(np.asarray(c, dtype=np.int64))
+    return reduce_sync(rec, counts, **reduce_kw)
+
+
+def sync_sweep_local(ctx, lp, snrs_db, streams_per_point, taps=None, seed=1, rank=0, world=1, tile=0, sto=None, cfo=None, sto_max=None,
+                     cfo_int_max=30, time_desync=True, freq_desync=True, mp_desync=True, rec=None, counts=None):
+    """This rank's share of the sync sweep through ``ofdm_sweep_sync``, WITHOUT synchronising: writes its cells of ``rec``
+    (n_snr, 9, streams_per_point) float64, fields :data:`SYNC_FIELDS`, and adds to ``counts`` (n_snr, 4) int64 {bit errors,
+    bits, detector failures, IFO misses}; both are zero-initialised device tensors when not given.  With ``sto`` and ``cfo``
+    every stream gets that STO / CFO; otherwise they are drawn as :func:`sweep_local` draws them (``sto_max`` defaults to
+    Nfft + Tg)."""
+    snr = np.ascontiguousarray(np.asarray(snrs_db, dtype=np.float64))
+    sp = _cabi.SyncParams()
+    sp.n_snr = snr.size
+    sp.snr_db_host = snr.ctypes.data_as(_cabi.pdbl)
+    sp.streams_per_point = int(streams_per_point)
+    sp.tile_streams = int(tile)
+    sp.rank, sp.world = int(rank), int(world)
+    sp.seed = int(seed)
+    t = None
+    if taps is not None and len(taps):
+        t = np.ascontiguousarray(np.asarray(taps, dtype=np.float64).reshape(-1, 2))
+        sp.taps_host = t.ctypes.data_as(_cabi.pdbl)
+        sp.n_taps = t.shape[0]
+    fixed = sto is not None or cfo is not None
+    sp.sto_mode = 1 if fixed else 0
+    sp.sto_fixed = int(sto or 0)
+    sp.cfo_fixed = float(cfo or 0.0)
+    sp.sto_max = int(lp.Nfft + lp.Tg if sto_max is None else sto_max)
+    sp.cfo_int_max = int(cfo_int_max)
+    sp.time_desync, sp.freq_desync, sp.mp_desync = int(bool(time_desync)), int(bool(freq_desync)), int(bool(mp_desync))
+    if rec is None:
+        rec = torch.zeros((snr.size, 9, int(streams_per_point)), dtype=torch.float64, device=ctx.device)
+    if counts is None:
+        counts = torch.zeros((snr.size, 4), dtype=torch.int64, device=ctx.device)
+    ctx._chk(ctx.lib.ofdm_sweep_sync(ctx.h, C.byref(lp), C.byref(sp), ctx.p(rec), ctx.p(counts)))
+    return rec, counts
+
+
+def sync_sweep(ctx, lp, snrs_db, streams_per_point, taps=None, seed=1, rank=0, world=1, tile=0, cfo_tol=0.02, **kw):
+    """Whole sync sweep: this rank's call, then one all-reduce each of the records and the counters, and the per-point
+    statistics of :func:`reduce_sync` (NMSE against mean |H|^2 of ``taps``); identical on every rank and for every world
+    size and tile."""
+    rec, cnt = sync_sweep_local(ctx, lp, snrs_db, streams_per_point, taps, seed, rank, world, tile, **kw)
+    ctx.sync()
+    return reduce_sync(rec, cnt, h_power=channel_power(taps, lp.Nfft, lp.N_carrier), sym_len=lp.Nfft + lp.Tg, cfo_tol=cfo_tol)
