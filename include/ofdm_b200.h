@@ -422,6 +422,41 @@ typedef struct ofdm_sync_params {
     int32_t time_desync, freq_desync, mp_desync;   /* receiver stages, as ofdm_rx_chain_t4_ex */
 } ofdm_sync_params;
 OFDM_API int ofdm_sweep_sync(ofdm_ctx*, const ofdm_link_params*, const ofdm_sync_params*, double* rec_dev, int64_t* counts_dev);
+/* Task-2 PAPR study (`Task 2/Main_model_Task_2.m:72-82`, `Task 2/README.md:54,69-71`): calculatePAPR of every transmitted
+ * stream and the distribution of calculate_window_PAPR over all its windows, for points k = 0..n_points-1 that differ in the
+ * scrambler flag and the payload.  Work item g = k * streams_per_point + j; the call processes the share
+ * ofdm_sweep_share(n_points * streams_per_point, rank, world) gives, in tiles of tile_streams streams that never straddle a
+ * point.  Stream (k, j) is the TX chain's serial stream of L = S * (Nfft + Tg) samples for `lp` with scramble =
+ * scramble_host[k] (lp->scramble is ignored); no channel is applied.  The payload depends on j only, not on k, so a plain
+ * and a scrambled point with the same p_one (or the same pool) transmit the same payloads -- a paired comparison:
+ *   - Bernoulli (pool_host NULL): bit i of stream j is 1 iff u_i < floor(p_one_host[k] * 2^32), u_i = word i mod 4 of
+ *     Philox4x32-10 at counter (i / 4, j) in a key space of its own -- the bits ofdm_payload_bernoulli writes;
+ *   - pool: bit i of stream j is pool bit (j * pool_stride + i) mod pool_bits (packed, the library's bit layout).
+ * papr_dev: n_points x streams_per_point doubles, [k][j] = calculatePAPR of the whole serial stream, cyclic prefixes included
+ * (`calculatePAPR.m:2-11`); only this call's share is written.
+ * hist_dev: n_points x n_bins int64, ADDED to (+=): every window of calculate_window_PAPR(x, Nfft) (length Nfft, step 1, L - Nfft
+ * + 1 per stream), with v its value rounded to the context's real type exactly as ofdm_window_papr returns it, counts in bin
+ * min(floor((double)v / bin_db), n_bins - 1); negative v (rounding) and NaN (an all-zero window) count in bin 0.  The CCDF at
+ * edge b * bin_db -- the fraction of windows with bin >= b -- is therefore exact; ofdm_ccdf gives the exact ecdf of stored values.
+ * The values do not depend on the rank count or the tile size; the caller sums both arrays over ranks (each PAPR cell is
+ * written by one rank, the histogram is integer).  FP32 and FP64 contexts, any power-of-two Nfft of the TX chain;
+ * OFDM_ERR_UNSUPPORTED when the statistics kernel's shared memory (2 Nfft (8 + sizeof(real)) + 4 n_bins bytes) exceeds the
+ * device's limit per block (FP64 at Nfft 8192). */
+typedef struct ofdm_papr_params {
+    int32_t n_points;
+    const int32_t* scramble_host;   /* n_points: 0 plain, 1 Scrambler with per-frame reset from lp->reg0_host */
+    const double* p_one_host;       /* n_points: P(bit = 1) of the Philox payload, 0 < p < 1; ignored when pool_host is set */
+    const uint32_t* pool_host;      /* optional packed payload pool (library bit layout), e.g. file_reader('eagle.tiff') */
+    int64_t pool_bits;              /* 1 .. 2^32 when pool_host is set */
+    int64_t pool_stride;            /* >= 0: stream j reads pool bits (j * pool_stride + i) mod pool_bits, i = 0 .. stream_bits-1 */
+    int64_t streams_per_point;
+    int64_t tile_streams;           /* 0 = 8192 (one signal buffer of tile x L complex samples is allocated) */
+    int32_t rank, world;
+    uint64_t seed;
+    double bin_db;                  /* histogram bin width in dB, > 0 */
+    int32_t n_bins;                 /* 1 .. 16384; the last bin also takes everything above it */
+} ofdm_papr_params;
+OFDM_API int ofdm_sweep_papr(ofdm_ctx*, const ofdm_link_params*, const ofdm_papr_params*, double* papr_dev, int64_t* hist_dev);
 /* first / count of the contiguous share of `total_streams` that (rank, world) processes */
 OFDM_API int ofdm_sweep_share(int64_t total_streams, int rank, int world, int64_t* first, int64_t* count);
 /* The sweep's synthetic inputs, also usable on their own: payload words of streams first_stream_id .. +n_streams-1
@@ -430,6 +465,12 @@ OFDM_API int ofdm_payload_bits(ofdm_ctx*, uint32_t* bits_dev, int64_t n_streams,
                                int64_t first_stream_id);
 OFDM_API int ofdm_draw_sto_cfo(ofdm_ctx*, int64_t B, uint64_t seed, int64_t first_stream_id, int sto_max, int cfo_int_max,
                                int32_t* nsto_dev, double* cfo_dev);
+/* The Bernoulli payload of ofdm_sweep_papr: streams first_stream_id .. +n_streams-1 of stream_bits bits each (any length,
+ * not padded to words) as ONE contiguous bitstream, the input ofdm_tx_chain takes; OFDM_BIT_WORDS(n_streams * stream_bits)
+ * words are written and the bits past the last stream are 0.  Bit i of stream j is 1 iff u_i < floor(p_one * 2^32), u_i =
+ * word i mod 4 of Philox4x32-10 at counter (i / 4, j) in a key space of its own; 0 < p_one < 1. */
+OFDM_API int ofdm_payload_bernoulli(ofdm_ctx*, uint32_t* bits_dev, int64_t n_streams, int64_t stream_bits, double p_one,
+                                    uint64_t seed, int64_t first_stream_id);
 
 #ifdef __cplusplus
 }

@@ -741,6 +741,52 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
         mxArray* cm = mxCreateDoubleMatrix(n, 4, mxREAL);
         for (i = 0; i < n; ++i) { int j; for (j = 0; j < 4; ++j) real_data(cm)[(size_t)j * n + i] = (double)ch[4 * i + j]; }
         OUT(1, cm);
+    } else if (!strcmp(op, "sweep_papr")) {   /* [hist (n_bins x n_points), PAPR (spp x n_points)] =
+                                                 sweep_papr(LINK..., scramble, p_one, streams_per_point, seed, bin_db, n_bins, pool, pool_stride):
+                                                 scramble / p_one one entry per point (p_one ignored with a pool); pool = 0/1 payload
+                                                 bits (e.g. file_reader's) or [] for the Philox Bernoulli payload; hist counts the
+                                                 window PAPR values in bins of bin_db dB, the last bin takes everything above it */
+        NEED(N_LINK + 8);
+        ofdm_link_params lp;
+        ofdm_papr_params pp;
+        parse_link(&A(0), &lp);
+        memset(&pp, 0, sizeof pp);
+        size_t n = mxGetNumberOfElements(A(N_LINK)), i;
+        if (!n) fail("ofdm:sweep_papr:points", "need at least one point");
+        size_t npool = mxGetNumberOfElements(A(N_LINK + 6));
+        if (!npool && mxGetNumberOfElements(A(N_LINK + 1)) != n) fail("ofdm:sweep_papr:p_one", "p_one must have one entry per point");
+        int32_t* scr = (int32_t*)hostbuf(n * 4);
+        for (i = 0; i < n; ++i) scr[i] = real_data(A(N_LINK))[i] != 0.0;
+        pp.n_points = (int32_t)n;
+        pp.scramble_host = scr;
+        pp.p_one_host = npool ? NULL : real_data(A(N_LINK + 1));
+        if (npool) {
+            uint32_t* pw = (uint32_t*)hostbuf(OFDM_BIT_WORDS(npool) * 4);
+            const double* pb = real_data(A(N_LINK + 6));
+            for (i = 0; i < npool; ++i) if (pb[i] != 0.0) pw[i >> 5] |= 1u << (i & 31);
+            pp.pool_host = pw;
+            pp.pool_bits = (int64_t)npool;
+            pp.pool_stride = (int64_t)mxGetScalar(A(N_LINK + 7));
+        }
+        pp.streams_per_point = (int64_t)mxGetScalar(A(N_LINK + 2));
+        pp.rank = 0; pp.world = 1;
+        pp.seed = (uint64_t)mxGetScalar(A(N_LINK + 3));
+        pp.bin_db = mxGetScalar(A(N_LINK + 4));
+        pp.n_bins = (int32_t)mxGetScalar(A(N_LINK + 5));
+        size_t spp = (size_t)(pp.streams_per_point > 0 ? pp.streams_per_point : 0), nb = (size_t)(pp.n_bins > 0 ? pp.n_bins : 0);
+        double* pd = (double*)devbuf(n * spp * 8 + 8);
+        int64_t* hd = (int64_t*)devbuf(n * nb * 8 + 8);
+        int64_t* hh = (int64_t*)hostbuf(n * nb * 8 + 8);
+        chk(ofdm_memset(g_ctx, pd, 0, n * spp * 8), "memset");
+        chk(ofdm_memset(g_ctx, hd, 0, n * nb * 8), "memset");
+        chk(ofdm_sweep_papr(g_ctx, &lp, &pp, pd, hd), op);
+        mxArray* hm = mxCreateDoubleMatrix(nb, n, mxREAL);
+        chk(ofdm_d2h(g_ctx, hh, hd, n * nb * 8), "d2h");
+        for (i = 0; i < n * nb; ++i) real_data(hm)[i] = (double)hh[i];
+        OUT(0, hm);
+        mxArray* pm = mxCreateDoubleMatrix(spp, n, mxREAL);
+        chk(ofdm_d2h(g_ctx, real_data(pm), pd, n * spp * 8), "d2h");
+        OUT(1, pm);
     } else if (!strcmp(op, "sweep_part2")) {   /* [NMSE (4 x n_points), BER (4 x n_points), per_run (mc_runs x 4*n_points), counts (12 x n_points),
                                                    runs (2 x n_points)] = sweep_part2(Nfft, T_Guard, N_carrier, N_symb, SpF, Constellation,
                                                    pilots, offsets, Ldict, pattern, bits, profile, fs, SNR, monteCarloRuns, seed, near_eps, tie_eps):

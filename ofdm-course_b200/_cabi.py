@@ -49,6 +49,13 @@ class SyncParams(C.Structure):
                 ("cfo_fixed", C.c_double), ("time_desync", C.c_int32), ("freq_desync", C.c_int32), ("mp_desync", C.c_int32)]
 
 
+class PaprParams(C.Structure):
+    """``ofdm_papr_params`` of include/ofdm_b200.h."""
+    _fields_ = [("n_points", C.c_int32), ("scramble_host", pi32), ("p_one_host", pdbl), ("pool_host", C.POINTER(C.c_uint32)),
+                ("pool_bits", C.c_int64), ("pool_stride", C.c_int64), ("streams_per_point", C.c_int64), ("tile_streams", C.c_int64),
+                ("rank", C.c_int32), ("world", C.c_int32), ("seed", C.c_uint64), ("bin_db", C.c_double), ("n_bins", C.c_int32)]
+
+
 # name -> (restype, argtypes); every symbol declared in include/ofdm_b200.h
 SIGNATURES = {
     "ofdm_ctx_create": (i32, [C.POINTER(vp), i32, i32]),
@@ -115,9 +122,11 @@ SIGNATURES = {
     "ofdm_sweep_mse": (i32, [vp, C.POINTER(LinkParams), C.POINTER(SweepParams), i32, vp, vp]),
     "ofdm_sweep_part2": (i32, [vp, C.POINTER(LinkParams), C.POINTER(Part2Params), vp, vp, vp]),
     "ofdm_sweep_sync": (i32, [vp, C.POINTER(LinkParams), C.POINTER(SyncParams), vp, vp]),
+    "ofdm_sweep_papr": (i32, [vp, C.POINTER(LinkParams), C.POINTER(PaprParams), vp, vp]),
     "ofdm_sweep_share": (i32, [i64, i32, i32, C.POINTER(i64), C.POINTER(i64)]),
     "ofdm_payload_bits": (i32, [vp, vp, i64, i64, u64, i64]),
     "ofdm_draw_sto_cfo": (i32, [vp, i64, u64, i64, i32, i32, vp, vp]),
+    "ofdm_payload_bernoulli": (i32, [vp, vp, i64, i64, dbl, u64, i64]),
     "ofdm_rx_chain_t4_ex": (i32, [vp, C.POINTER(LinkParams), vp, i64, i32, i32, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, dbl, vp]),
 }
 

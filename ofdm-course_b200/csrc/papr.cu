@@ -32,10 +32,47 @@ __global__ void papr_kernel(const cx<T>* __restrict__ x, int64_t L, double* __re
     }
 }
 
+// One half of the block scan of a window block, shared by window_papr_kernel and papr_stats_kernel so that both sum in
+// the same order: half 0 turns ssum / smax[0, W) into suffix (sum, max) scans (runs walk right to left), half 1 turns
+// [W, 2W) into prefix scans.  Each thread owns a run of `per` consecutive entries; run totals are combined with a warp
+// scan per warp and a serial pass over the warp totals.  Ends with a barrier.
+template <typename T>
+__device__ __forceinline__ void window_scan_half(double* ssum, T* smax, int W, int per, int half, int tid, int lane, int warp,
+                                                 double (*wsum)[PAPR_THREADS / 32], T (*wmax)[PAPR_THREADS / 32]) {
+    const int lo = tid * per, hi = min(lo + per, W);
+    double s = 0; T m = 0;
+    if (half == 0) { for (int j = hi - 1; j >= lo; --j) { s += ssum[j]; m = max(m, smax[j]); ssum[j] = s; smax[j] = m; } }
+    else { for (int j = lo; j < hi; ++j) { s += ssum[W + j]; m = max(m, smax[W + j]); ssum[W + j] = s; smax[W + j] = m; } }
+    // exclusive combination of the run totals: runs to the right (half 0) / to the left (half 1)
+    double es = s; T em = m;
+    for (int o = 1; o < 32; o <<= 1) {
+        const double ts = half == 0 ? __shfl_down_sync(0xffffffffu, es, o) : __shfl_up_sync(0xffffffffu, es, o);
+        const T tm = half == 0 ? __shfl_down_sync(0xffffffffu, em, o) : __shfl_up_sync(0xffffffffu, em, o);
+        const bool ok = half == 0 ? (lane + o < 32) : (lane >= o);
+        if (ok) { es += ts; em = max(em, tm); }
+    }
+    const int edge = half == 0 ? 0 : 31;          // lane holding the warp total
+    if (lane == edge) { wsum[half][warp] = es; wmax[half][warp] = em; }
+    __syncthreads();
+    double cs = 0; T cm = 0;                       // totals of the warps further right / left
+    if (half == 0) { for (int w = warp + 1; w < PAPR_THREADS / 32; ++w) { cs += wsum[0][w]; cm = max(cm, wmax[0][w]); } }
+    else { for (int w = 0; w < warp; ++w) { cs += wsum[1][w]; cm = max(cm, wmax[1][w]); } }
+    // carry = (inclusive warp scan - own run) + other warps
+    const double carry_s = es - s + cs;
+    T carry_m = cm;
+    {   // maximum has no inverse: redo the exclusive part from the neighbours' inclusive values
+        const T nb = half == 0 ? __shfl_down_sync(0xffffffffu, em, 1) : __shfl_up_sync(0xffffffffu, em, 1);
+        const bool ok = half == 0 ? (lane < 31) : (lane > 0);
+        if (ok) carry_m = max(carry_m, nb);
+    }
+    if (half == 0) { for (int j = lo; j < hi; ++j) { ssum[j] += carry_s; smax[j] = max(smax[j], carry_m); } }
+    else { for (int j = lo; j < hi; ++j) { ssum[W + j] += carry_s; smax[W + j] = max(smax[W + j], carry_m); } }
+    __syncthreads();
+}
+
 // ---- calculate_window_PAPR
 // One CTA produces the W outputs i = kW .. kW+W-1 of one stream.  Shared memory: power p[0..2W), then in place
-// suffix (max, sum) over [0, W) and prefix (max, sum) over [W, 2W).  Each thread owns a run of `per` consecutive
-// entries; run totals are combined with a warp scan per warp and a serial pass over the warp totals.
+// suffix (max, sum) over [0, W) and prefix (max, sum) over [W, 2W) (window_scan_half).
 template <typename T>
 __global__ void __launch_bounds__(PAPR_THREADS) window_papr_kernel(const cx<T>* __restrict__ x, int64_t L, int W, int64_t n_out, T* __restrict__ out) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -55,39 +92,9 @@ __global__ void __launch_bounds__(PAPR_THREADS) window_papr_kernel(const cx<T>* 
     }
     __syncthreads();
     const int per = (W + PAPR_THREADS - 1) / PAPR_THREADS;
-    // half 0: suffix scan over [0, W) (runs walk right to left); half 1: prefix scan over [W, 2W)
+    // half 0: suffix scan over [0, W); half 1: prefix scan over [W, 2W)
 #pragma unroll
-    for (int half = 0; half < 2; ++half) {
-        const int lo = tid * per, hi = min(lo + per, W);
-        double s = 0; T m = 0;
-        if (half == 0) { for (int j = hi - 1; j >= lo; --j) { s += ssum[j]; m = max(m, smax[j]); ssum[j] = s; smax[j] = m; } }
-        else { for (int j = lo; j < hi; ++j) { s += ssum[W + j]; m = max(m, smax[W + j]); ssum[W + j] = s; smax[W + j] = m; } }
-        // exclusive combination of the run totals: runs to the right (half 0) / to the left (half 1)
-        double es = s; T em = m;
-        for (int o = 1; o < 32; o <<= 1) {
-            const double ts = half == 0 ? __shfl_down_sync(0xffffffffu, es, o) : __shfl_up_sync(0xffffffffu, es, o);
-            const T tm = half == 0 ? __shfl_down_sync(0xffffffffu, em, o) : __shfl_up_sync(0xffffffffu, em, o);
-            const bool ok = half == 0 ? (lane + o < 32) : (lane >= o);
-            if (ok) { es += ts; em = max(em, tm); }
-        }
-        const int edge = half == 0 ? 0 : 31;          // lane holding the warp total
-        if (lane == edge) { wsum[half][warp] = es; wmax[half][warp] = em; }
-        __syncthreads();
-        double cs = 0; T cm = 0;                       // totals of the warps further right / left
-        if (half == 0) { for (int w = warp + 1; w < PAPR_THREADS / 32; ++w) { cs += wsum[0][w]; cm = max(cm, wmax[0][w]); } }
-        else { for (int w = 0; w < warp; ++w) { cs += wsum[1][w]; cm = max(cm, wmax[1][w]); } }
-        // carry = (inclusive warp scan - own run) + other warps
-        const double carry_s = es - s + cs;
-        T carry_m = cm;
-        {   // maximum has no inverse: redo the exclusive part from the neighbours' inclusive values
-            const T nb = half == 0 ? __shfl_down_sync(0xffffffffu, em, 1) : __shfl_up_sync(0xffffffffu, em, 1);
-            const bool ok = half == 0 ? (lane < 31) : (lane > 0);
-            if (ok) carry_m = max(carry_m, nb);
-        }
-        if (half == 0) { for (int j = lo; j < hi; ++j) { ssum[j] += carry_s; smax[j] = max(smax[j], carry_m); } }
-        else { for (int j = lo; j < hi; ++j) { ssum[W + j] += carry_s; smax[W + j] = max(smax[W + j], carry_m); } }
-        __syncthreads();
-    }
+    for (int half = 0; half < 2; ++half) window_scan_half<T>(ssum, smax, W, per, half, tid, lane, warp, wsum, wmax);
     for (int j = tid; j < W; j += PAPR_THREADS) {
         const int64_t i = i0 + j;
         if (i < n_out) {
@@ -119,6 +126,180 @@ extern "C" int ofdm_window_papr(ofdm_ctx* ctx, const void* x, int64_t B, int64_t
         if (smem > 48 * 1024) CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         k<<<dim3((unsigned)B, (unsigned)cdiv64(n_out, W)), PAPR_THREADS, smem, ctx->stream>>>((const cx<T>*)x, L, W, n_out, (T*)paprs);
     });
+    LAUNCH_CHECK(ctx);
+    return OFDM_OK;
+}
+
+// ---- PAPR statistics of a study (ofdm_sweep_papr, csrc/sweep_papr.cu) without storing a window value
+// One CTA walks the window blocks [k0, k1) of one stream (a chunk; a whole stream unless the batch is too small to fill the
+// GPU) and so reads data blocks k0 .. k1, each sample once (a chunk re-reads the first block of the next one).  Arithmetic
+// and layout are window_papr_kernel's, so every window value is bit-identical to ofdm_window_papr's: block k is
+// prefix-scanned in [W, 2W) while the suffix scan of block k-1 waits in [0, W), the windows starting in block k-1 are
+// evaluated from both, then block k is suffix-scanned in [0, W).  The samples of block k+1 are loaded into registers at
+// the top of iteration k and used at its end.  Every window value v goes to bin min(floor(v / bin_db), n_bins - 1) of a
+// shared int32 histogram (negative values from rounding and NaN, an all-zero window, to bin 0), flushed once per CTA into
+// the point's int64 row with integer atomics.  max |x|^2 of the stream is combined over chunks as the bit pattern of a
+// non-negative double (unsigned max orders those as the values).
+__device__ __forceinline__ float window_power(float2 v) { return __fmaf_rn(v.x, v.x, __fmul_rn(v.y, v.y)); }   // as window_papr_kernel's
+__device__ __forceinline__ double window_power(double2 v) { return __fma_rn(v.x, v.x, __dmul_rn(v.y, v.y)); }  // contracted p
+
+template <typename T, int PER>
+__global__ void __launch_bounds__(PAPR_THREADS) papr_stats_kernel(const cx<T>* __restrict__ x, int64_t L, int W, int64_t n_out, int64_t nbw,
+                                                                  int64_t chunk, int chunks, double bin_db, int n_bins,
+                                                                  unsigned long long* __restrict__ hist, unsigned long long* __restrict__ peak) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    double* ssum = (double*)smem_raw;                 // [0, W): suffix scan of the previous block; [W, 2W): prefix scan of this one
+    T* smax = (T*)(ssum + 2 * (size_t)W);
+    int* h = (int*)(smax + 2 * (size_t)W);            // n_bins counters
+    __shared__ double wsum[2][PAPR_THREADS / 32];
+    __shared__ T wmax[2][PAPR_THREADS / 32];
+    __shared__ double red[PAPR_THREADS / 32];
+    const int64_t b = blockIdx.x / chunks;
+    const int64_t k0 = (int64_t)(blockIdx.x % chunks) * chunk, k1 = min(k0 + chunk, nbw);
+    const cx<T>* r = x + b * L;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int per = (W + PAPR_THREADS - 1) / PAPR_THREADS;
+    for (int i = tid; i < n_bins; i += PAPR_THREADS) h[i] = 0;
+    cx<T> nx[PER];                                    // samples of the next block, in flight
+    T pw[PER];                                        // |x|^2 of this block's samples tid + m * PAPR_THREADS
+    double pk = 0;
+    auto load = [&](int64_t k) {
+#pragma unroll
+        for (int m = 0; m < PER; ++m) {
+            const int j = tid + m * PAPR_THREADS;
+            const int64_t n = k * W + j;
+            nx[m] = mk<T>(0, 0);
+            if (j < W && n < L) nx[m] = r[n];
+        }
+    };
+    auto power = [&]() {
+#pragma unroll
+        for (int m = 0; m < PER; ++m) {
+            pw[m] = window_power(nx[m]);
+            pk = fmax(pk, (double)nx[m].x * (double)nx[m].x + (double)nx[m].y * (double)nx[m].y);   // as papr_kernel
+        }
+    };
+    auto store = [&](int off) {
+#pragma unroll
+        for (int m = 0; m < PER; ++m) {
+            const int j = tid + m * PAPR_THREADS;
+            if (j < W) { ssum[off + j] = (double)pw[m]; smax[off + j] = pw[m]; }
+        }
+    };
+    load(k0);
+    power();
+    for (int64_t k = k0; k <= k1; ++k) {
+        if (k < k1) load(k + 1);
+        if (k > k0) {
+            store(W);
+            __syncthreads();
+            window_scan_half<T>(ssum, smax, W, per, 1, tid, lane, warp, wsum, wmax);
+            // the windows starting in block k-1, a run of consecutive ones per thread: equal bins are counted once per run
+            const int lo = tid * per, hi = min(lo + per, W);
+            int run_bin = 0, run_n = 0;
+            for (int j = lo; j < hi; ++j) {
+                if ((k - 1) * W + j >= n_out) break;
+                double s = ssum[j]; T m = smax[j];
+                if (j > 0) { s += ssum[W + j - 1]; m = max(m, smax[W + j - 1]); }
+                const T v = (T)(10.0 * log10((double)m / (s / (double)W)));
+                const double q = floor((double)v / bin_db);
+                const int bin = q >= (double)(n_bins - 1) ? n_bins - 1 : (q > 0 ? (int)q : 0);
+                if (bin != run_bin && run_n) { atomicAdd(&h[run_bin], run_n); run_n = 0; }
+                run_bin = bin;
+                ++run_n;
+            }
+            if (run_n) atomicAdd(&h[run_bin], run_n);
+            __syncthreads();
+        }
+        if (k < k1) {
+            store(0);
+            __syncthreads();
+            window_scan_half<T>(ssum, smax, W, per, 0, tid, lane, warp, wsum, wmax);
+            power();
+        }
+    }
+    __syncthreads();
+    for (int i = tid; i < n_bins; i += PAPR_THREADS) {
+        const int c = h[i];
+        if (c) atomicAdd(&hist[i], (unsigned long long)c);
+    }
+    for (int o = 16; o > 0; o >>= 1) pk = fmax(pk, __shfl_xor_sync(0xffffffffu, pk, o));
+    if (lane == 0) red[warp] = pk;
+    __syncthreads();
+    if (tid == 0) {
+        double m = 0;
+        for (int w = 0; w < PAPR_THREADS / 32; ++w) m = fmax(m, red[w]);
+        atomicMax(&peak[b], (unsigned long long)__double_as_longlong(m));
+    }
+}
+
+// calculatePAPR from the combined maximum and the stream power sum of ofdm_tx_chain_p
+__global__ void papr_finish_kernel(const unsigned long long* __restrict__ peak, const double* __restrict__ psum, int64_t B, int64_t L, double* __restrict__ out) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < B) out[i] = 10.0 * log10(__longlong_as_double((long long)peak[i]) / (psum[i] / (double)L));
+}
+
+template <typename T> static const void* papr_stats_kernel_for(int W) {
+    switch ((W + PAPR_THREADS - 1) / PAPR_THREADS) {
+    case 1: return (const void*)papr_stats_kernel<T, 1>;
+    case 2: return (const void*)papr_stats_kernel<T, 2>;
+    case 4: return (const void*)papr_stats_kernel<T, 4>;
+    case 8: return (const void*)papr_stats_kernel<T, 8>;
+    case 16: return (const void*)papr_stats_kernel<T, 16>;
+    case 32:
+        if constexpr (sizeof(T) == 4) return (const void*)papr_stats_kernel<T, 32>;   // FP64 at W = 8192 needs 256 KB of shared memory
+        else return nullptr;
+    default: return nullptr;
+    }
+}
+
+static size_t papr_stats_smem(int precision, int W, int n_bins) {
+    return 2 * (size_t)W * (sizeof(double) + (precision == OFDM_PREC_F64 ? sizeof(double) : sizeof(float))) + sizeof(int) * (size_t)n_bins;
+}
+
+// OFDM_OK when the statistics kernel runs at window length W (a power of two) with n_bins bins on the context's device,
+// OFDM_ERR_UNSUPPORTED (with its own message) when its shared memory exceeds the device's opt-in limit per block.
+int ofdm_papr_stats_check(ofdm_ctx* ctx, int W, int n_bins, const char* who) {
+    const void* k = ctx->precision == OFDM_PREC_F64 ? papr_stats_kernel_for<double>(W) : papr_stats_kernel_for<float>(W);
+    const size_t dyn = papr_stats_smem(ctx->precision, W, n_bins);
+    int optin = 0;
+    CUDA_TRY(ctx, cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, ctx->device));
+    size_t stat = 0;
+    if (k) {
+        cudaFuncAttributes a;
+        CUDA_TRY(ctx, cudaFuncGetAttributes(&a, k));
+        stat = a.sharedSizeBytes;
+    }
+    if (!k || dyn + stat > (size_t)optin)
+        return ctx_fail(ctx, OFDM_ERR_UNSUPPORTED, "%s: the PAPR statistics kernel needs %zu B of shared memory per block at Nfft %d with %d bins in %s, "
+                        "above this device's limit of %d B (use fewer bins or an FP32 context)", who, dyn + stat, W, n_bins,
+                        ctx->precision == OFDM_PREC_F64 ? "FP64" : "FP32", optin);
+    return OFDM_OK;
+}
+
+// Histogram (+= into hist, n_bins int64) and per-stream PAPR (papr, B doubles) of B streams of L samples at window length W;
+// psum: sum |x|^2 per stream (ofdm_tx_chain_p); peak: B scratch words.  ofdm_papr_stats_check must have passed.
+int ofdm_papr_stats(ofdm_ctx* ctx, const void* x, int64_t B, int64_t L, int W, const double* psum, double bin_db, int n_bins, int64_t* hist,
+                    double* papr, unsigned long long* peak) {
+    const void* k = ctx->precision == OFDM_PREC_F64 ? papr_stats_kernel_for<double>(W) : papr_stats_kernel_for<float>(W);
+    REQUIRE(ctx, k != nullptr, "no statistics kernel for this window length");
+    const size_t smem = papr_stats_smem(ctx->precision, W, n_bins);
+    CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    int per_sm = 0;
+    CUDA_TRY(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k, PAPR_THREADS, smem));
+    int64_t n_out = L - W + 1, nbw = cdiv64(n_out, W);
+    // two waves of CTAs at least; a chunk spans 8 window blocks or more, so the block it re-reads costs at most 1/8
+    int64_t chunks = std::min<int64_t>(std::max<int64_t>(1, cdiv64(2 * (int64_t)std::max(per_sm, 1) * ctx->sm_count, B)), std::max<int64_t>(1, nbw / 8));
+    int64_t chunk = cdiv64(nbw, chunks);
+    chunks = cdiv64(nbw, chunk);
+    REQUIRE(ctx, B * chunks < ((int64_t)1 << 31), "too many streams in one tile");
+    CUDA_TRY(ctx, cudaMemsetAsync(peak, 0, sizeof(unsigned long long) * (size_t)B, ctx->stream));
+    int ichunks = (int)chunks;
+    unsigned long long* h = (unsigned long long*)hist;
+    void* args[] = {(void*)&x, &L, &W, &n_out, &nbw, &chunk, &ichunks, &bin_db, &n_bins, &h, &peak};
+    CUDA_TRY(ctx, cudaLaunchKernel(k, dim3((unsigned)(B * chunks)), dim3(PAPR_THREADS), args, smem, ctx->stream));
+    ctx->launches++;
+    papr_finish_kernel<<<(unsigned)cdiv64(B, 256), 256, 0, ctx->stream>>>(peak, psum, B, L, papr);
     LAUNCH_CHECK(ctx);
     return OFDM_OK;
 }

@@ -451,6 +451,13 @@ class Context:
         k = int(cnt.item())
         return xs[:k], cc[:k]
 
+    def payload_bernoulli(self, n_streams, stream_bits, p_one, seed=1, first_stream_id=0):
+        """The Bernoulli payload of ``ofdm_sweep_papr``: streams first_stream_id .. + n_streams - 1 of stream_bits bits as one
+        contiguous packed bitstream (int32 words, the input of :meth:`tx_chain`)."""
+        out = torch.empty(((int(n_streams) * int(stream_bits) + 31) // 32,), dtype=torch.int32, device=self.device)
+        self._chk(self.lib.ofdm_payload_bernoulli(self.h, self.p(out), int(n_streams), int(stream_bits), float(p_one), int(seed), int(first_stream_id)))
+        return out
+
     # ---------------------------------------------------------------- fused chains
     def tx_chain(self, lp, bits_dev, B, want_power=False):
         """TX chain; with ``want_power`` also returns sum |x|^2 per stream (float64, B) for ``channel_t5(power_sum=...)``."""

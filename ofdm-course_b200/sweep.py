@@ -15,6 +15,9 @@ which is exact because every cell is written by exactly one rank.
 
 ``sync_sweep`` is Task 4's own study (``ofdm_sweep_sync`` in csrc/sweep_sync.cu): the synchroniser's estimates, the
 channel-estimate error and the MER of every stream of the Task-4 chain, one record per stream, reduced the same way.
+
+``papr_sweep`` is Task 2's study (``ofdm_sweep_papr`` in csrc/sweep_papr.cu): the PAPR of every transmitted stream and an
+integer histogram of the PAPR of all its Nfft-sample windows, plain against scrambled, one all-reduce each.
 """
 from __future__ import annotations
 
@@ -276,3 +279,91 @@ def sync_sweep(ctx, lp, snrs_db, streams_per_point, taps=None, seed=1, rank=0, w
     rec, cnt = sync_sweep_local(ctx, lp, snrs_db, streams_per_point, taps, seed, rank, world, tile, **kw)
     ctx.sync()
     return reduce_sync(rec, cnt, h_power=channel_power(taps, lp.Nfft, lp.N_carrier), sym_len=lp.Nfft + lp.Tg, cfo_tol=cfo_tol)
+
+
+def papr_sweep_local(ctx, lp, points, streams_per_point, seed=1, rank=0, world=1, tile=0, bin_db=0.01, n_bins=4000, pool=None, pool_stride=0,
+                     hist=None, papr=None):
+    """This rank's share of the PAPR study through ``ofdm_sweep_papr``, WITHOUT synchronising.  ``points``: a list of
+    ``(scramble, p_one)``; ``p_one`` is P(bit = 1) of the Philox payload and is ignored when ``pool`` (0/1 payload bits, e.g.
+    ``realisations.file_reader``) is given: stream j then transmits pool bits (j * pool_stride + i) mod len(pool).  Writes
+    its cells of ``papr`` (n_points, streams_per_point) float64 and adds to ``hist`` (n_points, n_bins) int64, window
+    PAPR v in bin min(floor(v / bin_db), n_bins - 1); both are zero-initialised device tensors when not given."""
+    pts = [(int(bool(s)), p) for s, p in points]
+    scr = np.ascontiguousarray(np.array([s for s, _ in pts], dtype=np.int32))
+    pone = np.ascontiguousarray(np.array([0.5 if p is None else float(p) for _, p in pts], dtype=np.float64))
+    pp = _cabi.PaprParams()
+    pp.n_points = len(pts)
+    pp.scramble_host = scr.ctypes.data_as(_cabi.pi32)
+    pp.p_one_host = pone.ctypes.data_as(_cabi.pdbl)
+    words = None
+    if pool is not None:
+        bits = np.asarray(pool).ravel()
+        words = np.ascontiguousarray(np.packbits(bits.astype(np.uint8), bitorder="little"))
+        words = np.concatenate([words, np.zeros((-words.size) % 4, dtype=np.uint8)]).view(np.uint32)
+        pp.pool_host = words.ctypes.data_as(C.POINTER(C.c_uint32))
+        pp.pool_bits = int(bits.size)
+        pp.pool_stride = int(pool_stride)
+    pp.streams_per_point = int(streams_per_point)
+    pp.tile_streams = int(tile)
+    pp.rank, pp.world = int(rank), int(world)
+    pp.seed = int(seed)
+    pp.bin_db = float(bin_db)
+    pp.n_bins = int(n_bins)
+    if hist is None:
+        hist = torch.zeros((len(pts), int(n_bins)), dtype=torch.int64, device=ctx.device)
+    if papr is None:
+        papr = torch.zeros((len(pts), int(streams_per_point)), dtype=torch.float64, device=ctx.device)
+    ctx._chk(ctx.lib.ofdm_sweep_papr(ctx.h, C.byref(lp), C.byref(pp), ctx.p(papr), ctx.p(hist)))
+    return hist, papr
+
+
+def papr_ccdf(hist):
+    """CCDF at the bin edges b * bin_db of an (n_points, n_bins) or (n_bins,) histogram: the fraction of windows whose bin is
+    >= b, i.e. P(PAPR >= b * bin_db) (exact at the edges; the last bin holds everything above its edge)."""
+    h = np.asarray(hist, dtype=np.int64)
+    tail = np.cumsum(h[..., ::-1], axis=-1)[..., ::-1]
+    return tail / np.maximum(tail[..., :1], 1)
+
+
+def papr_exceedance(hist, bin_db, prob):
+    """The smallest bin edge whose CCDF is <= prob -- the PAPR "exceeded with probability prob" that `Task 2/README.md:69-71`
+    reads off calculateCCDF's curve, to within one bin above it.  One value per point of an (n_points, n_bins) histogram."""
+    c = papr_ccdf(hist)
+    below = c <= prob
+    idx = np.where(below.any(axis=-1), below.argmax(axis=-1), c.shape[-1])
+    return idx * float(bin_db)
+
+
+def reduce_papr(hist, papr, bin_db=0.01):
+    """Sum the histogram (n_points, n_bins) int64 and the per-stream PAPR (n_points, streams_per_point) float64 over all
+    ranks -- one all-reduce each, exact because the histogram is integer and every PAPR cell is written by one rank (no-op
+    without an initialised process group).  Returns a dict of NumPy arrays, identical on every rank: ``hist``, ``edges``
+    (b * bin_db), ``ccdf`` at the edges (:func:`papr_ccdf`), ``papr`` and its mean per point ``papr_mean``."""
+    if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
+        dist.all_reduce(hist, op=dist.ReduceOp.SUM)
+        dist.all_reduce(papr, op=dist.ReduceOp.SUM)
+    h = hist.cpu().numpy()
+    p = papr.cpu().numpy()
+    return {"hist": h, "edges": np.arange(h.shape[-1]) * float(bin_db), "ccdf": papr_ccdf(h), "papr": p, "papr_mean": p.mean(axis=-1)}
+
+
+def run_papr_sweep(points, streams_per_point, tile, compute, rank=0, world=1, n_bins=4000, bin_db=0.01):
+    """Generic host driver of the PAPR study (used with a stand-in ``compute`` in the gloo tests).
+    ``compute(point_index, point, first_stream, n_streams) -> (hist[n_bins], papr[n_streams])`` processes one tile on this
+    rank; the result is that of :func:`reduce_papr`."""
+    points = list(points)
+    hist = torch.zeros((len(points), int(n_bins)), dtype=torch.int64)
+    papr = torch.zeros((len(points), int(streams_per_point)), dtype=torch.float64)
+    for (k, s0, n) in tiles(len(points), streams_per_point, tile, rank, world):
+        h, p = compute(k, points[k], s0, n)
+        hist[k] += torch.as_tensor(np.asarray(h, dtype=np.int64))
+        papr[k, s0:s0 + n] = torch.as_tensor(np.asarray(p, dtype=np.float64))
+    return reduce_papr(hist, papr, bin_db)
+
+
+def papr_sweep(ctx, lp, points, streams_per_point, seed=1, rank=0, world=1, tile=0, bin_db=0.01, n_bins=4000, pool=None, pool_stride=0):
+    """Whole PAPR study: this rank's call (:func:`papr_sweep_local`), then :func:`reduce_papr`; identical on every rank and
+    for every world size and tile."""
+    hist, papr = papr_sweep_local(ctx, lp, points, streams_per_point, seed, rank, world, tile, bin_db, n_bins, pool, pool_stride)
+    ctx.sync()
+    return reduce_papr(hist, papr, bin_db)
