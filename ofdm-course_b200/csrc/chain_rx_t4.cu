@@ -544,7 +544,7 @@ __global__ void __launch_bounds__(T4_THREADS, 2) rx_t4_fast_kernel(T4Params p, T
             for (int w = tid; w < words; w += T4_THREADS) {
                 const uint32_t R = raw_word(w);
                 uint32_t o = R;
-                if (p.scramble) {
+                if (p.scramble) {                                   // descramble_word written out: the call reschedules this kernel
                     const uint32_t P = w ? raw_word(w - 1) : 0u;
                     const unsigned long long X = ((unsigned long long)R << 32) | P;
                     o = (uint32_t)((X ^ (X << 13) ^ (X << 14)) >> 32);
@@ -729,7 +729,7 @@ __global__ void __launch_bounds__(T4_THREADS, 2) t4_sym_kernel(T4Params p, T4Fas
     for (int q = lane; q < p.Np; q += 32) Po[q] = E[p.pil0[q]];
 }
 
-// Statistics of the sweep variant (t4_post_stats_kernel, ofdm_sweep_sync): what the stream's receiver reports besides its bits.
+// Statistics of the sweep variant (t4_post_kernel<Q, false, true>, ofdm_sweep_sync): what the stream's receiver reports besides its bits.
 struct T4Stats {
     const double2* Htrue;      // true response H(1:N_carrier), double
     double* rec;               // 9 fields x rec_stride doubles; this launch's stream b at rec[f * rec_stride + b]
@@ -751,270 +751,23 @@ __device__ __forceinline__ void t4_mer16(float2 e, float two_a, float a_in, floa
     s2 += er * er + ei * ei;
 }
 
-// t4_post_stats_kernel below is this kernel's twin for ofdm_sweep_sync, the same body line for line plus the statistics: a
-// change to the estimators, the channel estimate, the decisions or the descrambler here must be made there as well
-// (tests/test_gpu_sweep_sync.py compares the two chains' estimates and error counts bit for bit).
-template <bool QAM16, bool NEAR>
-__global__ void __launch_bounds__(T4_THREADS, 4) t4_post_kernel(T4Params p, T4FastExtra fx, PlanDev<float> plan, DevConst<float> con, int64_t B,
-                                                                const float2* __restrict__ Yd_all, const float2* __restrict__ Yp_all,
-                                                                const uint32_t* __restrict__ txbits, int64_t total_bits, uint32_t* __restrict__ outbits,
-                                                                unsigned long long* __restrict__ counts, double* __restrict__ tau_out,
-                                                                double* __restrict__ phase_out, float2* __restrict__ Hout, float near_eps) {
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    __shared__ double red[32];
-    __shared__ int red_i[32];
-    const int tid = threadIdx.x, lane = tid & 31;
-    const int M = p.Np * p.S;
-    // layout: region A = [angles (float) | rotations | decisions / raw words] (aliased in time), Yp (later: partial sums, then Gd), G, yk, dk
-    const size_t ang_bytes = sizeof(float) * (size_t)M, rot_bytes = sizeof(double2) * (size_t)p.Np, dec_bytes = (size_t)p.S * p.Nd;
-    float* ang = (float*)smem_raw;
-    float2* Yp = (float2*)(smem_raw + (max(max(ang_bytes, rot_bytes), max(dec_bytes, sizeof(float2) * (size_t)T4_THREADS)) + 15) / 16 * 16);
-    float2* G = Yp + M;
-    float2* yk = G + p.Nc;
-    float2* dk = yk + plan.n_knots;
-    const int fw = (p.frame_bits + 31) >> 5;
-    const int64_t b = blockIdx.x;
-    const float2* Yd = Yd_all + b * (int64_t)p.S * p.Nd;
-    const int64_t stream_bits = (int64_t)p.frame_bits * p.frames;
-    const int step_q = T4_THREADS % p.Np;                    // pilot index of item i = tid + T4_THREADS * j, advanced without a division
-    {
-        const float2* src = Yp_all + b * (int64_t)M;
-        for (int i = tid; i < M; i += T4_THREADS) Yp[i] = src[i];
-    }
-    __syncthreads();
-    // ---- fine_sync estimators (`Task 4/fine_sync.m:25-35,47-52`), products in double, angles in FP32 (as in the fused kernel)
-    double tau = 0.0, phase = 0.0;
-    if (p.time_desync || p.freq_desync) {
-        const double inv_c = 1.0 / (2.0 * CUDART_PI * (double)(p.pil0[1] - p.pil0[0]));       // tau_j = angle_j / (2 pi deltak)
-        auto q_at = [&](int i) -> double2 { return cmulc(p.pilots_d[i], to_d(Yp[i])); };
-        const int n = M - 1;
-        for (int j0 = 0; j0 < n; j0 += T4_THREADS) {          // angle of q_{j+1} conj(q_j): q_j once per thread, q_{j+1} from the next lane
-            const int j = j0 + tid;
-            double2 qa = make_double2(0.0, 0.0), qb;
-            if (j < M) qa = q_at(j);
-            qb.x = __shfl_down_sync(0xffffffffu, qa.x, 1);
-            qb.y = __shfl_down_sync(0xffffffffu, qa.y, 1);
-            if (lane == 31 && j + 1 < M) qb = q_at(j + 1);
-            if (j < n) { const double2 d = cmulc(qb, qa); ang[j] = atan2f((float)d.y, (float)d.x); }
-        }
-        __syncthreads();
-        const int CH = (n + T4_THREADS - 1) / T4_THREADS;
-        const int lo = min(tid * CH, n), hi = min(lo + CH, n);
-        int cmask = 0;
-        for (int j = max(lo, 1); j < hi; ++j) { double d = fabs((double)ang[j] - (double)ang[j - 1]) * inv_c; cmask += (d < 1e-3 && d != 0.0); }   // the difference first: exactly zero for equal angles
-        int rank = block_exclusive_scan(cmask, red_i);
-        double sum = 0; int kept = 0;
-        for (int j = max(lo, 1); j < hi; ++j) {
-            const double tj = (double)ang[j] * inv_c, d = fabs((double)ang[j] - (double)ang[j - 1]) * inv_c;
-            if (d < 1e-3 && d != 0.0) { if (rank >= p.Np) { sum += tj; ++kept; } ++rank; }
-        }
-        sum = block_sum(sum, red);
-        double nk = block_sum((double)kept, red);
-        tau = sum / nk;
-        double2* prot = (double2*)smem_raw;
-        __syncthreads();
-        for (int q = tid; q < p.Np; q += T4_THREADS) {
-            double sn = 0.0, cs = 1.0;
-            if (p.time_desync) sincospi(2.0 * tau * (double)p.pil0[q], &sn, &cs);
-            prot[q] = make_double2(cs, sn);
-        }
-        __syncthreads();
-        double ps = 0; int pn = 0;
-        for (int i = tid, pq = tid % p.Np; i < M; i += T4_THREADS) {
-            double2 rxv = to_d(Yp[i]);
-            if (p.time_desync) rxv = cmul(rxv, prot[pq]);
-            double2 qq = cmulc(p.pilots_d[i], rxv);
-            double a = (double)atan2f((float)qq.y, (float)qq.x);
-            if (fabs(a) > 1e-3) { ps += a; ++pn; }
-            pq += step_q; if (pq >= p.Np) pq -= p.Np;
-        }
-        ps = block_sum(ps, red);
-        double pk = block_sum((double)pn, red);
-        phase = ps / pk;
-        if (tid == 0) { if (tau_out) tau_out[b] = tau; if (phase_out) phase_out[b] = phase; }
-    }
-    {
-        double s2 = 0.0, c2 = 1.0;
-        if (p.freq_desync) sincos(phase, &s2, &c2);
-        for (int k = tid; k < p.Nc; k += T4_THREADS) {
-            double sn = 0.0, cs = 1.0;
-            if (p.time_desync || p.freq_desync) {
-                double s1, c1;
-                sincospi(p.time_desync ? 2.0 * tau * (double)k : 0.0, &s1, &c1);
-                cs = c1 * c2 - s1 * s2; sn = s1 * c2 + c1 * s2;
-            }
-            G[k] = make_float2((float)cs, (float)sn);
-        }
-    }
-    __syncthreads();
-    if (p.mp_desync) {
-        // symbol-averaged pilot LS values: PARTS threads per pilot (consecutive lanes = consecutive pilots: conflict-free shared
-        // reads, coalesced pilot table), partial sums combined in a fixed order
-        const int PARTS = min(min(T4_THREADS / p.Np, 4), p.S);
-        float2* part = (float2*)smem_raw;
-        if (tid < PARTS * p.Np) {
-            const int pt = tid / p.Np, q = tid - pt * p.Np;
-            const float2 g = G[p.pil0[q]];
-            float sr = 0.f, si = 0.f;
-            for (int s = pt; s < p.S; s += PARTS) { const float2 v = cdiv(cmul(Yp[s * p.Np + q], g), p.pilots[(int64_t)s * p.Np + q]); sr += v.x; si += v.y; }
-            part[tid] = make_float2(sr, si);
-        }
-        __syncthreads();
-        for (int q = tid; q < p.Np; q += T4_THREADS) {
-            float sr = 0.f, si = 0.f;
-            for (int pt = 0; pt < PARTS; ++pt) { sr += part[pt * p.Np + q].x; si += part[pt * p.Np + q].y; }
-            yk[q] = make_float2(sr / (float)p.S, si / (float)p.S);
-        }
-        __syncthreads();
-        float2* Hrow = Hout ? Hout + b * p.Nc : nullptr;
-        plan_apply_fn<float>(plan, yk, dk, [&](int k, float2 h) {
-            if (Hrow) Hrow[k] = h;
-            G[k] = cdiv(G[k], h);
-        });
-    }
-    __syncthreads();
-    float2* Gd = Yp;                                             // one-tap equaliser of the data carriers in payload order
-    for (int dr = tid; dr < p.Nd; dr += T4_THREADS) { const int c = p.data0[dr]; Gd[dr] = c < p.Nc ? G[c] : make_float2(0.f, 0.f); }
-    __syncthreads();
-    int errs = 0, nears = 0;
-    if (QAM16 && (stream_bits & 31) == 0 && p.frame_bits >= 64 && (p.Nd & 3) == 0) {
-        // word-aligned 16QAM streams: one thread decides the eight consecutive payload symbols of a 32-bit word (64 contiguous
-        // bytes of the compact data-carrier array); a group of four never straddles two OFDM symbols because Nd % 4 == 0
-        const int words = (int)(stream_bits >> 5);
-        uint32_t* rawW = (uint32_t*)smem_raw;
-        const float4* Yv = reinterpret_cast<const float4*>(Yd);
-        for (int w = tid; w < words; w += T4_THREADS) {
-            float4 y[4];
-#pragma unroll
-            for (int u = 0; u < 4; ++u) y[u] = __ldg(Yv + 4 * w + u);
-            const int i0 = 8 * w;
-            const int dr0 = i0 - (i0 / p.Nd) * p.Nd;
-            const int dr1 = dr0 + 4 >= p.Nd ? 0 : dr0 + 4;
-            float4 g[4];
-            g[0] = *reinterpret_cast<const float4*>(Gd + dr0); g[1] = *reinterpret_cast<const float4*>(Gd + dr0 + 2);
-            g[2] = *reinterpret_cast<const float4*>(Gd + dr1); g[3] = *reinterpret_cast<const float4*>(Gd + dr1 + 2);
-            uint32_t R = 0;
-#pragma unroll
-            for (int u = 0; u < 4; ++u) {
-                const float2 e0 = cmul(make_float2(y[u].x, y[u].y), make_float2(g[u].x, g[u].y));
-                const float2 e1 = cmul(make_float2(y[u].z, y[u].w), make_float2(g[u].z, g[u].w));
-                float m0 = 1.f, m1 = 1.f;
-                R |= demap16_nib<NEAR>(e0.x, e0.y, fx.two_a, &m0) << (8 * u);
-                R |= demap16_nib<NEAR>(e1.x, e1.y, fx.two_a, &m1) << (8 * u + 4);
-                if (NEAR) nears += (m0 < near_eps) + (m1 < near_eps);
-            }
-            rawW[w] = R;
-        }
-        __syncthreads();
-        const uint32_t* tb = txbits ? txbits + b * words : nullptr;
-        uint32_t* ob = outbits ? outbits + b * words : nullptr;
-        for (int w = tid; w < words; w += T4_THREADS) {
-            const uint32_t R = rawW[w];
-            uint32_t o = R;
-            if (p.scramble) {
-                const uint32_t P = w ? rawW[w - 1] : 0u;
-                const unsigned long long X = ((unsigned long long)R << 32) | P;
-                o = (uint32_t)((X ^ (X << 13) ^ (X << 14)) >> 32);
-                const int fl = (32 * w + 31) / p.frame_bits;
-                const int t = fl * p.frame_bits - 32 * w;
-                if (t > -14) {
-                    const int sh = 32 + t;
-                    const unsigned long long keep = ~0ull << sh;
-                    const unsigned long long hist = sh >= 32 ? ((unsigned long long)p.prev0 << (sh - 32)) : ((unsigned long long)p.prev0 >> (32 - sh));
-                    const unsigned long long Xf = (X & keep) | (hist & ~keep);
-                    const uint32_t of = (uint32_t)((Xf ^ (Xf << 13) ^ (Xf << 14)) >> 32);
-                    const uint32_t before = t > 0 ? ((1u << t) - 1u) : 0u;
-                    o = (o & before) | (of & ~before);
-                }
-            }
-            if (tb) errs += __popc(o ^ tb[w]);
-            if (ob) ob[w] = o;
-        }
-    } else {
-        uint8_t* dec = (uint8_t*)smem_raw;
-        for (int dr = tid; dr < p.Nd; dr += T4_THREADS) {
-            const float2 g = Gd[dr];
-            const float2* Yc = Yd + dr;
-            for (int s0 = 0; s0 < p.S; s0 += 10) {
-                float2 y[10];
-#pragma unroll
-                for (int u = 0; u < 10; ++u) y[u] = (s0 + u < p.S) ? ldg_stream(Yc + (int64_t)(s0 + u) * p.Nd) : make_float2(0.f, 0.f);
-#pragma unroll
-                for (int u = 0; u < 10; ++u)
-                    if (s0 + u < p.S) {
-                        const float2 e = cmul(y[u], g);
-                        float margin = 1.f;
-                        uint32_t code;
-                        if (QAM16) code = demap16_nib<NEAR>(e.x, e.y, fx.two_a, &margin);
-                        else code = (uint32_t)nearest_idx(con, e.x, e.y, &margin);
-                        if (NEAR && margin < near_eps) ++nears;
-                        dec[(s0 + u) * p.Nd + dr] = (uint8_t)code;
-                    }
-            }
-        }
-        __syncthreads();
-        const int fpb = p.SpF * p.Nd;
-        auto packed = [&](const uint8_t* fr, int wd) -> uint32_t {
-            uint32_t word = 0;
-            if (QAM16) {
-#pragma unroll
-                for (int j = 0; j < 8; ++j) { const int q = 8 * wd + j; if (q < fpb) word |= (uint32_t)fr[q] << (4 * j); }
-            } else {
-                const int b0 = 32 * wd, b1 = min(b0 + 32, p.frame_bits);
-                for (int q = b0 / p.bps; q * p.bps < b1; ++q) {
-                    int idx = fr[q];
-                    for (int i = 0; i < p.bps; ++i) {
-                        int pos = q * p.bps + i;
-                        if (pos >= b0 && pos < b1 && ((idx >> (p.bps - 1 - i)) & 1)) word |= 1u << (pos - b0);
-                    }
-                }
-            }
-            return word;
-        };
-        for (int item = tid; item < p.frames * fw; item += T4_THREADS) {
-            const int f = item / fw, wd = item - f * fw;
-            const uint8_t* fr = dec + (size_t)f * fpb;
-            const uint32_t cw = packed(fr, wd);
-            uint32_t o = cw;
-            if (p.scramble) {
-                const uint32_t prev = wd ? packed(fr, wd - 1) : p.prev0;
-                o = cw ^ ((cw << 13) | (prev >> 19)) ^ ((cw << 14) | (prev >> 18));
-            }
-            const int n = min(32, p.frame_bits - 32 * wd);
-            if (n < 32) o &= (1u << n) - 1u;
-            const int64_t base = b * stream_bits + (int64_t)f * p.frame_bits;
-            if (txbits) errs += __popc(o ^ bits_get32(txbits, base + 32 * (int64_t)wd, min(total_bits, base + p.frame_bits)));
-            if (outbits) bits_put(outbits, base + 32 * (int64_t)wd, n, o);
-        }
-    }
-    errs = block_sum(errs, red_i);
-    nears = block_sum(nears, red_i);
-    if (tid == 0 && counts) {
-        if (errs) atomicAdd(&counts[0], (unsigned long long)errs);
-        atomicAdd(&counts[1], (unsigned long long)stream_bits);
-        if (nears) atomicAdd(&counts[2], (unsigned long long)nears);
-    }
-}
-
-// Statistics variant of t4_post_kernel for ofdm_sweep_sync, a sibling kernel so that t4_post_kernel's four instantiations keep
-// their code: the same chain and arithmetic (no output bits, H or near-boundary count), and the same CTA also
+// STATS (ofdm_sweep_sync, NEAR false): the same chain and arithmetic without output bits, tau / phase, H or near-boundary
+// count, and the same CTA also
 //   * accumulates the channel-estimate error sum |H_est(k) - H(k)|^2 in double against st.Htrue while the spline emits H_est
 //     (never stored), with mse_kernel's terms;
 //   * accumulates the MER sums of `MER_func.m:7-25` while the data carriers are decided;
 //   * reduces both with the fixed-order block_sum, writes the stream's record and adds {detector failure, IFO = -1} to the
 //     point's row {errors, bits, detector failures, IFO misses} with integer atomics.
-// The constant locals at the top stand for t4_post_kernel's switched-off outputs, so that the body reads line for line as its.
-template <bool QAM16>
-__global__ void __launch_bounds__(T4_THREADS, 4) t4_post_stats_kernel(T4Params p, T4FastExtra fx, PlanDev<float> plan, DevConst<float> con, int64_t B,
-                                                                      const float2* __restrict__ Yd_all, const float2* __restrict__ Yp_all,
-                                                                      const uint32_t* __restrict__ txbits, int64_t total_bits,
-                                                                      unsigned long long* __restrict__ counts, T4Stats st) {
-    constexpr bool NEAR = false;
-    const float near_eps = 0.f;
-    uint32_t* const outbits = nullptr;
-    double* const tau_out = nullptr;
-    double* const phase_out = nullptr;
-    float2* const Hout = nullptr;
+// st is the last parameter so that the other parameters keep their offsets; the kernels without STATS do not read it.
+template <bool QAM16, bool NEAR, bool STATS>
+__global__ void __launch_bounds__(T4_THREADS, 4) t4_post_kernel(T4Params p, T4FastExtra fx, PlanDev<float> plan, DevConst<float> con, int64_t B,
+                                                                const float2* __restrict__ Yd_all, const float2* __restrict__ Yp_all,
+                                                                const uint32_t* __restrict__ txbits, int64_t total_bits, uint32_t* __restrict__ outbits,
+                                                                unsigned long long* __restrict__ counts, double* __restrict__ tau_out,
+                                                                double* __restrict__ phase_out, float2* __restrict__ Hout, float near_eps, T4Stats st) {
+    if constexpr (STATS) {                                       // switched-off outputs: their branches go at compile time
+        outbits = nullptr; tau_out = nullptr; phase_out = nullptr; Hout = nullptr; near_eps = 0.f;
+    }
     extern __shared__ __align__(16) unsigned char smem_raw[];
     __shared__ double red[32];
     __shared__ int red_i[32];
@@ -1102,7 +855,7 @@ __global__ void __launch_bounds__(T4_THREADS, 4) t4_post_stats_kernel(T4Params p
         }
     }
     __syncthreads();
-    double herr = 0.0, mer1 = 0.0, mer2 = 0.0;
+    double herr = 0.0, mer1 = 0.0, mer2 = 0.0;                   // STATS only
     if (p.mp_desync) {
         // symbol-averaged pilot LS values: PARTS threads per pilot (consecutive lanes = consecutive pilots: conflict-free shared
         // reads, coalesced pilot table), partial sums combined in a fixed order
@@ -1125,9 +878,11 @@ __global__ void __launch_bounds__(T4_THREADS, 4) t4_post_stats_kernel(T4Params p
         float2* Hrow = Hout ? Hout + b * p.Nc : nullptr;
         plan_apply_fn<float>(plan, yk, dk, [&](int k, float2 h) {
             if (Hrow) Hrow[k] = h;
-            const double2 t = st.Htrue[k];                       // the terms of mse_kernel, in double
-            const double dr = t.x - (double)h.x, di = t.y - (double)h.y;
-            herr += dr * dr + di * di;
+            if constexpr (STATS) {
+                const double2 t = st.Htrue[k];                   // the terms of mse_kernel, in double
+                const double dr = t.x - (double)h.x, di = t.y - (double)h.y;
+                herr += dr * dr + di * di;
+            }
             G[k] = cdiv(G[k], h);
         });
     }
@@ -1161,8 +916,10 @@ __global__ void __launch_bounds__(T4_THREADS, 4) t4_post_stats_kernel(T4Params p
                 R |= demap16_nib<NEAR>(e0.x, e0.y, fx.two_a, &m0) << (8 * u);
                 R |= demap16_nib<NEAR>(e1.x, e1.y, fx.two_a, &m1) << (8 * u + 4);
                 if (NEAR) nears += (m0 < near_eps) + (m1 < near_eps);
-                t4_mer16(e0, fx.two_a, st.a_in, st.a_out, mer1, mer2);
-                t4_mer16(e1, fx.two_a, st.a_in, st.a_out, mer1, mer2);
+                if constexpr (STATS) {
+                    t4_mer16(e0, fx.two_a, st.a_in, st.a_out, mer1, mer2);
+                    t4_mer16(e1, fx.two_a, st.a_in, st.a_out, mer1, mer2);
+                }
             }
             rawW[w] = R;
         }
@@ -1172,7 +929,7 @@ __global__ void __launch_bounds__(T4_THREADS, 4) t4_post_stats_kernel(T4Params p
         for (int w = tid; w < words; w += T4_THREADS) {
             const uint32_t R = rawW[w];
             uint32_t o = R;
-            if (p.scramble) {
+            if (p.scramble) {                                       // descramble_word written out: the call reschedules this kernel
                 const uint32_t P = w ? rawW[w - 1] : 0u;
                 const unsigned long long X = ((unsigned long long)R << 32) | P;
                 o = (uint32_t)((X ^ (X << 13) ^ (X << 14)) >> 32);
@@ -1209,11 +966,13 @@ __global__ void __launch_bounds__(T4_THREADS, 4) t4_post_stats_kernel(T4Params p
                         if (QAM16) code = demap16_nib<NEAR>(e.x, e.y, fx.two_a, &margin);
                         else code = (uint32_t)nearest_idx(con, e.x, e.y, &margin);
                         if (NEAR && margin < near_eps) ++nears;
-                        if (QAM16) t4_mer16(e, fx.two_a, st.a_in, st.a_out, mer1, mer2);
-                        else {                                   // `MER_func.m:7-25` as mer_kernel: the decided (nearest) point
-                            const double ir = con.re[code], ii = con.im[code], er = ir - (double)e.x, ei = ii - (double)e.y;
-                            mer1 += ir * ir + ii * ii;
-                            mer2 += er * er + ei * ei;
+                        if constexpr (STATS) {
+                            if (QAM16) t4_mer16(e, fx.two_a, st.a_in, st.a_out, mer1, mer2);
+                            else {                               // `MER_func.m:7-25` as mer_kernel: the decided (nearest) point
+                                const double ir = con.re[code], ii = con.im[code], er = ir - (double)e.x, ei = ii - (double)e.y;
+                                mer1 += ir * ir + ii * ii;
+                                mer2 += er * er + ei * ei;
+                            }
                         }
                         dec[(s0 + u) * p.Nd + dr] = (uint8_t)code;
                     }
@@ -1261,25 +1020,27 @@ __global__ void __launch_bounds__(T4_THREADS, 4) t4_post_stats_kernel(T4Params p
         atomicAdd(&counts[1], (unsigned long long)stream_bits);
         if (nears) atomicAdd(&counts[2], (unsigned long long)nears);
     }
-    herr = block_sum(herr, red);                                  // fixed-order block reductions
-    mer1 = block_sum(mer1, red);
-    mer2 = block_sum(mer2, red);
-    if (tid == 0) {
-        const int ifo = p.freq_desync ? st.ifo[b] : 0;
-        const int fail = st.fail ? st.fail[b] : 0;
-        double* r = st.rec + b;
-        const int64_t sd = st.rec_stride;
-        r[0] = p.time_desync ? (double)st.tg[b] : 0.0;
-        r[sd] = p.freq_desync ? st.fo[b] : 0.0;
-        r[2 * sd] = (double)ifo;
-        r[3 * sd] = tau;
-        r[4 * sd] = phase;
-        r[5 * sd] = p.mp_desync ? herr / (double)p.Nc : CUDART_NAN;
-        r[6 * sd] = 10.0 * log10(mer1 / mer2);
-        r[7 * sd] = (double)st.nsto[b];
-        r[8 * sd] = st.cfo[b];
-        if (fail) atomicAdd(&counts[2], 1ull);                    // row {errors, bits, detector failures, IFO misses}
-        if (ifo < 0) atomicAdd(&counts[3], 1ull);
+    if constexpr (STATS) {
+        herr = block_sum(herr, red);                              // fixed-order block reductions
+        mer1 = block_sum(mer1, red);
+        mer2 = block_sum(mer2, red);
+        if (tid == 0) {
+            const int ifo = p.freq_desync ? st.ifo[b] : 0;
+            const int fail = st.fail ? st.fail[b] : 0;
+            double* r = st.rec + b;
+            const int64_t sd = st.rec_stride;
+            r[0] = p.time_desync ? (double)st.tg[b] : 0.0;
+            r[sd] = p.freq_desync ? st.fo[b] : 0.0;
+            r[2 * sd] = (double)ifo;
+            r[3 * sd] = tau;
+            r[4 * sd] = phase;
+            r[5 * sd] = p.mp_desync ? herr / (double)p.Nc : CUDART_NAN;
+            r[6 * sd] = 10.0 * log10(mer1 / mer2);
+            r[7 * sd] = (double)st.nsto[b];
+            r[8 * sd] = st.cfo[b];
+            if (fail) atomicAdd(&counts[2], 1ull);                    // row {errors, bits, detector failures, IFO misses}
+            if (ifo < 0) atomicAdd(&counts[3], 1ull);
+        }
     }
 }
 
@@ -1440,6 +1201,96 @@ int ofdm_tx1024_fast(ofdm_ctx* ctx, const ofdm_link_params* lp, const uint32_t* 
 extern "C" int ofdm_cp_autocorr(ofdm_ctx* ctx, const void* rx, int64_t B, int64_t L, int W, int Nfft, void* autocorr, int32_t* tg_pos, double* freq_off,
                                 int32_t* fail);
 
+// T4Params of a link with its device tables (0-based carriers, pilots in FP32 and double, twiddles) and the spline plan of
+// interp1 over the carriers (no edge extension).  Error messages name the entry point fn.
+static int t4_setup(ofdm_ctx* ctx, const char* fn, const ofdm_link_params* lp, int bps, int time_desync, int freq_desync, int mp_desync, T4Params& p,
+                    const InterpPlan*& pl) {
+    p.Nfft = lp->Nfft; p.logN = ilog2(lp->Nfft); p.Tg = lp->Tg; p.Nc = lp->N_carrier; p.S = lp->S; p.SpF = lp->SpF; p.Nd = lp->Nd; p.Np = lp->Np;
+    p.bps = bps; p.scramble = lp->scramble; p.frame_bits = lp->SpF * lp->Nd * bps; p.frames = lp->S / lp->SpF;
+    p.time_desync = time_desync != 0; p.freq_desync = freq_desync != 0; p.mp_desync = mp_desync != 0;
+    p.prev0 = ofdm_reg_to_prev(lp->reg0_host);
+    std::vector<int32_t> d0(lp->Nd), p0(lp->Np);
+    for (int i = 0; i < lp->Nd; ++i) {
+        if (lp->data_carriers_host[i] < 1 || lp->data_carriers_host[i] > lp->Nfft) return ctx_fail(ctx, OFDM_ERR_INVALID, "%s: data carrier out of range", fn);
+        d0[i] = lp->data_carriers_host[i] - 1;
+    }
+    for (int i = 0; i < lp->Np; ++i) {
+        if (lp->pilot_carriers_host[i] < 1 || lp->pilot_carriers_host[i] > lp->N_carrier) return ctx_fail(ctx, OFDM_ERR_INVALID, "%s: pilot carrier out of range", fn);
+        if (i > 0 && lp->pilot_carriers_host[i] <= lp->pilot_carriers_host[i - 1]) return ctx_fail(ctx, OFDM_ERR_INVALID, "%s: pilot carriers must increase", fn);
+        p0[i] = lp->pilot_carriers_host[i] - 1;
+    }
+    p.data0 = (const int32_t*)ctx_blob(ctx, d0.data(), sizeof(int32_t) * d0.size());
+    p.pil0 = (const int32_t*)ctx_blob(ctx, p0.data(), sizeof(int32_t) * p0.size());
+    p.pilots = (const float2*)ofdm_upload_pilots(ctx, lp->pilot_vals_host, (size_t)lp->Np * lp->S);
+    p.pilots_d = (const double2*)ctx_blob(ctx, lp->pilot_vals_host, sizeof(double) * 2 * (size_t)lp->Np * lp->S);
+    p.tw = (const float2*)ctx_twiddles(ctx, lp->Nfft);
+    std::vector<int32_t> q(lp->N_carrier);
+    for (int i = 0; i < lp->N_carrier; ++i) q[i] = i + 1;
+    pl = ctx_plan(ctx, lp->pilot_carriers_host, lp->Np, 0, q.data(), lp->N_carrier, OFDM_INTERP_SPLINE);
+    if (!(p.data0 && p.pil0 && p.pilots && p.pilots_d && p.tw && pl)) return ctx_fail(ctx, OFDM_ERR_INVALID, "%s: device upload failed", fn);
+    return OFDM_OK;
+}
+
+static const size_t T4_TILES = sizeof(float2) * (T4_THREADS / 32) * 32 * T4F_EROW;   // one 32 x 33 transpose tile per warp
+static const int64_t T4_SPLIT_CHUNK = 16384;                   // streams per pass of the split chain: 2.6 GB of kept bins at the Task-4 shape
+
+// dynamic shared memory of t4_post_kernel: region A (angles | rotations | decisions / raw words), then Yp, G, yk, dk
+static size_t t4_post_smem(const T4Params& p, const InterpPlan* pl) {
+    return (std::max(std::max(sizeof(float) * (size_t)p.S * p.Np, 16 * (size_t)p.Np), std::max(8 * (size_t)T4_THREADS, (size_t)p.S * p.Nd)) + 15) / 16 * 16 +
+           sizeof(float2) * ((size_t)p.S * p.Np + p.Nc + 2 * (size_t)pl->n_knots) + 32;
+}
+
+typedef void (*t4_post_t)(T4Params, T4FastExtra, PlanDev<float>, DevConst<float>, int64_t, const float2*, const float2*, const uint32_t*, int64_t,
+                          uint32_t*, unsigned long long*, double*, double*, float2*, float, T4Stats);
+
+// The split Task-4 chain (Nfft = 1024): t4_ifo_kernel -> t4_sym_kernel -> post, each kernel at its own occupancy, in passes
+// of at most T4_SPLIT_CHUNK streams (the caller makes sure an unaligned batch fits one pass).  tg / fo are the detector's
+// estimates, ifo is written when the chain corrects the frequency.  post gets the BER outputs (each may be NULL) or, for a
+// STATS instantiation, st with its per-stream pointers at stream 0.
+static int t4_split_run(ofdm_ctx* ctx, const ofdm_link_params* lp, const T4Params& p, const T4FastExtra& fx, const InterpPlan* pl, t4_post_t post,
+                        const void* rx, int64_t B, int64_t L, const int32_t* tg, const double* fo, int32_t* ifo, const uint32_t* tx_bits,
+                        uint32_t* out_bits, int64_t* counts, double* tau, double* phase, float2* H, float near_eps, const T4Stats* st) {
+    const int64_t CH = std::min<int64_t>(B, T4_SPLIT_CHUNK);
+    const int groups = (p.S + T4_THREADS / 32 - 1) / (T4_THREADS / 32);
+    const size_t sym_smem = T4_TILES + sizeof(float2) * 1024, post_smem = t4_post_smem(p, pl);
+    auto symk = p.Nc <= 416 ? t4_sym_kernel<13> : t4_sym_kernel<32>;
+    CUDA_TRY(ctx, cudaFuncSetAttribute(t4_ifo_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T4_TILES));
+    CUDA_TRY(ctx, cudaFuncSetAttribute(symk, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sym_smem));
+    CUDA_TRY(ctx, cudaFuncSetAttribute(post, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)post_smem));
+    float2* bins = nullptr;
+    CUDA_TRY(ctx, cudaMallocAsync((void**)&bins, sizeof(float2) * (size_t)CH * p.S * ((size_t)p.Nd + p.Np), ctx->stream));
+    float2* Yd_all = bins;
+    float2* Yp_all = bins + (size_t)CH * p.S * p.Nd;
+    const int64_t stream_bits = (int64_t)p.frame_bits * p.frames, words = stream_bits / 32;
+    int rc = OFDM_OK;
+    // (Running the post kernel of one chunk on a side stream under the symbol kernel of the next was tried: the symbol
+    // kernel's two CTAs hold every register of an SM, nothing co-resides, and the smaller chunks only add tails.)
+    for (int64_t c0 = 0; c0 < B && rc == OFDM_OK; c0 += CH) {
+        const int64_t nb = std::min(CH, B - c0);
+        const float2* rxc = (const float2*)rx + c0 * L;
+        if (p.freq_desync) {
+            t4_ifo_kernel<<<(unsigned)cdiv64(nb, T4_THREADS / 32), T4_THREADS, T4_TILES, ctx->stream>>>(fx, rxc, nb, L, p.Tg, p.time_desync, tg + c0, fo + c0, ifo + c0);
+            ctx->launches++;
+        }
+        symk<<<(unsigned)(nb * groups), T4_THREADS, sym_smem, ctx->stream>>>(p, fx, rxc, nb, L, groups, tg + c0, fo + c0, ifo + c0, Yd_all, Yp_all);
+        T4Stats s{};
+        if (st) {
+            s = *st;
+            s.rec += c0; s.tg += c0; s.fo += c0; s.ifo += c0; s.nsto += c0; s.cfo += c0;
+            if (s.fail) s.fail += c0;
+        }
+        post<<<(unsigned)nb, T4_THREADS, post_smem, ctx->stream>>>(p, fx, plan_dev<float>(pl), make_devconst<float>(lp->constellation), nb, Yd_all, Yp_all,
+                                                                   tx_bits ? tx_bits + c0 * words : nullptr, nb * stream_bits,
+                                                                   out_bits ? out_bits + c0 * words : nullptr, (unsigned long long*)counts,
+                                                                   tau ? tau + c0 : nullptr, phase ? phase + c0 : nullptr, H ? H + c0 * p.Nc : nullptr, near_eps, s);
+        ctx->launches += 2;
+        cudaError_t e = cudaGetLastError();
+        if (e != cudaSuccess) rc = ctx_fail(ctx, OFDM_ERR_CUDA, "%s launch failed: %s", st ? "statistics chain" : "split Task-4 chain", cudaGetErrorString(e));
+    }
+    cudaFreeAsync(bins, ctx->stream);
+    return rc;
+}
+
 extern "C" int ofdm_rx_chain_t4(ofdm_ctx* ctx, const ofdm_link_params* lp, const void* rx, int64_t B, int time_desync, int freq_desync, int mp_desync,
                                 const uint32_t* tx_bits, uint32_t* out_bits, int64_t* counts, int32_t* tg_dev, double* fo_dev, int32_t* ifo_dev,
                                 double* tau_dev, double* phase_dev, void* H_dev, double near_eps) {
@@ -1460,26 +1311,9 @@ extern "C" int ofdm_rx_chain_t4_ex(ofdm_ctx* ctx, const ofdm_link_params* lp, co
     REQUIRE(ctx, ct.bps > 0, "unknown constellation");
     const int64_t L = (int64_t)lp->S * (lp->Nfft + lp->Tg);
     T4Params p;
-    p.Nfft = lp->Nfft; p.logN = ilog2(lp->Nfft); p.Tg = lp->Tg; p.Nc = lp->N_carrier; p.S = lp->S; p.SpF = lp->SpF; p.Nd = lp->Nd; p.Np = lp->Np;
-    p.bps = ct.bps; p.scramble = lp->scramble; p.frame_bits = lp->SpF * lp->Nd * ct.bps; p.frames = lp->S / lp->SpF;
-    p.time_desync = time_desync != 0; p.freq_desync = freq_desync != 0; p.mp_desync = mp_desync != 0;
-    p.prev0 = ofdm_reg_to_prev(lp->reg0_host);
-    std::vector<int32_t> d0(lp->Nd), p0(lp->Np);
-    for (int i = 0; i < lp->Nd; ++i) { REQUIRE(ctx, lp->data_carriers_host[i] >= 1 && lp->data_carriers_host[i] <= lp->Nfft, "data carrier out of range"); d0[i] = lp->data_carriers_host[i] - 1; }
-    for (int i = 0; i < lp->Np; ++i) {
-        REQUIRE(ctx, lp->pilot_carriers_host[i] >= 1 && lp->pilot_carriers_host[i] <= lp->N_carrier, "pilot carrier out of range");
-        REQUIRE(ctx, i == 0 || lp->pilot_carriers_host[i] > lp->pilot_carriers_host[i - 1], "pilot carriers must increase");
-        p0[i] = lp->pilot_carriers_host[i] - 1;
-    }
-    p.data0 = (const int32_t*)ctx_blob(ctx, d0.data(), sizeof(int32_t) * d0.size());
-    p.pil0 = (const int32_t*)ctx_blob(ctx, p0.data(), sizeof(int32_t) * p0.size());
-    p.pilots = (const float2*)ofdm_upload_pilots(ctx, lp->pilot_vals_host, (size_t)lp->Np * lp->S);
-    p.pilots_d = (const double2*)ctx_blob(ctx, lp->pilot_vals_host, sizeof(double) * 2 * (size_t)lp->Np * lp->S);
-    p.tw = (const float2*)ctx_twiddles(ctx, lp->Nfft);
-    std::vector<int32_t> q(lp->N_carrier);
-    for (int i = 0; i < lp->N_carrier; ++i) q[i] = i + 1;
-    const InterpPlan* pl = ctx_plan(ctx, lp->pilot_carriers_host, lp->Np, 0, q.data(), lp->N_carrier, OFDM_INTERP_SPLINE);   // interp1 over the carriers, no edge extension
-    REQUIRE(ctx, p.data0 && p.pil0 && p.pilots && p.pilots_d && p.tw && pl, "device upload failed");
+    const InterpPlan* pl = nullptr;
+    int rc = t4_setup(ctx, __func__, lp, ct.bps, time_desync, freq_desync, mp_desync, p, pl);
+    if (rc) return rc;
     const int grid = (int)std::min<int64_t>(B, (int64_t)ctx->sm_count * 2);
     // scratch: [estimates: tg int32 | fo double] + per-CTA parking area
     const size_t park = sizeof(float2) * (size_t)grid * lp->S * lp->N_carrier;
@@ -1490,7 +1324,6 @@ extern "C" int ofdm_rx_chain_t4_ex(ofdm_ctx* ctx, const ofdm_link_params* lp, co
     int32_t* tg_s = (int32_t*)(fo_s + B);
     if (!fo_dev) fo_dev = fo_s;
     if (!tg_dev) tg_dev = tg_s;
-    int rc = OFDM_OK;
     if (time_desync || freq_desync) rc = ofdm_cp_autocorr(ctx, rx, B, L, lp->Tg, lp->Nfft, nullptr, tg_dev, fo_dev, fail_dev);
     if (rc == OFDM_OK) {
         const int64_t stream_bits = (int64_t)p.frame_bits * p.frames;
@@ -1503,17 +1336,11 @@ extern "C" int ofdm_rx_chain_t4_ex(ofdm_ctx* ctx, const ofdm_link_params* lp, co
         // fast path: Nfft = 1024, warp-per-symbol register FFT (rx_t4_fast_kernel)
         bool fast_done = false;
         if (rc == OFDM_OK && p.Nfft == 1024 && !getenv("OFDM_B200_NO_FAST")) {
-            const size_t tiles = sizeof(float2) * (size_t)(T4_THREADS / 32) * 32 * T4F_EROW, taus = sizeof(double) * (size_t)p.S * p.Np;
-            const size_t fsmem = (std::max(tiles, taus) + 15) / 16 * 16 + sizeof(float2) * (1024 + (size_t)p.S * p.Np + p.S + p.Nc + 2 * (size_t)pl->n_knots) + 32;
-            if (fsmem <= 111 * 1024 && (size_t)p.S * p.Nd <= std::max(tiles, taus)) {
-                std::vector<float> twt(2 * 1024);
-                for (int k1 = 0; k1 < 32; ++k1)
-                    for (int n2 = 0; n2 < 32; ++n2) {
-                        const long double a = -2.0L * 3.14159265358979323846264338327950288L * (long double)((n2 * k1) & 1023) / 1024.0L;
-                        twt[2 * (32 * k1 + n2)] = (float)cosl(a); twt[2 * (32 * k1 + n2) + 1] = (float)sinl(a);
-                    }
+            const size_t taus = sizeof(double) * (size_t)p.S * p.Np;
+            const size_t fsmem = (std::max(T4_TILES, taus) + 15) / 16 * 16 + sizeof(float2) * (1024 + (size_t)p.S * p.Np + p.S + p.Nc + 2 * (size_t)pl->n_knots) + 32;
+            if (fsmem <= 111 * 1024 && (size_t)p.S * p.Nd <= std::max(T4_TILES, taus)) {
                 T4FastExtra fx;
-                fx.tw_t = (const float2*)ctx_blob(ctx, twt.data(), sizeof(float) * twt.size());
+                fx.tw_t = (const float2*)t4_twiddle_blob(ctx);
                 fx.two_a = 2.f * (float)ct.re[12];
                 const bool q16 = lp->constellation == OFDM_16QAM, near = near_eps > 0.0, small = p.Nc <= 416;
                 typedef void (*kern_t)(T4Params, T4FastExtra, PlanDev<float>, DevConst<float>, const float2*, int64_t, int64_t, const int32_t*, const double*, float2*,
@@ -1522,50 +1349,16 @@ extern "C" int ofdm_rx_chain_t4_ex(ofdm_ctx* ctx, const ofdm_link_params* lp, co
                                            : (near ? rx_t4_fast_kernel<13, false, true> : rx_t4_fast_kernel<13, false, false>))
                                     : (q16 ? (near ? rx_t4_fast_kernel<32, true, true> : rx_t4_fast_kernel<32, true, false>)
                                            : (near ? rx_t4_fast_kernel<32, false, true> : rx_t4_fast_kernel<32, false, false>));
-                // large batches: the same arithmetic as three kernels, each at its own occupancy (t4_ifo / t4_sym / t4_post);
-                // ofdm_rx_t4_sync_stats repeats this setup and these conditions for ofdm_sweep_sync: keep the two in step
-                const int64_t SPLIT_CHUNK = 16384;                      // streams per pass: 2.6 GB of kept bins at the Task-4 shape
+                // large batches: the same arithmetic as three kernels, each at its own occupancy (t4_split_run)
                 const bool aligned = stream_bits % 32 == 0;
-                const size_t post_smem = (std::max(std::max(sizeof(float) * (size_t)p.S * p.Np, 16 * (size_t)p.Np), std::max(8 * (size_t)T4_THREADS, (size_t)p.S * p.Nd)) + 15) / 16 * 16 + sizeof(float2) * ((size_t)p.S * p.Np + p.Nc + 2 * (size_t)pl->n_knots) + 32;
-                const size_t sym_smem = tiles + sizeof(float2) * 1024;
-                if (fx.tw_t && B >= 512 && (aligned || B <= SPLIT_CHUNK) && post_smem <= 100 * 1024 && p.Np <= T4_THREADS && p.Nd <= p.S * p.Np && !getenv("OFDM_B200_T4_FUSED")) {
-                    const int64_t CH = std::min<int64_t>(B, SPLIT_CHUNK);
-                    const int groups = (p.S + T4_THREADS / 32 - 1) / (T4_THREADS / 32);
-                    float2* bins = nullptr;
-                    cudaError_t e = cudaMallocAsync((void**)&bins, sizeof(float2) * (size_t)CH * p.S * ((size_t)p.Nd + p.Np), ctx->stream);
-                    if (e != cudaSuccess) rc = ctx_fail(ctx, OFDM_ERR_CUDA, "cudaMallocAsync failed: %s", cudaGetErrorString(e));
-                    float2* Yd_all = bins;
-                    float2* Yp_all = bins + (size_t)CH * p.S * p.Nd;
+                if (fx.tw_t && B >= 512 && (aligned || B <= T4_SPLIT_CHUNK) && t4_post_smem(p, pl) <= 100 * 1024 && p.Np <= T4_THREADS && p.Nd <= p.S * p.Np &&
+                    !getenv("OFDM_B200_T4_FUSED")) {
                     int32_t* ifo_ptr = ifo_dev ? ifo_dev : tg_s + B;      // the scratch holds two int32 per stream
-                    if (rc == OFDM_OK && !freq_desync && ifo_dev) cudaMemsetAsync(ifo_dev, 0, sizeof(int32_t) * B, ctx->stream);
-                    typedef void (*post_t)(T4Params, T4FastExtra, PlanDev<float>, DevConst<float>, int64_t, const float2*, const float2*, const uint32_t*, int64_t,
-                                           uint32_t*, unsigned long long*, double*, double*, float2*, float);
-                    post_t post = q16 ? (near ? t4_post_kernel<true, true> : t4_post_kernel<true, false>) : (near ? t4_post_kernel<false, true> : t4_post_kernel<false, false>);
-                    auto symk = small ? t4_sym_kernel<13> : t4_sym_kernel<32>;
-                    cudaFuncSetAttribute(t4_ifo_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tiles);
-                    cudaFuncSetAttribute(symk, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sym_smem);
-                    cudaFuncSetAttribute(post, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)post_smem);
-                    const int64_t words = stream_bits / 32;
-                    // (Running the post kernel of one chunk on a side stream under the symbol kernel of the next was tried: the symbol
-                    // kernel's two CTAs hold every register of an SM, nothing co-resides, and the smaller chunks only add tails.)
-                    for (int64_t c0 = 0; c0 < B && rc == OFDM_OK; c0 += CH) {
-                        const int64_t nb = std::min(CH, B - c0);
-                        const float2* rxc = (const float2*)rx + c0 * L;
-                        if (freq_desync) {
-                            t4_ifo_kernel<<<(unsigned)cdiv64(nb, T4_THREADS / 32), T4_THREADS, tiles, ctx->stream>>>(fx, rxc, nb, L, p.Tg, time_desync, tg_dev + c0, fo_dev + c0, ifo_ptr + c0);
-                            ctx->launches++;
-                        }
-                        symk<<<(unsigned)(nb * groups), T4_THREADS, sym_smem, ctx->stream>>>(p, fx, rxc, nb, L, groups, tg_dev + c0, fo_dev + c0, ifo_ptr + c0, Yd_all, Yp_all);
-                        post<<<(unsigned)nb, T4_THREADS, post_smem, ctx->stream>>>(p, fx, plan_dev<float>(pl), make_devconst<float>(lp->constellation), nb, Yd_all, Yp_all,
-                                                                                   tx_bits ? tx_bits + c0 * words : nullptr, nb * stream_bits,
-                                                                                   out_bits ? out_bits + c0 * words : nullptr, (unsigned long long*)counts,
-                                                                                   tau_dev ? tau_dev + c0 : nullptr, phase_dev ? phase_dev + c0 : nullptr,
-                                                                                   H_dev ? (float2*)H_dev + c0 * p.Nc : nullptr, (float)near_eps);
-                        ctx->launches += 2;
-                        e = cudaGetLastError();
-                        if (e != cudaSuccess) rc = ctx_fail(ctx, OFDM_ERR_CUDA, "split Task-4 chain launch failed: %s", cudaGetErrorString(e));
-                    }
-                    if (bins) cudaFreeAsync(bins, ctx->stream);
+                    if (!freq_desync && ifo_dev) cudaMemsetAsync(ifo_dev, 0, sizeof(int32_t) * B, ctx->stream);
+                    t4_post_t post = q16 ? (near ? t4_post_kernel<true, true, false> : t4_post_kernel<true, false, false>)
+                                         : (near ? t4_post_kernel<false, true, false> : t4_post_kernel<false, false, false>);
+                    rc = t4_split_run(ctx, lp, p, fx, pl, post, rx, B, L, tg_dev, fo_dev, ifo_ptr, tx_bits, out_bits, counts, tau_dev, phase_dev, (float2*)H_dev,
+                                      (float)near_eps, nullptr);
                     fast_done = true;
                 } else if (fx.tw_t) {
                     cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fsmem);
@@ -1594,9 +1387,8 @@ extern "C" int ofdm_rx_chain_t4_ex(ofdm_ctx* ctx, const ofdm_link_params* lp, co
     return rc;
 }
 
-// Receiver of ofdm_sweep_sync (sweep_sync.cu, not exported; its setup and split-chain conditions are those of
-// ofdm_rx_chain_t4_ex's split path, kept in step with it): AutoCorrFunction, then the split chain t4_ifo_kernel ->
-// t4_sym_kernel -> t4_post_stats_kernel for ANY batch size (ofdm_rx_chain_t4_ex takes it from 512 streams on), so every
+// Receiver of ofdm_sweep_sync (sweep_sync.cu, not exported): AutoCorrFunction, then the split chain of ofdm_rx_chain_t4_ex
+// with t4_post_kernel's STATS instantiation for ANY batch size (ofdm_rx_chain_t4_ex takes it from 512 streams on), so every
 // estimate and decision is that of ofdm_rx_chain_t4_ex's split chain on the same streams.  tg / fo / ifo / fail are B-stream
 // scratch the call fills; nsto / cfo are the true impairments; Htrue_dev the double N_carrier table; rec the record of the
 // first stream (9 fields, stride rec_stride); row the point's counters {errors, bits, detector failures, IFO misses}, +=.
@@ -1610,76 +1402,28 @@ int ofdm_rx_t4_sync_stats(ofdm_ctx* ctx, const ofdm_link_params* lp, const void*
     ConstTable ct = host_constellation(lp->constellation);
     REQUIRE(ctx, ct.bps > 0, "unknown constellation");
     const int64_t L = (int64_t)lp->S * (lp->Nfft + lp->Tg);
+    const int64_t stream_bits = (int64_t)lp->S * lp->Nd * ct.bps;
+    REQUIRE(ctx, stream_bits % 32 == 0 || B <= T4_SPLIT_CHUNK, "the statistics chain takes at most 16,384 unaligned streams per call");
     T4Params p;
-    p.Nfft = 1024; p.logN = 10; p.Tg = lp->Tg; p.Nc = lp->N_carrier; p.S = lp->S; p.SpF = lp->SpF; p.Nd = lp->Nd; p.Np = lp->Np;
-    p.bps = ct.bps; p.scramble = lp->scramble; p.frame_bits = lp->SpF * lp->Nd * ct.bps; p.frames = lp->S / lp->SpF;
-    p.time_desync = time_desync != 0; p.freq_desync = freq_desync != 0; p.mp_desync = mp_desync != 0;
-    p.prev0 = ofdm_reg_to_prev(lp->reg0_host);
-    const int64_t stream_bits = (int64_t)p.frame_bits * p.frames;
-    REQUIRE(ctx, stream_bits % 32 == 0 || B <= 16384, "the statistics chain takes at most 16,384 unaligned streams per call");
-    std::vector<int32_t> d0(lp->Nd), p0(lp->Np);
-    for (int i = 0; i < lp->Nd; ++i) { REQUIRE(ctx, lp->data_carriers_host[i] >= 1 && lp->data_carriers_host[i] <= lp->Nfft, "data carrier out of range"); d0[i] = lp->data_carriers_host[i] - 1; }
-    for (int i = 0; i < lp->Np; ++i) {
-        REQUIRE(ctx, lp->pilot_carriers_host[i] >= 1 && lp->pilot_carriers_host[i] <= lp->N_carrier, "pilot carrier out of range");
-        REQUIRE(ctx, i == 0 || lp->pilot_carriers_host[i] > lp->pilot_carriers_host[i - 1], "pilot carriers must increase");
-        p0[i] = lp->pilot_carriers_host[i] - 1;
-    }
-    p.data0 = (const int32_t*)ctx_blob(ctx, d0.data(), sizeof(int32_t) * d0.size());
-    p.pil0 = (const int32_t*)ctx_blob(ctx, p0.data(), sizeof(int32_t) * p0.size());
-    p.pilots = (const float2*)ofdm_upload_pilots(ctx, lp->pilot_vals_host, (size_t)lp->Np * lp->S);
-    p.pilots_d = (const double2*)ctx_blob(ctx, lp->pilot_vals_host, sizeof(double) * 2 * (size_t)lp->Np * lp->S);
-    p.tw = (const float2*)ctx_twiddles(ctx, 1024);
-    std::vector<int32_t> q(lp->N_carrier);
-    for (int i = 0; i < lp->N_carrier; ++i) q[i] = i + 1;
-    const InterpPlan* pl = ctx_plan(ctx, lp->pilot_carriers_host, lp->Np, 0, q.data(), lp->N_carrier, OFDM_INTERP_SPLINE);
+    const InterpPlan* pl = nullptr;
+    int rc = t4_setup(ctx, __func__, lp, ct.bps, time_desync, freq_desync, mp_desync, p, pl);
+    if (rc) return rc;
     T4FastExtra fx;
     fx.tw_t = (const float2*)t4_twiddle_blob(ctx);
     fx.two_a = 2.f * (float)ct.re[12];
-    REQUIRE(ctx, p.data0 && p.pil0 && p.pilots && p.pilots_d && p.tw && pl && fx.tw_t, "device upload failed");
+    REQUIRE(ctx, fx.tw_t, "device upload failed");
     // the split-chain conditions of ofdm_rx_chain_t4_ex, each with its own message
-    const size_t tiles = sizeof(float2) * (size_t)(T4_THREADS / 32) * 32 * T4F_EROW;
-    const size_t post_smem = (std::max(std::max(sizeof(float) * (size_t)p.S * p.Np, 16 * (size_t)p.Np), std::max(8 * (size_t)T4_THREADS, (size_t)p.S * p.Nd)) + 15) / 16 * 16 + sizeof(float2) * ((size_t)p.S * p.Np + p.Nc + 2 * (size_t)pl->n_knots) + 32;
-    const size_t sym_smem = tiles + sizeof(float2) * 1024;
+    const size_t post_smem = t4_post_smem(p, pl);
     if (post_smem > 100 * 1024) return ctx_fail(ctx, OFDM_ERR_UNSUPPORTED, "stream shape needs %zu bytes of shared memory in the statistics kernel (at most 100 KB)", post_smem);
     if (p.Np > T4_THREADS) return ctx_fail(ctx, OFDM_ERR_UNSUPPORTED, "the statistics chain supports at most %d pilots", T4_THREADS);
     if (p.Nd > p.S * p.Np) return ctx_fail(ctx, OFDM_ERR_UNSUPPORTED, "the statistics chain needs Nd <= S * Np");
 
-    int rc = OFDM_OK;
     if (time_desync || freq_desync) rc = ofdm_cp_autocorr(ctx, rx, B, L, lp->Tg, 1024, nullptr, tg, fo, fail);
     if (rc) return rc;
-    const int64_t SPLIT_CHUNK = 16384;
-    const int64_t CH = std::min<int64_t>(B, SPLIT_CHUNK);
-    const int groups = (p.S + T4_THREADS / 32 - 1) / (T4_THREADS / 32);
-    const bool q16 = lp->constellation == OFDM_16QAM, small = p.Nc <= 416;
-    auto post = q16 ? t4_post_stats_kernel<true> : t4_post_stats_kernel<false>;
-    auto symk = small ? t4_sym_kernel<13> : t4_sym_kernel<32>;
-    CUDA_TRY(ctx, cudaFuncSetAttribute(t4_ifo_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tiles));
-    CUDA_TRY(ctx, cudaFuncSetAttribute(symk, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sym_smem));
-    CUDA_TRY(ctx, cudaFuncSetAttribute(post, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)post_smem));
-    float2* bins = nullptr;
-    CUDA_TRY(ctx, cudaMallocAsync((void**)&bins, sizeof(float2) * (size_t)CH * p.S * ((size_t)p.Nd + p.Np), ctx->stream));
-    float2* Yd_all = bins;
-    float2* Yp_all = bins + (size_t)CH * p.S * p.Nd;
-    const int64_t words = stream_bits / 32;
     T4Stats st;
-    st.Htrue = (const double2*)Htrue_dev; st.rec_stride = rec_stride;
+    st.Htrue = (const double2*)Htrue_dev; st.rec = rec; st.rec_stride = rec_stride;
+    st.tg = tg; st.fo = fo; st.ifo = ifo; st.fail = (time_desync || freq_desync) ? fail : nullptr; st.nsto = nsto; st.cfo = cfo;
     st.a_in = (float)fabs(ct.re[12]); st.a_out = (float)fabs(ct.re[8]);     // 16QAM: re = 1 and 3 (`constellation_func.m`)
-    for (int64_t c0 = 0; c0 < B && rc == OFDM_OK; c0 += CH) {
-        const int64_t nb = std::min(CH, B - c0);
-        const float2* rxc = (const float2*)rx + c0 * L;
-        if (freq_desync) {
-            t4_ifo_kernel<<<(unsigned)cdiv64(nb, T4_THREADS / 32), T4_THREADS, tiles, ctx->stream>>>(fx, rxc, nb, L, p.Tg, time_desync, tg + c0, fo + c0, ifo + c0);
-            ctx->launches++;
-        }
-        symk<<<(unsigned)(nb * groups), T4_THREADS, sym_smem, ctx->stream>>>(p, fx, rxc, nb, L, groups, tg + c0, fo + c0, ifo + c0, Yd_all, Yp_all);
-        st.rec = rec + c0; st.tg = tg + c0; st.fo = fo + c0; st.ifo = ifo + c0; st.fail = (time_desync || freq_desync) && fail ? fail + c0 : nullptr;
-        st.nsto = nsto + c0; st.cfo = cfo + c0;
-        post<<<(unsigned)nb, T4_THREADS, post_smem, ctx->stream>>>(p, fx, plan_dev<float>(pl), make_devconst<float>(lp->constellation), nb, Yd_all, Yp_all,
-                                                                   tx_bits + c0 * words, nb * stream_bits, (unsigned long long*)row, st);
-        ctx->launches += 2;
-        cudaError_t e = cudaGetLastError();
-        if (e != cudaSuccess) rc = ctx_fail(ctx, OFDM_ERR_CUDA, "statistics chain launch failed: %s", cudaGetErrorString(e));
-    }
-    cudaFreeAsync(bins, ctx->stream);
-    return rc;
+    const t4_post_t post = lp->constellation == OFDM_16QAM ? t4_post_kernel<true, false, true> : t4_post_kernel<false, false, true>;
+    return t4_split_run(ctx, lp, p, fx, pl, post, rx, B, L, tg, fo, ifo, tx_bits, nullptr, row, nullptr, nullptr, nullptr, 0.f, &st);
 }

@@ -138,6 +138,27 @@ __device__ __forceinline__ void bits_put(uint32_t* w, int64_t pos, int n, uint32
     atomicOr(&w[wi], v << sh);
     if (sh + n > 32) atomicOr(&w[wi + 1], v >> (32 - sh));
 }
+// Word w of DeScrambler(s) for a word-aligned stream of frames of frame_bits >= 64 bits, from the raw words R = s word w and
+// P = s word w - 1 (0 at w = 0): out[i] = s[i] ^ s[i-13] ^ s[i-14] on the 64-bit window (P : R).  Frames need not be word
+// aligned: where a frame starts inside the window the bits below it are replaced by the initial register's history prev0
+// (`DeScrambler.m:8-13` with the per-frame reset of `Main_model_Task_4.m:350-364`), and the word's bits before the boundary
+// keep the previous frame's history.
+__device__ __forceinline__ uint32_t descramble_word(uint32_t R, uint32_t P, int w, int frame_bits, uint32_t prev0) {
+    auto window = [](unsigned long long x) { return (uint32_t)((x ^ (x << 13) ^ (x << 14)) >> 32); };
+    const unsigned long long X = ((unsigned long long)R << 32) | P;
+    uint32_t o = window(X);
+    const int fl = (32 * w + 31) / frame_bits;                  // frame of the word's last bit
+    const int t = fl * frame_bits - 32 * w;                     // its start relative to this word: (-frame_bits, 31]
+    if (t > -14) {
+        const int sh = 32 + t;                                  // window position of the frame's first bit, 19..63
+        const unsigned long long keep = ~0ull << sh;
+        const unsigned long long hist = sh >= 32 ? ((unsigned long long)prev0 << (sh - 32)) : ((unsigned long long)prev0 >> (32 - sh));
+        const uint32_t of = window((X & keep) | (hist & ~keep));
+        const uint32_t before = t > 0 ? ((1u << t) - 1u) : 0u;  // bits of this word that still belong to the previous frame
+        o = (o & before) | (of & ~before);
+    }
+    return o;
+}
 
 // ------------------------------------------------------------------ constellation tables
 struct ConstTable {

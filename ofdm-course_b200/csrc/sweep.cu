@@ -18,8 +18,8 @@
 // the TX chain on p with its scrambler IS the TX chain on s without it (checked bit for bit in
 // tests/test_gpu_chain.py).  The three-tap descrambler runs at memory speed on 5 KB per stream, whereas the scrambler
 // inside the TX kernel is eleven log-depth doublings per frame, a quarter of that kernel's time.
-#include "common.cuh"
 #include "philox.cuh"
+#include "sweep_common.cuh"
 
 uint32_t ofdm_reg_to_prev(const uint8_t* reg);
 
@@ -61,21 +61,7 @@ __global__ void descramble_streams_kernel(const uint32_t* __restrict__ in, uint3
     if (i >= n_words) return;
     const int w = (int)(i % words_per_stream);                 // word inside its stream (streams are word aligned)
     const uint32_t R = in[i];
-    const uint32_t P = w ? in[i - 1] : 0u;
-    const unsigned long long X = ((unsigned long long)R << 32) | P;
-    uint32_t o = (uint32_t)((X ^ (X << 13) ^ (X << 14)) >> 32);
-    const int fl = (32 * w + 31) / frame_bits;                  // frame of the word's last bit
-    const int t = fl * frame_bits - 32 * w;                     // its start relative to this word: (-frame_bits, 31]
-    if (t > -14) {
-        const int sh = 32 + t;
-        const unsigned long long keep = ~0ull << sh;
-        const unsigned long long hist = sh >= 32 ? ((unsigned long long)prev0 << (sh - 32)) : ((unsigned long long)prev0 >> (32 - sh));
-        const unsigned long long Xf = (X & keep) | (hist & ~keep);
-        const uint32_t of = (uint32_t)((Xf ^ (Xf << 13) ^ (Xf << 14)) >> 32);
-        const uint32_t before = t > 0 ? ((1u << t) - 1u) : 0u;
-        o = (o & before) | (of & ~before);
-    }
-    out[i] = o;
+    out[i] = descramble_word(R, w ? in[i - 1] : 0u, w, frame_bits, prev0);
 }
 
 __global__ void fill_double_kernel(double* __restrict__ p, int64_t n, double v) {
@@ -133,21 +119,16 @@ extern "C" int ofdm_sweep_ber(ofdm_ctx* ctx, const ofdm_link_params* lp, const o
     const int64_t words = stream_bits / 32;
     const int64_t L = (int64_t)lp->S * (lp->Nfft + lp->Tg);
     const size_t esz = ctx->precision == OFDM_PREC_F64 ? sizeof(double2) : sizeof(float2);
-    int64_t tile = sp->tile_streams > 0 ? sp->tile_streams : 8192;    // whole tiles of 8,192 streams keep the persistent kernels' tails below 1 %
-    tile = std::min<int64_t>(tile, sp->streams_per_point);
 
     // multipath impulse response on the device (`get_MP_channel_resp.m:2-19`), in the context's complex type
     void* h_dev = nullptr;
     int D = 0;
     if (sp->n_taps > 0) {
-        int maxd = 0;
-        for (int k = 0; k < sp->n_taps; ++k) {
-            REQUIRE(ctx, sp->taps_host[2 * k] >= 0 && sp->taps_host[2 * k] < 4096 && sp->taps_host[2 * k] == floor(sp->taps_host[2 * k]), "tap delays must be integers in [0, 4096)");
-            maxd = std::max(maxd, (int)sp->taps_host[2 * k]);
-        }
-        D = maxd + 1;
+        std::vector<double> h;
+        REQUIRE(ctx, sweep_dense_taps(sp->taps_host, sp->n_taps, 4096, h), "tap delays must be integers in [0, 4096)");
+        D = (int)h.size();
         std::vector<double> hd(2 * (size_t)D, 0.0);
-        for (int k = 0; k < sp->n_taps; ++k) hd[2 * (size_t)sp->taps_host[2 * k]] = sp->taps_host[2 * k + 1];   // later rows overwrite, as the script's loop does
+        for (int d = 0; d < D; ++d) hd[2 * (size_t)d] = h[d];
         if (ctx->precision == OFDM_PREC_F64) h_dev = ctx_blob(ctx, hd.data(), sizeof(double) * hd.size());
         else { std::vector<float> hf(hd.begin(), hd.end()); h_dev = ctx_blob(ctx, hf.data(), sizeof(float) * hf.size()); }
         REQUIRE(ctx, h_dev != nullptr, "device upload failed");
@@ -160,48 +141,33 @@ extern "C" int ofdm_sweep_ber(ofdm_ctx* ctx, const ofdm_link_params* lp, const o
         unit_tap = ctx->precision == OFDM_PREC_F64 ? ctx_blob(ctx, one_d, sizeof one_d) : ctx_blob(ctx, one_f, sizeof one_f);
         REQUIRE(ctx, unit_tap != nullptr, "device upload failed");
     }
-    int64_t first = 0, count = 0;
-    ofdm_sweep_share((int64_t)sp->n_snr * sp->streams_per_point, sp->rank, sp->world, &first, &count);
-    if (count == 0) return OFDM_OK;
+    // whole tiles of 8,192 streams keep the persistent kernels' tails below 1 %
+    const SweepTiles tiles(sp->n_snr, sp->streams_per_point, sp->rank, sp->world, sp->tile_streams, 8192);
+    if (tiles.count == 0) return OFDM_OK;
+    const int64_t tile = tiles.tile;
 
     // stream-ordered temporaries, sized for one tile and reused by every tile of the call
-    const size_t sig_b = esz * (size_t)L * tile, bits_b = sizeof(uint32_t) * (size_t)words * tile;
     const bool t4 = sp->chain == OFDM_SWEEP_TASK4;
-    const size_t small_b = (sizeof(double) * 3 + sizeof(int32_t) * 2) * (size_t)tile + 256;
-    unsigned char* pool = nullptr;
-    const size_t sig_al = (sig_b + 255) / 256 * 256, bits_al = (bits_b + 255) / 256 * 256;
-    CUDA_TRY(ctx, cudaMallocAsync((void**)&pool, sig_al * (t4 ? 3 : 2) + 2 * bits_al + small_b, ctx->stream));
-    void* tx = pool;
-    void* rx = pool + sig_al;
-    void* tmp = t4 ? (void*)(pool + 2 * sig_al) : nullptr;
-    uint32_t* sbits = (uint32_t*)(pool + sig_al * (t4 ? 3 : 2));            // scrambled frames s (Philox)
-    uint32_t* bits = (uint32_t*)((unsigned char*)sbits + bits_al);          // payload p = DeScrambler(s): the reference bits
-    double* snr_d = (double*)((unsigned char*)bits + bits_al);
+    const size_t sig_b = esz * (size_t)L * tile, bits_b = sizeof(uint32_t) * (size_t)words * tile, d_b = sizeof(double) * tile, i_b = sizeof(int32_t) * tile;
+    SweepScratch scr(ctx);
+    CUDA_TRY(ctx, scr.alloc({sig_b, sig_b, t4 ? sig_b : 0, bits_b, bits_b, d_b, d_b, d_b, i_b, i_b}));
+    void* tx = scr.get<void>(0);
+    void* rx = scr.get<void>(1);
+    void* tmp = t4 ? scr.get<void>(2) : nullptr;
+    uint32_t* sbits = scr.get<uint32_t>(3);                                 // scrambled frames s (Philox)
+    uint32_t* bits = lp->scramble ? scr.get<uint32_t>(4) : sbits;           // payload p = DeScrambler(s): the reference bits (no scrambler: p = s)
+    double* snr_d = scr.get<double>(5);
+    double* psum = scr.get<double>(6);
+    double* cfo_d = scr.get<double>(7);
+    int32_t* sto_d = scr.get<int32_t>(8);
+    int32_t* fail_d = scr.get<int32_t>(9);
     ofdm_link_params lp_tx = *lp;                                           // the TX side maps s directly
     lp_tx.scramble = 0;
-    const int64_t frames = lp->S / lp->SpF, frame_bits = stream_bits / frames;
-    if (!lp->scramble) bits = sbits;                                        // no scrambler in the chain: p = s
-    const uint32_t prev0 = ofdm_reg_to_prev(lp->reg0_host);
-    double* psum = snr_d + tile;
-    double* cfo_d = psum + tile;
-    int32_t* sto_d = (int32_t*)(cfo_d + tile);
-    int32_t* fail_d = sto_d + tile;
 
-    int rc = OFDM_OK;
-    int64_t g = first;
-    const int64_t g_end = first + count;
-    while (g < g_end && rc == OFDM_OK) {
-        const int64_t i = g / sp->streams_per_point;                              // SNR point of this tile
-        const int64_t n = std::min<int64_t>(std::min<int64_t>(tile, g_end - g), (i + 1) * sp->streams_per_point - g);
+    const int rc = tiles.walk([&](int64_t i, int64_t, int64_t g, int64_t n) {   // i: SNR point of this tile
         int64_t* row = counts_dev + 4 * i;
-        rc = ofdm_payload_bits(ctx, sbits, n, words, sp->seed, g);
-        if (rc == OFDM_OK && lp->scramble) {
-            if (frame_bits >= 64) {
-                descramble_streams_kernel<<<(unsigned)cdiv64(n * words, 256), 256, 0, ctx->stream>>>(sbits, bits, n * words, (int)words, (int)frame_bits, prev0);
-                ctx->launches++;
-            } else rc = ofdm_descramble(ctx, sbits, bits, n * frames, frame_bits, lp->reg0_host, nullptr);
-        }
-        if (rc) break;
+        int rc = ofdm_sweep_tile_payload(ctx, lp, sbits, bits, n, words, sp->seed, g);
+        if (rc) return rc;
         fill_double_kernel<<<(unsigned)cdiv64(n, 256), 256, 0, ctx->stream>>>(snr_d, n, sp->snr_db_host[i]);
         ctx->launches++;
         if (!t4) {
@@ -231,16 +197,13 @@ extern "C" int ofdm_sweep_ber(ofdm_ctx* ctx, const ofdm_link_params* lp, const o
                 ctx->launches++;
             }
         }
-        g += n;
-    }
-    cudaError_t e = cudaGetLastError();
-    if (rc == OFDM_OK && e != cudaSuccess) rc = ctx_fail(ctx, OFDM_ERR_CUDA, "sweep launch failed: %s", cudaGetErrorString(e));
-    cudaFreeAsync(pool, ctx->stream);
-    return rc;
+        return rc;
+    });
+    return scr.finish(rc, "sweep launch failed");
 }
 
-// The payload of streams g .. g + n - 1 exactly as ofdm_sweep_ber draws it (not exported; ofdm_sweep_sync uses it): Philox
-// words s into sbits, and p = DeScrambler(s) into bits when the chain scrambles (otherwise p = s and bits is not written).
+// The payload of streams g .. g + n - 1 exactly as ofdm_sweep_ber draws it (not exported): Philox words s into sbits, and
+// p = DeScrambler(s) into bits when the chain scrambles (otherwise p = s and bits is not written).
 int ofdm_sweep_tile_payload(ofdm_ctx* ctx, const ofdm_link_params* lp, uint32_t* sbits, uint32_t* bits, int64_t n, int64_t words, uint64_t seed, int64_t g) {
     int rc = ofdm_payload_bits(ctx, sbits, n, words, seed, g);
     if (rc != OFDM_OK || !lp->scramble) return rc;

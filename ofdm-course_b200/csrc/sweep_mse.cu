@@ -16,6 +16,7 @@
 #include "fft.cuh"
 #include "philox.cuh"
 #include "pursuit_common.cuh"
+#include "sweep_common.cuh"
 
 int ofdm_stream_power_sum(ofdm_ctx* ctx, const void* in, int64_t B, int64_t L, double* power_sum);
 int ofdm_mmse_ce_meas(ofdm_ctx* ctx, const void* y, int64_t B, const int32_t* loc, int Np, int Nc, const void* h, int h_len, const double* snr_db,
@@ -113,12 +114,9 @@ extern "C" int ofdm_sweep_mse(ofdm_ctx* ctx, const ofdm_link_params* lp, const o
     REQUIRE(ctx, Ldict >= Np, "Ldict must be >= Np (MP_estimate searches the first Np columns)");
     REQUIRE(ctx, Ldict <= Nfft, "Ldict must be <= Nfft");
     REQUIRE(ctx, lp->Nd >= 0 && (lp->Nd == 0 || lp->data_carriers_host), "bad data-carrier list");
-    int D = 0;
-    for (int k = 0; k < K; ++k) {
-        const double d = sp->taps_host[2 * k];
-        REQUIRE(ctx, d >= 0 && d < Nfft && d == floor(d), "tap delays must be integers in [0, Nfft)");
-        D = std::max(D, (int)d + 1);
-    }
+    std::vector<double> h;                                    // later rows overwrite, as `get_MP_channel_resp.m:14`
+    REQUIRE(ctx, sweep_dense_taps(sp->taps_host, K, Nfft, h), "tap delays must be integers in [0, Nfft)");
+    const int D = (int)h.size();
     const int64_t L = (int64_t)S * (Nfft + Tg);
     const size_t esz = f64 ? sizeof(double2) : sizeof(float2);
     int64_t words = 0;
@@ -130,9 +128,7 @@ extern "C" int ofdm_sweep_mse(ofdm_ctx* ctx, const ofdm_link_params* lp, const o
         words = stream_bits / 32;
     }
 
-    // the channel's non-zero taps in ascending delay, in the context's type (later rows overwrite, as `get_MP_channel_resp.m:14`)
-    std::vector<double> h(D, 0.0);
-    for (int k = 0; k < K; ++k) h[(int)sp->taps_host[2 * k]] = sp->taps_host[2 * k + 1];
+    // the channel's non-zero taps in ascending delay, in the context's type
     std::vector<double> hv_d;
     std::vector<float> hv_f;
     std::vector<int> hd;
@@ -156,33 +152,28 @@ extern "C" int ofdm_sweep_mse(ofdm_ctx* ctx, const ofdm_link_params* lp, const o
     const size_t fe_smem = esz * (size_t)(2 * Nfft + D - 1) + (esz + sizeof(int)) * (size_t)nnz;
     REQUIRE(ctx, fe_smem <= 227 * 1024, "symbol too long for the shared-memory front end");
 
-    int64_t first = 0, count = 0;
-    ofdm_sweep_share((int64_t)sp->n_snr * sp->streams_per_point, sp->rank, sp->world, &first, &count);
-    if (count == 0) return OFDM_OK;
-    int64_t tile = sp->tile_streams > 0 ? sp->tile_streams : 8192;
-    tile = std::min<int64_t>(tile, sp->streams_per_point);
+    const SweepTiles tiles(sp->n_snr, sp->streams_per_point, sp->rank, sp->world, sp->tile_streams, 8192);
+    if (tiles.count == 0) return OFDM_OK;
+    const int64_t tile = tiles.tile;
 
     // stream-ordered temporaries, sized for one tile and reused by every tile of the call
     const bool shared_tx = lp->Nd == 0;                       // pilots only (`Main_model_Task_5.m:24-33`): one TX stream for all
-    auto al = [](size_t x) { return (x + 255) / 256 * 256; };
-    const size_t b_Ht = al(esz * Nfft), b_ps = al(sizeof(double) * tile), b_snr = b_ps, b_near = al(sizeof(int32_t) * tile),
-                 b_y = al(esz * (size_t)tile * Np), b_nc = al(esz * (size_t)tile * Nc), b_pur = al(esz * (size_t)tile * Nfft),
-                 b_tx = al(esz * (size_t)L * (shared_tx ? 1 : tile)), b_aux = shared_tx ? al(esz * (size_t)S * Nfft) : al(sizeof(uint32_t) * (size_t)words * tile);
-    unsigned char* pool = nullptr;
-    CUDA_TRY(ctx, cudaMallocAsync((void**)&pool, b_Ht + b_ps + 2 * b_snr + b_near + b_y + 3 * b_nc + b_pur + b_tx + b_aux, ctx->stream));
-    unsigned char* q = pool;
-    void* Htrue = q; q += b_Ht;
-    double* psum = (double*)q; q += b_ps;
-    double* snr_d = (double*)q; q += b_snr;
-    void* sigma = q; q += b_snr;
-    int32_t* near = (int32_t*)q; q += b_near;
-    void* y = q; q += b_y;
-    void* Hls = q; q += b_nc;
-    void* hls = q; q += b_nc;
-    void* Hmm = q; q += b_nc;
-    void* Hpur = q; q += b_pur;
-    void* tx = q; q += b_tx;
-    void* aux = q;                                            // TX grid (pilots only) or the payload words of a tile
+    const size_t b_d = sizeof(double) * tile, b_nc = esz * (size_t)tile * Nc;
+    SweepScratch scr(ctx);
+    CUDA_TRY(ctx, scr.alloc({esz * Nfft, b_d, b_d, b_d, sizeof(int32_t) * tile, esz * (size_t)tile * Np, b_nc, b_nc, b_nc, esz * (size_t)tile * Nfft,
+                             esz * (size_t)L * (shared_tx ? 1 : tile), shared_tx ? esz * (size_t)S * Nfft : sizeof(uint32_t) * (size_t)words * tile}));
+    void* Htrue = scr.get<void>(0);
+    double* psum = scr.get<double>(1);
+    double* snr_d = scr.get<double>(2);
+    void* sigma = scr.get<void>(3);
+    int32_t* near = scr.get<int32_t>(4);
+    void* y = scr.get<void>(5);
+    void* Hls = scr.get<void>(6);
+    void* hls = scr.get<void>(7);
+    void* Hmm = scr.get<void>(8);
+    void* Hpur = scr.get<void>(9);
+    void* tx = scr.get<void>(10);
+    void* aux = scr.get<void>(11);                            // TX grid (pilots only) or the payload words of a tile
 
     int rc = OFDM_OK;
     {
@@ -204,16 +195,13 @@ extern "C" int ofdm_sweep_mse(ofdm_ctx* ctx, const ofdm_link_params* lp, const o
     }
 
     const int64_t spp = sp->streams_per_point;
-    int64_t g = first;
-    const int64_t g_end = first + count;
-    while (g < g_end && rc == OFDM_OK) {
-        const int64_t i = g / spp;                                                    // SNR point of this tile
-        const int64_t n = std::min<int64_t>(std::min<int64_t>(tile, g_end - g), (i + 1) * spp - g);
+    if (rc == OFDM_OK) rc = tiles.walk([&](int64_t i, int64_t j0, int64_t g, int64_t n) {   // i: SNR point of this tile
         const double snr = sp->snr_db_host[i];
+        int rc = OFDM_OK;
         if (!shared_tx) {
             rc = ofdm_payload_bits(ctx, (uint32_t*)aux, n, words, sp->seed, g);
             if (rc == OFDM_OK) rc = ofdm_tx_chain_p(ctx, &lp_tx, (const uint32_t*)aux, n, tx, psum);
-            if (rc) break;
+            if (rc) return rc;
         }
         DISPATCH_T(ctx, {
             mse_prep_kernel<T><<<(unsigned)cdiv64(n, 256), 256, 0, ctx->stream>>>(n, L, snr, psum, shared_tx ? 0 : 1, snr_d, (T*)sigma);
@@ -222,7 +210,7 @@ extern "C" int ofdm_sweep_mse(ofdm_ctx* ctx, const ofdm_link_params* lp, const o
                 (const cx<T>*)tw, p0_dev, (const cx<T>*)xp_dev, Np, (cx<T>*)y);
         });
         ctx->launches += 2;
-        double* row = mse_dev + (size_t)i * 4 * spp + (g - i * spp);                  // [i][e][j], e = LS, MMSE, MP, OMP
+        double* row = mse_dev + (size_t)i * 4 * spp + j0;                             // [i][e][j], e = LS, MMSE, MP, OMP
         rc = ofdm_interpolate(ctx, y, n, lp->pilot_carriers_host, Np, Nc, OFDM_INTERP_SPLINE, Hls);         // LS_CE
         if (rc == OFDM_OK) rc = ofdm_fft(ctx, Hls, hls, n, Nc, 1);                                              // h = ifft(H_LS), `:179`
         if (rc == OFDM_OK) rc = ofdm_mmse_ce_meas(ctx, y, n, lp->pilot_carriers_host, Np, Nc, hls, Nc, snr_d, Hmm);
@@ -237,10 +225,7 @@ extern "C" int ofdm_sweep_mse(ofdm_ctx* ctx, const ofdm_link_params* lp, const o
             mse_counts_kernel<<<1, 256, 0, ctx->stream>>>(near, n, counts_dev + 2 * i);
             ctx->launches++;
         }
-        g += n;
-    }
-    cudaError_t e = cudaGetLastError();
-    if (rc == OFDM_OK && e != cudaSuccess) rc = ctx_fail(ctx, OFDM_ERR_CUDA, "MSE sweep launch failed: %s", cudaGetErrorString(e));
-    cudaFreeAsync(pool, ctx->stream);
-    return rc;
+        return rc;
+    });
+    return scr.finish(rc, "MSE sweep launch failed");
 }

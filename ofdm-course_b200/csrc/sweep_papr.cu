@@ -8,8 +8,8 @@
 // point's scramble flag, then papr_stats_kernel (papr.cu), which turns the TX streams into the point's window-PAPR histogram
 // and the per-stream PAPR without storing a window value.  The payload depends on j only, so the points of one study
 // transmit the same payloads: plain against scrambled is a paired comparison, as the reference's one image is.
-#include "common.cuh"
 #include "philox.cuh"
+#include "sweep_common.cuh"
 
 #include <cmath>
 
@@ -117,37 +117,29 @@ extern "C" int ofdm_sweep_papr(ofdm_ctx* ctx, const ofdm_link_params* lp, const 
     const int64_t L = (int64_t)lp->S * (lp->Nfft + lp->Tg);
     const int64_t spp = pp->streams_per_point;
 
-    int64_t first = 0, count = 0;
-    ofdm_sweep_share((int64_t)pp->n_points * spp, pp->rank, pp->world, &first, &count);
-    if (count == 0) return OFDM_OK;
-    int64_t tile = pp->tile_streams > 0 ? pp->tile_streams : 8192;   // 3.8 GB of FP32 signal at the Task-2 shape
-    tile = std::min<int64_t>(tile, spp);
+    const SweepTiles tiles(pp->n_points, spp, pp->rank, pp->world, pp->tile_streams, 8192);   // 3.8 GB of FP32 signal at the Task-2 shape
+    if (tiles.count == 0) return OFDM_OK;
+    const int64_t tile = tiles.tile;
 
     // one stream-ordered allocation per call: signal, payload, power sums, maxima and (when given) the pool.  The pool is
     // not put in the context's blob cache: a call must not evict other tables, nor keep a large pool alive after it returns.
     const size_t esz = ctx->precision == OFDM_PREC_F64 ? sizeof(double2) : sizeof(float2);
-    auto al = [](size_t x) { return (x + 255) / 256 * 256; };
     const int64_t pool_words = pp->pool_host ? cdiv64(pp->pool_bits, 32) : 0;
-    const size_t b_sig = al(esz * (size_t)L * tile), b_bits = al(sizeof(uint32_t) * (size_t)(cdiv64(tile * stream_bits, 32) + 1)),
-                 b_d = al(sizeof(double) * tile), b_pool = al(sizeof(uint32_t) * (size_t)pool_words);
-    unsigned char* buf = nullptr;
-    CUDA_TRY(ctx, cudaMallocAsync((void**)&buf, b_sig + b_bits + 2 * b_d + b_pool, ctx->stream));
-    unsigned char* q = buf;
-    void* tx = q; q += b_sig;
-    uint32_t* bits = (uint32_t*)q; q += b_bits;
-    double* psum = (double*)q; q += b_d;
-    unsigned long long* peak = (unsigned long long*)q; q += b_d;
-    uint32_t* pool = pp->pool_host ? (uint32_t*)q : nullptr;
+    SweepScratch scr(ctx);
+    CUDA_TRY(ctx, scr.alloc({esz * (size_t)L * tile, sizeof(uint32_t) * (size_t)(cdiv64(tile * stream_bits, 32) + 1), sizeof(double) * tile,
+                             sizeof(double) * tile, sizeof(uint32_t) * (size_t)pool_words}));
+    void* tx = scr.get<void>(0);
+    uint32_t* bits = scr.get<uint32_t>(1);
+    double* psum = scr.get<double>(2);
+    unsigned long long* peak = scr.get<unsigned long long>(3);
+    uint32_t* pool = pp->pool_host ? scr.get<uint32_t>(4) : nullptr;
     if (pool) rc = cudaMemcpyAsync(pool, pp->pool_host, sizeof(uint32_t) * (size_t)pool_words, cudaMemcpyHostToDevice, ctx->stream) == cudaSuccess
                        ? OFDM_OK : ctx_fail(ctx, OFDM_ERR_CUDA, "ofdm_sweep_papr: pool upload failed");
     const int64_t stride = pp->pool_host ? pp->pool_stride % pp->pool_bits : 0;
 
     ofdm_link_params lpk = *lp;
-    int64_t g = first;
-    const int64_t g_end = first + count;
-    while (g < g_end && rc == OFDM_OK) {
-        const int64_t k = g / spp, j0 = g - k * spp;                   // point and first stream of this tile
-        const int64_t n = std::min<int64_t>(std::min<int64_t>(tile, g_end - g), (k + 1) * spp - g);
+    if (rc == OFDM_OK) rc = tiles.walk([&](int64_t k, int64_t j0, int64_t g, int64_t n) {   // point and first stream of this tile
+        int rc = OFDM_OK;
         if (pool) {
             const int64_t total = n * stream_bits;
             pool_bits_kernel<<<(unsigned)cdiv64(cdiv64(total, 32), 256), 256, 0, ctx->stream>>>(pool, pp->pool_bits, stride, bits, total, stream_bits, j0);
@@ -157,10 +149,7 @@ extern "C" int ofdm_sweep_papr(ofdm_ctx* ctx, const ofdm_link_params* lp, const 
         if (rc == OFDM_OK) rc = ofdm_tx_chain_p(ctx, &lpk, bits, n, tx, psum);
         if (rc == OFDM_OK)
             rc = ofdm_papr_stats(ctx, tx, n, L, lp->Nfft, psum, pp->bin_db, pp->n_bins, hist_dev + k * pp->n_bins, papr_dev + g, peak);
-        g += n;
-    }
-    cudaError_t e = cudaGetLastError();
-    if (rc == OFDM_OK && e != cudaSuccess) rc = ctx_fail(ctx, OFDM_ERR_CUDA, "ofdm_sweep_papr launch failed: %s", cudaGetErrorString(e));
-    cudaFreeAsync(buf, ctx->stream);
-    return rc;
+        return rc;
+    });
+    return scr.finish(rc, "ofdm_sweep_papr launch failed");
 }

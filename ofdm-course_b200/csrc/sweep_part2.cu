@@ -19,6 +19,7 @@
 // Each (point, estimator, run) NMSE cell is written by exactly one call; counters are integer sums.  No floating-point atomics.
 #include "fft.cuh"
 #include "pursuit_common.cuh"
+#include "sweep_common.cuh"
 
 int ofdm_mmse_ce_meas(ofdm_ctx* ctx, const void* y, int64_t B, const int32_t* loc, int Np, int Nc, const void* h, int h_len, const double* snr_db,
                       void* H);
@@ -200,41 +201,35 @@ extern "C" int ofdm_sweep_part2(ofdm_ctx* ctx, const ofdm_link_params* base, con
     const size_t smem = p2_smem(esz, Nfft, D);
     REQUIRE(ctx, smem <= 227 * 1024, "symbol plus fading response too long for the shared-memory kernels");
 
-    int64_t first = 0, count = 0;
-    ofdm_sweep_share((int64_t)P * pp->mc_runs, pp->rank, pp->world, &first, &count);
-    if (count == 0) return OFDM_OK;
-    const int64_t tile = std::min<int64_t>(pp->tile_runs > 0 ? pp->tile_runs : P2_DEFAULT_TILE, pp->mc_runs);
+    const SweepTiles tiles(P, pp->mc_runs, pp->rank, pp->world, pp->tile_runs, P2_DEFAULT_TILE);
+    if (tiles.count == 0) return OFDM_OK;
+    const int64_t tile = tiles.tile;
     const int64_t L = (int64_t)S * (Nfft + Tg);
 
     // stream-ordered temporaries, sized for one tile and reused by every tile of the call
-    auto al = [](size_t x) { return (x + 255) / 256 * 256; };
-    const size_t b_sig = al(esz * (size_t)L), b_h = al(esz * (size_t)tile * D), b_y = al(esz * (size_t)tile * Nc),
-                 b_nc = al(esz * (size_t)tile * Nc), b_nf = al(esz * (size_t)tile * Nfft), b_snr = al(sizeof(double) * tile),
-                 b_near = al(sizeof(int32_t) * tile), b_idx = al(sizeof(int32_t) * Nc), b_xp = al(esz * Nc),
-                 b_pay = al(sizeof(uint32_t) * (size_t)OFDM_BIT_WORDS(max_bits));
-    unsigned char* pool = nullptr;
-    CUDA_TRY(ctx, cudaMallocAsync((void**)&pool, 2 * b_sig + b_h + b_y + 3 * b_nc + 3 * b_nf + b_snr + b_near + 2 * b_idx + b_xp + b_pay,
-                                  ctx->stream));
-    unsigned char* q = pool;
-    void* tx = q; q += b_sig;
-    void* txn = q; q += b_sig;
-    void* h = q; q += b_h;
-    void* y = q; q += b_y;                                    // y of up to Nc pilots
-    void* hpad = q; q += b_nc;                                // true CIR zero-padded to N_carrier (the MMSE input, `:176-177`)
-    void* Hls = q; q += b_nc;
-    void* Hmm = q; q += b_nc;
-    void* Hf = q; q += b_nf;                                  // fft(h zero-padded to Nfft), `:155`
-    void* Hmp = q; q += b_nf;                                 // first holds h zero-padded to Nfft
-    void* Homp = q; q += b_nf;
-    double* snr_d = (double*)q; q += b_snr;
-    int32_t* near = (int32_t*)q; q += b_near;
+    const size_t b_sig = esz * (size_t)L, b_nc = esz * (size_t)tile * Nc, b_nf = esz * (size_t)tile * Nfft, b_idx = sizeof(int32_t) * Nc;
+    SweepScratch scr(ctx);
+    CUDA_TRY(ctx, scr.alloc({b_sig, b_sig, esz * (size_t)tile * D, b_nc, b_nc, b_nc, b_nc, b_nf, b_nf, b_nf, sizeof(double) * tile, sizeof(int32_t) * tile,
+                             b_idx, b_idx, esz * Nc, sizeof(uint32_t) * (size_t)OFDM_BIT_WORDS(max_bits)}));
+    void* tx = scr.get<void>(0);
+    void* txn = scr.get<void>(1);
+    void* h = scr.get<void>(2);
+    void* y = scr.get<void>(3);                               // y of up to Nc pilots
+    void* hpad = scr.get<void>(4);                            // true CIR zero-padded to N_carrier (the MMSE input, `:176-177`)
+    void* Hls = scr.get<void>(5);
+    void* Hmm = scr.get<void>(6);
+    void* Hf = scr.get<void>(7);                              // fft(h zero-padded to Nfft), `:155`
+    void* Hmp = scr.get<void>(8);                             // first holds h zero-padded to Nfft
+    void* Homp = scr.get<void>(9);
+    double* snr_d = scr.get<double>(10);
+    int32_t* near = scr.get<int32_t>(11);
     // The per-point inputs that kernels read across the tiles of a point, and the SNR, live in this pool and not in the
     // context's blob cache: a call over many layouts uploads new blobs at every point (ofdm_tx_chain's tables), and the cache
     // frees a generation that is no longer requested.  Blobs fetched inside a callee are only read by its own launches.
-    int32_t* p0_dev = (int32_t*)q; q += b_idx;                // the point's pilots, 0-based
-    int32_t* dc0_dev = (int32_t*)q; q += b_idx;               // the point's data carriers, 0-based
-    void* xp_dev = q; q += b_xp;                              // pilotValues(:,1) in the context's type
-    uint32_t* pay_dev = (uint32_t*)q;                         // the point's payload prefix
+    int32_t* p0_dev = scr.get<int32_t>(12);                   // the point's pilots, 0-based
+    int32_t* dc0_dev = scr.get<int32_t>(13);                  // the point's data carriers, 0-based
+    void* xp_dev = scr.get<void>(14);                         // pilotValues(:,1) in the context's type
+    uint32_t* pay_dev = scr.get<uint32_t>(15);                // the point's payload prefix
 
     int rc = OFDM_OK;
     auto ck = [ctx](cudaError_t e) { return e == cudaSuccess ? OFDM_OK : ctx_fail(ctx, OFDM_ERR_CUDA, "part-2 sweep: %s", cudaGetErrorString(e)); };
@@ -259,12 +254,9 @@ extern "C" int ofdm_sweep_part2(ofdm_ctx* ctx, const ofdm_link_params* base, con
     const int32_t* pc = nullptr;
     int64_t stream_bits = 0;
 
-    int64_t g = first;
-    const int64_t g_end = first + count;
-    while (g < g_end && rc == OFDM_OK) {
-        const int k = (int)(g / pp->mc_runs);
-        const int64_t r0 = g - (int64_t)k * pp->mc_runs;
-        const int64_t n = std::min<int64_t>(std::min<int64_t>(tile, g_end - g), pp->mc_runs - r0);
+    if (rc == OFDM_OK) rc = tiles.walk([&](int64_t point, int64_t r0, int64_t, int64_t n) {
+        const int k = (int)point;
+        int rc = OFDM_OK;
         if (k != cur) {
             // the point's layout (`Task5_part2.m:50-80`): data carriers are the complement of the pilots in 1..N_carrier
             pc = pp->pilot_carriers_host + off[k];
@@ -295,7 +287,7 @@ extern "C" int ofdm_sweep_part2(ofdm_ctx* ctx, const ofdm_link_params* base, con
                             : cudaMemcpyAsync(xp_dev, xp_f.data(), esz * Np, cudaMemcpyHostToDevice, ctx->stream));
             if (rc == OFDM_OK)
                 rc = ck(cudaMemcpyAsync(pay_dev, words.data(), sizeof(uint32_t) * words.size(), cudaMemcpyHostToDevice, ctx->stream));
-            if (rc) break;
+            if (rc) return rc;
             ofdm_link_params lk = *base;                             // scrambling off, as `Task5_part2.m:99-115`
             lk.Nd = Nd; lk.Np = Np;
             lk.data_carriers_host = dc.data(); lk.pilot_carriers_host = pc; lk.pilot_vals_host = pv.data();
@@ -303,11 +295,11 @@ extern "C" int ofdm_sweep_part2(ofdm_ctx* ctx, const ofdm_link_params* base, con
             if (!lk.reg0_host) lk.reg0_host = no_register;           // read only when scrambling
             rc = ofdm_tx_chain(ctx, &lk, pay_dev, 1, tx);
             if (rc == OFDM_OK) rc = ofdm_add_noise(ctx, tx, 1, L, snr_d, nullptr, pp->seed, k, txn, nullptr);   // once per point, `:132`
-            if (rc) break;
+            if (rc) return rc;
             cur = k;
         }
         rc = ofdm_tdl_channel(ctx, pp->profile, pp->fs_hz, n, pp->seed, (int64_t)k * P2_RUN_KEY + r0, D, h, nullptr);
-        if (rc) break;
+        if (rc) return rc;
         DISPATCH_T(ctx, {
             part2_front_end_kernel<T><<<(unsigned)n, P2_THREADS, smem, ctx->stream>>>((const cx<T>*)txn, L, (const cx<T>*)h, D, Nfft, ilog2(Nfft), Tg,
                                                                                      (const cx<T>*)tw, p0_dev, (const cx<T>*)xp_dev, Np, (cx<T>*)y);
@@ -329,7 +321,7 @@ extern "C" int ofdm_sweep_part2(ofdm_ctx* ctx, const ofdm_link_params* base, con
         if (rc == OFDM_OK) rc = ofdm_mse(ctx, Hf, Nfft, Hmm, Nc, n, Nc, row + pp->mc_runs);
         if (rc == OFDM_OK) rc = ofdm_mse(ctx, Hf, Nfft, Hmp, Nfft, n, Nc, row + 2 * pp->mc_runs);
         if (rc == OFDM_OK) rc = ofdm_mse(ctx, Hf, Nfft, Homp, Nfft, n, Nc, row + 3 * pp->mc_runs);
-        if (rc) break;
+        if (rc) return rc;
         int64_t* cnt = counts_dev + (size_t)k * 12;
         DISPATCH_T(ctx, {
             P2Est<T> est;
@@ -341,10 +333,7 @@ extern "C" int ofdm_sweep_part2(ofdm_ctx* ctx, const ofdm_link_params* base, con
         });
         part2_runs_kernel<<<1, 256, 0, ctx->stream>>>(near, n, stream_bits, runs_dev + 2 * (size_t)k, cnt);
         ctx->launches += 2;
-        g += n;
-    }
-    cudaError_t e = cudaGetLastError();
-    if (rc == OFDM_OK && e != cudaSuccess) rc = ctx_fail(ctx, OFDM_ERR_CUDA, "part-2 sweep launch failed: %s", cudaGetErrorString(e));
-    cudaFreeAsync(pool, ctx->stream);
-    return rc;
+        return OFDM_OK;
+    });
+    return scr.finish(rc, "part-2 sweep launch failed");
 }

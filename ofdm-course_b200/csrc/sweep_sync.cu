@@ -5,14 +5,13 @@
 // and the MER of every run (`:374`).  This call runs the Task-4 chain of ofdm_sweep_ber -- same share rule (ofdm_sweep_share),
 // stream numbering g = snr_index * streams_per_point + j, tiles that never straddle a point, and the Philox keys of the
 // payload, noise and STO / CFO draws -- so with sto_mode 0 and every desync flag on it transmits the same streams.  The
-// receiver is the split Task-4 chain with a statistics variant of its last kernel (chain_rx_t4.cu: t4_post_stats_kernel),
+// receiver is the split Task-4 chain with the statistics variant of its last kernel (chain_rx_t4.cu: t4_post_kernel's STATS),
 // which writes one record per stream and adds to the point's counters; the estimated response is never stored.
 // Streams need not be word aligned (Task 4 at 25 % pilots: 59,800 bits): stream g then carries the first stream_bits bits of
 // the Philox words ofdm_payload_bits draws for it (ceil(stream_bits / 32) words), packed into one contiguous bitstream.
 // Every record cell is written by exactly one rank, counters are integer atomics, so the caller's sums over ranks are exact.
-#include "common.cuh"
+#include "sweep_common.cuh"
 
-int ofdm_sweep_tile_payload(ofdm_ctx* ctx, const ofdm_link_params* lp, uint32_t* sbits, uint32_t* bits, int64_t n, int64_t words, uint64_t seed, int64_t g);
 int ofdm_rx_t4_sync_stats(ofdm_ctx* ctx, const ofdm_link_params* lp, const void* rx, int64_t B, int time_desync, int freq_desync, int mp_desync,
                           const uint32_t* tx_bits, int64_t* row, int32_t* tg, double* fo, int32_t* ifo, int32_t* fail, const int32_t* nsto,
                           const double* cfo, const double* Htrue_dev, double* rec, int64_t rec_stride);
@@ -75,18 +74,10 @@ extern "C" int ofdm_sweep_sync(ofdm_ctx* ctx, const ofdm_link_params* lp, const 
 
     // the channel: impulse response in FP32 for the channel kernel, and the true response H(1:N_carrier) in double
     // (`get_MP_channel_resp.m:2-19`: later rows overwrite; H = fft(h, Nfft)), one table per call
-    int D = 1;
     std::vector<double> h(1, 1.0);                                                  // no multipath: a single unit tap, H = 1
-    if (sp->n_taps > 0) {
-        D = 0;
-        for (int k = 0; k < sp->n_taps; ++k) {
-            const double d = sp->taps_host[2 * k];
-            REQUIRE(ctx, d >= 0 && d < Nfft && d == floor(d), "ofdm_sweep_sync: tap delays must be integers in [0, Nfft)");
-            D = std::max(D, (int)d + 1);
-        }
-        h.assign(D, 0.0);
-        for (int k = 0; k < sp->n_taps; ++k) h[(int)sp->taps_host[2 * k]] = sp->taps_host[2 * k + 1];
-    }
+    if (sp->n_taps > 0)
+        REQUIRE(ctx, sweep_dense_taps(sp->taps_host, sp->n_taps, Nfft, h), "ofdm_sweep_sync: tap delays must be integers in [0, Nfft)");
+    const int D = (int)h.size();
     std::vector<float> hf(2 * (size_t)D, 0.f);
     for (int d = 0; d < D; ++d) hf[2 * d] = (float)h[d];
     std::vector<double> Ht(2 * (size_t)Nc, 0.0);
@@ -104,44 +95,35 @@ extern "C" int ofdm_sweep_sync(ofdm_ctx* ctx, const ofdm_link_params* lp, const 
     const double* Ht_dev = (const double*)ctx_blob(ctx, Ht.data(), sizeof(double) * Ht.size());
     REQUIRE(ctx, h_dev && Ht_dev, "ofdm_sweep_sync: device upload failed");
 
-    int64_t first = 0, count = 0;
-    ofdm_sweep_share((int64_t)sp->n_snr * sp->streams_per_point, sp->rank, sp->world, &first, &count);
-    if (count == 0) return OFDM_OK;
-    int64_t tile = sp->tile_streams > 0 ? sp->tile_streams : 8192;
-    tile = std::min<int64_t>(tile, sp->streams_per_point);
-    if (!aligned) tile = std::min<int64_t>(tile, 16384);                            // the receiver takes unaligned streams in one pass
+    SweepTiles tiles(sp->n_snr, sp->streams_per_point, sp->rank, sp->world, sp->tile_streams, 8192);
+    if (tiles.count == 0) return OFDM_OK;
+    if (!aligned) tiles.tile = std::min<int64_t>(tiles.tile, 16384);               // the receiver takes unaligned streams in one pass
+    const int64_t tile = tiles.tile;
 
     // stream-ordered temporaries, sized for one tile and reused by every tile of the call
-    auto al = [](size_t x) { return (x + 255) / 256 * 256; };
-    const size_t b_sig = al(sizeof(float2) * (size_t)L * tile), b_bits = al(sizeof(uint32_t) * (size_t)(words + 1) * tile), b_d = al(sizeof(double) * tile),
-                 b_i = al(sizeof(int32_t) * tile);
-    unsigned char* pool = nullptr;
-    CUDA_TRY(ctx, cudaMallocAsync((void**)&pool, 2 * b_sig + (aligned ? 2 : 3) * b_bits + 4 * b_d + 4 * b_i, ctx->stream));
-    unsigned char* q = pool;
-    void* tx = q; q += b_sig;
-    void* rx = q; q += b_sig;
-    uint32_t* sbits = (uint32_t*)q; q += b_bits;                                     // scrambled frames s (Philox)
-    uint32_t* bits = (uint32_t*)q; q += b_bits;                                      // payload p = DeScrambler(s)
-    double* snr_d = (double*)q; q += b_d;
-    double* psum = (double*)q; q += b_d;
-    double* cfo_d = (double*)q; q += b_d;
-    double* fo_d = (double*)q; q += b_d;
-    int32_t* sto_d = (int32_t*)q; q += b_i;
-    int32_t* tg_d = (int32_t*)q; q += b_i;
-    int32_t* ifo_d = (int32_t*)q; q += b_i;
-    int32_t* fail_d = (int32_t*)q; q += b_i;
-    uint32_t* raw = aligned ? nullptr : (uint32_t*)q;                                // padded Philox words of unaligned streams
-    if (!lp->scramble) bits = sbits;
+    const size_t b_sig = sizeof(float2) * (size_t)L * tile, b_bits = sizeof(uint32_t) * (size_t)(words + 1) * tile, b_d = sizeof(double) * tile,
+                 b_i = sizeof(int32_t) * tile;
+    SweepScratch scr(ctx);
+    CUDA_TRY(ctx, scr.alloc({b_sig, b_sig, b_bits, b_bits, b_d, b_d, b_d, b_d, b_i, b_i, b_i, b_i, aligned ? 0 : b_bits}));
+    void* tx = scr.get<void>(0);
+    void* rx = scr.get<void>(1);
+    uint32_t* sbits = scr.get<uint32_t>(2);                                          // scrambled frames s (Philox)
+    uint32_t* bits = lp->scramble ? scr.get<uint32_t>(3) : sbits;                    // payload p = DeScrambler(s)
+    double* snr_d = scr.get<double>(4);
+    double* psum = scr.get<double>(5);
+    double* cfo_d = scr.get<double>(6);
+    double* fo_d = scr.get<double>(7);
+    int32_t* sto_d = scr.get<int32_t>(8);
+    int32_t* tg_d = scr.get<int32_t>(9);
+    int32_t* ifo_d = scr.get<int32_t>(10);
+    int32_t* fail_d = scr.get<int32_t>(11);
+    uint32_t* raw = scr.get<uint32_t>(12);                                           // padded Philox words of unaligned streams
     ofdm_link_params lp_tx = *lp;                                                    // as ofdm_sweep_ber: the TX maps s directly
     lp_tx.scramble = 0;
 
     const int64_t spp = sp->streams_per_point;
-    int rc = OFDM_OK;
-    int64_t g = first;
-    const int64_t g_end = first + count;
-    while (g < g_end && rc == OFDM_OK) {
-        const int64_t i = g / spp;                                                   // SNR point of this tile
-        const int64_t n = std::min<int64_t>(std::min<int64_t>(tile, g_end - g), (i + 1) * spp - g);
+    const int rc = tiles.walk([&](int64_t i, int64_t j0, int64_t g, int64_t n) {      // i: SNR point of this tile
+        int rc;
         if (aligned) rc = ofdm_sweep_tile_payload(ctx, lp, sbits, bits, n, words, sp->seed, g);
         else {
             rc = ofdm_payload_bits(ctx, raw, n, words, sp->seed, g);
@@ -151,7 +133,7 @@ extern "C" int ofdm_sweep_sync(ofdm_ctx* ctx, const ofdm_link_params* lp, const 
             }
             if (rc == OFDM_OK && lp->scramble) rc = ofdm_descramble(ctx, sbits, bits, n * (lp->S / lp->SpF), stream_bits / (lp->S / lp->SpF), lp->reg0_host, nullptr);
         }
-        if (rc) break;
+        if (rc) return rc;
         sync_fill_kernel<<<(unsigned)cdiv64(n, 256), 256, 0, ctx->stream>>>(n, sp->snr_db_host[i], snr_d, sp->sto_mode, sp->sto_fixed, sp->cfo_fixed, sto_d, cfo_d);
         ctx->launches++;
         // Task 4 order: Noise -> add_STO -> add_CFO -> multipath (`Main_model_Task_4.m:95,103,110,263-264`), one pass
@@ -160,11 +142,8 @@ extern "C" int ofdm_sweep_sync(ofdm_ctx* ctx, const ofdm_link_params* lp, const 
         if (rc == OFDM_OK) rc = ofdm_channel_t4_p(ctx, tx, n, L, snr_d, psum, nullptr, sp->seed, g, sto_d, cfo_d, Nfft, h_dev, D, rx);
         if (rc == OFDM_OK)
             rc = ofdm_rx_t4_sync_stats(ctx, lp, rx, n, sp->time_desync, sp->freq_desync, sp->mp_desync, bits, counts_dev + 4 * i, tg_d, fo_d, ifo_d, fail_d,
-                                       sto_d, cfo_d, Ht_dev, rec_dev + i * 9 * spp + (g - i * spp), spp);
-        g += n;
-    }
-    cudaError_t e = cudaGetLastError();
-    if (rc == OFDM_OK && e != cudaSuccess) rc = ctx_fail(ctx, OFDM_ERR_CUDA, "ofdm_sweep_sync launch failed: %s", cudaGetErrorString(e));
-    cudaFreeAsync(pool, ctx->stream);
-    return rc;
+                                       sto_d, cfo_d, Ht_dev, rec_dev + i * 9 * spp + j0, spp);
+        return rc;
+    });
+    return scr.finish(rc, "ofdm_sweep_sync launch failed");
 }

@@ -119,12 +119,11 @@ def sweep(ctx, combs, mc_runs, payload, *, block=None, rank=0, world=1, reg_pilo
         nm[k, r0:r0 + n] = torch.from_numpy(nmse)
         er[k] += torch.from_numpy(errs)
         nb[k] += n * bits_run
-    if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
-        dev = ctx.device if dist.get_backend() == "nccl" else "cpu"
-        nm, er, nb = nm.to(dev), er.to(dev), nb.to(dev)
-        for t in (nm, er, nb):
-            dist.all_reduce(t, op=dist.ReduceOp.SUM)
-        nm, er, nb = nm.cpu(), er.cpu(), nb.cpu()
+    from .sweep import all_reduce_sum                            # sweep imports this module
+    if dist.is_available() and dist.is_initialized() and dist.get_backend() == "nccl":
+        nm, er, nb = nm.to(ctx.device), er.to(ctx.device), nb.to(ctx.device)
+    all_reduce_sum(nm, er, nb)
+    nm, er, nb = nm.cpu(), er.cpu(), nb.cpu()
     NMSE = nm.mean(dim=1).numpy().T                               # mean over the Monte-Carlo runs, :311-314
     BER = (er.double() / nb.double()[:, None]).numpy().T          # equal run sizes: mean of per-run BERs, :305-308
     return NMSE, BER
@@ -157,9 +156,8 @@ def reduce_part2(per_run, counts, runs):
     """Sum the per-run NMSE (n_points, 4, mc_runs) float64, the counts (n_points, 4, 3) and the runs (n_points, 2) int64 over
     all ranks (no-op without an initialised process group), then form ``sweep``'s results with its own arithmetic.
     Returns (NMSE[4, n_points], BER[4, n_points], per_run, counts, runs) as NumPy arrays, identical on every rank."""
-    if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
-        for t in (per_run, counts, runs):
-            dist.all_reduce(t, op=dist.ReduceOp.SUM)         # exact: every NMSE cell is non-zero on one rank only
+    from .sweep import all_reduce_sum                            # sweep imports this module
+    all_reduce_sum(per_run, counts, runs)                        # exact: every NMSE cell is non-zero on one rank only
     per, cnt, rn = per_run.cpu().numpy(), counts.cpu().numpy(), runs.cpu().numpy()
     nm = torch.from_numpy(np.ascontiguousarray(per.transpose(0, 2, 1)))      # the (point, run, estimator) layout of sweep
     er = torch.from_numpy(np.ascontiguousarray(cnt[:, :, 0]))

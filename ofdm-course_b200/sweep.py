@@ -51,13 +51,19 @@ def tiles(n_snr, streams_per_point, tile, rank=0, world=1):
     return out
 
 
+def all_reduce_sum(*tensors):
+    """Sum each tensor in place over all ranks (no-op without an initialised process group of more than one rank)."""
+    if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
+        for t in tensors:
+            dist.all_reduce(t, op=dist.ReduceOp.SUM)
+
+
 def reduce_counts(counts, device=None):
     """Sum an int64 counter tensor over all ranks (no-op without an initialised process group)."""
     t = counts if isinstance(counts, torch.Tensor) else torch.as_tensor(np.asarray(counts), dtype=torch.int64)
     if device is not None:
         t = t.to(device)
-    if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
-        dist.all_reduce(t, op=dist.ReduceOp.SUM)
+    all_reduce_sum(t)
     return t
 
 
@@ -113,9 +119,7 @@ def reduce_mse(per_stream, counts):
     """Sum the per-stream MSE array (n_snr, 4, streams_per_point) float64 and the counters (n_snr, 2) int64 over all ranks
     (no-op without an initialised process group) and take the mean over the streams of each point on the host.
     Returns (mean[n_snr, 4], per_stream, counts) as NumPy arrays, identical on every rank."""
-    if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
-        dist.all_reduce(per_stream, op=dist.ReduceOp.SUM)     # exact: every cell is non-zero on one rank only
-        dist.all_reduce(counts, op=dist.ReduceOp.SUM)
+    all_reduce_sum(per_stream, counts)                        # exact: every cell is non-zero on one rank only
     per = per_stream.cpu().numpy()
     return per.mean(axis=2), per, counts.cpu().numpy()
 
@@ -200,9 +204,7 @@ def reduce_sync(rec, counts, h_power=1.0, sym_len=1152, cfo_tol=0.02):
       h_err_mean over the non-NaN cells, h_err_nan (NaN cells), nmse = h_err_mean / h_power;
       mer_db: mean of the finite per-stream MER values in dB;
     plus ``rec`` and ``counts`` themselves."""
-    if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
-        dist.all_reduce(rec, op=dist.ReduceOp.SUM)
-        dist.all_reduce(counts, op=dist.ReduceOp.SUM)
+    all_reduce_sum(rec, counts)
     r = rec.cpu().numpy()
     c = counts.cpu().numpy()
     n = r.shape[2]
@@ -339,9 +341,7 @@ def reduce_papr(hist, papr, bin_db=0.01):
     ranks -- one all-reduce each, exact because the histogram is integer and every PAPR cell is written by one rank (no-op
     without an initialised process group).  Returns a dict of NumPy arrays, identical on every rank: ``hist``, ``edges``
     (b * bin_db), ``ccdf`` at the edges (:func:`papr_ccdf`), ``papr`` and its mean per point ``papr_mean``."""
-    if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
-        dist.all_reduce(hist, op=dist.ReduceOp.SUM)
-        dist.all_reduce(papr, op=dist.ReduceOp.SUM)
+    all_reduce_sum(hist, papr)
     h = hist.cpu().numpy()
     p = papr.cpu().numpy()
     return {"hist": h, "edges": np.arange(h.shape[-1]) * float(bin_db), "ccdf": papr_ccdf(h), "papr": p, "papr_mean": p.mean(axis=-1)}
