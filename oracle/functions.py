@@ -23,7 +23,7 @@ __all__ = [
     "interpolate", "equalize_signal", "OMP_estimate", "MP_estimate", "BER_func", "MER_func",
     "interp1_spline", "sensing_matrix_dft", "pilot_layout_percent", "pilot_layout_comb",
     "calculatePAPR", "calculate_window_PAPR", "calculateCCDF", "DEFAULT_REGISTER",
-    "Scrambler_fast", "DeScrambler_fast",
+    "Scrambler_fast", "DeScrambler_fast", "near_margin",
 ]
 
 #: initial scrambler register used by every script (`Task 4/Main_model_Task_4.m:43`)
@@ -151,6 +151,17 @@ def demapping(pad, IQ, Constellation):
     if pad != -1:
         bits = bits[: bits.size - pad]                          # :21-23
     return bits
+
+
+def near_margin(iq, Constellation):
+    """Decision margin of each symbol of ``demapping``: second-smallest minus smallest squared
+    distance to the constellation points, in float64 (0 on a decision boundary).  This is the
+    quantity the device demappers compare with ``near_eps`` (not a reference function)."""
+    dictionary, _ = constellation_func(Constellation)
+    IQ = np.asarray(iq).ravel().astype(np.complex128)
+    dist = (IQ.real[None, :] - dictionary.real[:, None]) ** 2 + (IQ.imag[None, :] - dictionary.imag[:, None]) ** 2
+    two = np.partition(dist, 1, axis=0)[:2]
+    return two[1] - two[0]
 
 
 # --------------------------------------------------------------------------- a6

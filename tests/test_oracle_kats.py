@@ -276,3 +276,24 @@ def test_fast_scrambler_forms_equal_the_loops(L):
         c, rc = O.DeScrambler(reg, a)
         d, rd = O.DeScrambler_fast(reg, a)
         assert np.array_equal(c, d) and np.array_equal(rc, rd) and np.array_equal(c, x)
+
+
+def test_near_margin_known_answers():
+    """near_margin = second-smallest minus smallest squared distance; for 16QAM that is 2 * (2a) * (distance of the nearer
+    axis to its decision boundary), a = 1/sqrt(10) -- the closed form the Nfft-4096 receiver counts with."""
+    a = 1 / np.sqrt(10)
+    u = 1e-3
+    iq = np.array([a + 1j * a, (2 * a - u) + 1j * a, 3.5 * a - 3j * a, u - 1j * a, 0.0 + 0j, -3 * a + 1j * (2 * a + u)])
+    want = np.array([4 * a * a, 4 * a * u, 4 * a * a, 4 * a * u, 0.0, 4 * a * u])
+    got = O.near_margin(iq, "16QAM")
+    assert got.dtype == np.float64 and np.allclose(got, want, rtol=1e-12, atol=1e-15)
+    assert np.allclose(O.near_margin([0.3, -2.0, 0.0], "BPSK"), [1.2, 8.0, 0.0], rtol=1e-14, atol=1e-15)
+    assert abs(O.near_margin([0.5j], "QPSK")[0]) < 1e-15
+    d, _ = O.constellation_func("8PSK")
+    assert np.allclose(O.near_margin(d, "8PSK"), (2 * np.sin(np.pi / 8)) ** 2, rtol=1e-12)
+    # the separable closed form on random symbols (both axes, inner and outer decision regions)
+    rng = np.random.default_rng(5)
+    z = (rng.standard_normal(2000) + 1j * rng.standard_normal(2000)) * 0.8
+    ax, ay = np.abs(z.real), np.abs(z.imag)
+    closed = 4 * a * np.minimum(np.minimum(ax, np.abs(ax - 2 * a)), np.minimum(ay, np.abs(ay - 2 * a)))
+    assert np.allclose(O.near_margin(z, "16QAM"), closed, rtol=1e-9, atol=1e-14)
