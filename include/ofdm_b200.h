@@ -472,6 +472,45 @@ OFDM_API int ofdm_draw_sto_cfo(ofdm_ctx*, int64_t B, uint64_t seed, int64_t firs
 OFDM_API int ofdm_payload_bernoulli(ofdm_ctx*, uint32_t* bits_dev, int64_t n_streams, int64_t stream_bits, double p_one,
                                     uint64_t seed, int64_t first_stream_id);
 
+/* ---- device groups: one call runs a sweep on several GPUs of the process ------------------------------------------------- */
+/* A group holds one context per entry of `devices`, in the given order: member i is rank i of world n_devices.  Ids are CUDA
+ * device ordinals (0-based) and may repeat -- two members on one GPU are two contexts there, valid and bit-identical.
+ * ofdm_group_create returns OFDM_ERR_INVALID for n_devices <= 0, a NULL list or a bad precision, and OFDM_ERR_NODEVICE for an id
+ * without an sm_100 device; on failure *out is NULL and nothing is left allocated.  The members are created on threads of their
+ * own, so the calling thread's current device is what it was before.
+ *
+ * ofdm_group_sweep_* run the ofdm_sweep_* call of the same name on every member at once, one host thread per member for the
+ * duration of the call.  The rank / world fields of the params are ignored (the group sets them); every other field means what
+ * it means for the single-context call, and the same checks apply.  Outputs are HOST arrays of the shape and layout of the
+ * single-context call's device arrays, and are overwritten (not added to):
+ *   - integer arrays (counters, the PAPR histogram, part-2 runs) are the sum over the members;
+ *   - per-stream / per-run cells (mse, rec, papr, nmse) are copied from the member whose ofdm_sweep_share range holds them, so
+ *     -0.0 and NaN payloads survive;
+ * the result is bit-identical to the single-context call with world = 1.  Each member zeroes its own device outputs, runs the
+ * sweep on its own stream, copies its results back and synchronises; its device buffers are kept for the next call
+ * (grow-only) and freed by ofdm_group_destroy.  Nothing is left running or enqueued when a call returns.  A member whose share
+ * is empty (more members than streams) launches nothing and contributes zeros.
+ * If a member fails, the call returns the status of the lowest-index failing member and ofdm_group_last_error reads
+ * "device <id> (member <i>): <that member's ofdm_last_error>"; the host outputs are then unspecified and the group stays
+ * usable.  One call at a time per group. */
+typedef struct ofdm_group ofdm_group;
+OFDM_API int ofdm_group_create(ofdm_group** out, const int* devices, int n_devices, int precision);
+OFDM_API void ofdm_group_destroy(ofdm_group* g);   /* NULL: no-op */
+OFDM_API const char* ofdm_group_last_error(const ofdm_group* g);
+OFDM_API int ofdm_group_size(const ofdm_group* g);
+/* counts_host: n_snr x 4 int64 */
+OFDM_API int ofdm_group_sweep_ber(ofdm_group*, const ofdm_link_params*, const ofdm_sweep_params*, int64_t* counts_host);
+/* mse_host: n_snr x 4 x streams_per_point doubles; counts_host: n_snr x 2 int64 */
+OFDM_API int ofdm_group_sweep_mse(ofdm_group*, const ofdm_link_params*, const ofdm_sweep_params*, int Ldict, double* mse_host,
+                                  int64_t* counts_host);
+/* rec_host: n_snr x 9 x streams_per_point doubles; counts_host: n_snr x 4 int64 */
+OFDM_API int ofdm_group_sweep_sync(ofdm_group*, const ofdm_link_params*, const ofdm_sync_params*, double* rec_host, int64_t* counts_host);
+/* papr_host: n_points x streams_per_point doubles; hist_host: n_points x n_bins int64 */
+OFDM_API int ofdm_group_sweep_papr(ofdm_group*, const ofdm_link_params*, const ofdm_papr_params*, double* papr_host, int64_t* hist_host);
+/* nmse_host: n_points x 4 x mc_runs doubles; counts_host: n_points x 4 x 3 int64; runs_host: n_points x 2 int64 */
+OFDM_API int ofdm_group_sweep_part2(ofdm_group*, const ofdm_link_params* base, const ofdm_part2_params*, double* nmse_host,
+                                    int64_t* counts_host, int64_t* runs_host);
+
 #ifdef __cplusplus
 }
 #endif

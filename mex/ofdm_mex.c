@@ -12,6 +12,8 @@
  * type, 0/1 double bits -> packed words, 1-based double indices -> int32, host <-> device copies.
  * No computation happens here and there is no CPU fallback: without an sm_100 GPU every op fails
  * with ofdm:ctx:nodevice.  The matlab/<Name>.m wrappers give each op the reference's signature.
+ * The five sweep ops run on the device set of ofdm_mex('devices', ids) (0-based CUDA ids, default [0]: one context on
+ * device 0); any other set runs them through one ofdm_group, every other op stays on device 0.
  */
 #include <math.h>
 #include <stdint.h>
@@ -29,6 +31,12 @@
 
 static ofdm_ctx* g_ctx = NULL;
 static int g_prec = OFDM_PREC_F32;
+/* the device set of the five sweep ops (ofdm_mex('devices', ids), 0-based CUDA ids): [0] runs them on g_ctx, any other set
+ * on g_group, built on first use and rebuilt after a precision switch */
+#define MAX_DEVICES 64
+static int g_devices[MAX_DEVICES] = {0};
+static int g_ndevices = 1;
+static ofdm_group* g_group = NULL;
 
 /* ---- scratch bookkeeping: everything allocated during one call is released on exit or error ---- */
 #define MAX_TMP 96
@@ -40,16 +48,20 @@ static void release_all(void) {
     for (i = 0; i < g_nhost; ++i) free(g_host[i]);
     g_ndev = g_nhost = 0;
 }
-static void at_exit(void) { release_all(); if (g_ctx) { ofdm_ctx_destroy(g_ctx); g_ctx = NULL; } }
-static void fail(const char* id, const char* msg) { release_all(); mexErrMsgIdAndTxt(id, "%s", msg); }
-static void chk(int rc, const char* op) {
-    if (rc != OFDM_OK) {
-        char buf[640];
-        strncpy(buf, op, 64); buf[64] = 0; strcat(buf, ": ");
-        strncat(buf, g_ctx ? ofdm_last_error(g_ctx) : "no context", 500);
-        fail("ofdm:call:failed", buf);
-    }
+static void at_exit(void) {
+    release_all();
+    if (g_ctx) { ofdm_ctx_destroy(g_ctx); g_ctx = NULL; }
+    ofdm_group_destroy(g_group); g_group = NULL;
 }
+static void fail(const char* id, const char* msg) { release_all(); mexErrMsgIdAndTxt(id, "%s", msg); }
+static void fail_call(const char* op, const char* text) {
+    char buf[640];
+    strncpy(buf, op, 64); buf[64] = 0; strcat(buf, ": ");
+    strncat(buf, text, 500);
+    fail("ofdm:call:failed", buf);
+}
+static void chk(int rc, const char* op) { if (rc != OFDM_OK) fail_call(op, g_ctx ? ofdm_last_error(g_ctx) : "no context"); }
+static void chk_group(int rc, const char* op) { if (rc != OFDM_OK) fail_call(op, ofdm_group_last_error(g_group)); }
 static void* hostbuf(size_t bytes) {
     void* p = calloc(bytes ? bytes : 1, 1);
     if (!p || g_nhost >= MAX_TMP) fail("ofdm:mem:host", "host allocation failed");
@@ -70,6 +82,16 @@ static void ensure_ctx(void) {
         if (rc != OFDM_OK) mexErrMsgIdAndTxt("ofdm:ctx:create", "ofdm_ctx_create failed (%d)", rc);
         mexAtExit(at_exit);
     }
+}
+/* the group of the sweep ops, or NULL when the device set is the default [0] (the single-context path) */
+static ofdm_group* sweep_group(void) {
+    int rc;
+    if (g_ndevices == 1 && g_devices[0] == 0) return NULL;
+    if (g_group) return g_group;
+    rc = ofdm_group_create(&g_group, g_devices, g_ndevices, g_prec);
+    if (rc == OFDM_ERR_NODEVICE) fail("ofdm:devices:nodevice", "a device of the set is not an sm_100 GPU of this host");
+    if (rc != OFDM_OK) mexErrMsgIdAndTxt("ofdm:devices:create", "ofdm_group_create failed (%d)", rc);
+    return g_group;
 }
 static size_t esz(void) { return g_prec == OFDM_PREC_F64 ? 2 * sizeof(double) : 2 * sizeof(float); }
 static size_t rsz(void) { return g_prec == OFDM_PREC_F64 ? sizeof(double) : sizeof(float); }
@@ -237,6 +259,34 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
     }
     ensure_ctx();
 
+    if (!strcmp(op, "devices")) {   /* ids = ofdm_mex('devices' [, ids]): the 0-based CUDA devices of the five sweep ops */
+        if (nrhs > 1) {
+            size_t n = mxGetNumberOfElements(A(0)), i;
+            int ids[MAX_DEVICES];
+            if (!mxIsDouble(A(0)) || mxIsComplex(A(0))) mexErrMsgIdAndTxt("ofdm:devices:type", "device ids must be real doubles");
+            if (n == 0) mexErrMsgIdAndTxt("ofdm:devices:empty", "need at least one device id");
+            if (n > MAX_DEVICES) mexErrMsgIdAndTxt("ofdm:devices:count", "at most %d device ids", MAX_DEVICES);
+            for (i = 0; i < n; ++i) {
+                double v = real_data(A(0))[i];
+                if (!(v >= 0 && v <= 1e6 && v == floor(v))) mexErrMsgIdAndTxt("ofdm:devices:id", "device ids are 0-based integers >= 0");
+                ids[i] = (int)v;
+            }
+            ofdm_group_destroy(g_group); g_group = NULL;
+            memcpy(g_devices, ids, n * sizeof(int));
+            g_ndevices = (int)n;
+            if (!(g_ndevices == 1 && g_devices[0] == 0) && ofdm_group_create(&g_group, g_devices, g_ndevices, g_prec) != OFDM_OK) {
+                g_devices[0] = 0; g_ndevices = 1;                   /* back to the default set */
+                mexErrMsgIdAndTxt("ofdm:devices:nodevice", "a device of the set is not an sm_100 GPU of this host; the set is [0] again");
+            }
+        }
+        {
+            mxArray* dm = mxCreateDoubleMatrix(1, (size_t)g_ndevices, mxREAL);
+            int i;
+            for (i = 0; i < g_ndevices; ++i) real_data(dm)[i] = g_devices[i];
+            OUT(0, dm);
+        }
+        return;
+    }
     if (!strcmp(op, "Scrambler") || !strcmp(op, "DeScrambler")) {            /* [seq, Register] = f(Register, sequence) */
         NEED(2);
         size_t L = mxGetNumberOfElements(A(1)), i;
@@ -634,11 +684,14 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
             for (k2 = 0; k2 < K; ++k2) { taps[2 * k2] = tp[k2]; taps[2 * k2 + 1] = tp[K + k2]; }
             sp.taps_host = taps; sp.n_taps = K;
         }
-        int64_t* cd = (int64_t*)devbuf(n * 32);
         int64_t* ch = (int64_t*)hostbuf(n * 32);
-        chk(ofdm_memset(g_ctx, cd, 0, n * 32), "memset");
-        chk(ofdm_sweep_ber(g_ctx, &lp, &sp, cd), op);
-        chk(ofdm_d2h(g_ctx, ch, cd, n * 32), "d2h");
+        if (sweep_group()) chk_group(ofdm_group_sweep_ber(g_group, &lp, &sp, ch), op);
+        else {
+            int64_t* cd = (int64_t*)devbuf(n * 32);
+            chk(ofdm_memset(g_ctx, cd, 0, n * 32), "memset");
+            chk(ofdm_sweep_ber(g_ctx, &lp, &sp, cd), op);
+            chk(ofdm_d2h(g_ctx, ch, cd, n * 32), "d2h");
+        }
         mxArray* cm = mxCreateDoubleMatrix(n, 4, mxREAL);
         for (i = 0; i < n; ++i) { int j; for (j = 0; j < 4; ++j) real_data(cm)[(size_t)j * n + i] = (double)ch[4 * i + j]; }
         OUT(0, cm);
@@ -670,15 +723,18 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
         int comb = lp.pilot_carriers_host[1] - lp.pilot_carriers_host[0];
         int Ldict = nrhs > N_LINK + 6 ? (int)mxGetScalar(A(N_LINK + 5)) : (comb > 0 ? (lp.N_carrier + comb - 1) / comb : 0);
         size_t spp = (size_t)(sp.streams_per_point > 0 ? sp.streams_per_point : 0), cells = n * 4 * spp;
-        double* md = (double*)devbuf(cells * 8 + 8);
-        int64_t* cd = (int64_t*)devbuf(n * 16);
         double* mh = (double*)hostbuf(cells * 8 + 8);
         int64_t* ch = (int64_t*)hostbuf(n * 16);
-        chk(ofdm_memset(g_ctx, md, 0, cells * 8), "memset");
-        chk(ofdm_memset(g_ctx, cd, 0, n * 16), "memset");
-        chk(ofdm_sweep_mse(g_ctx, &lp, &sp, Ldict, md, cd), op);
-        chk(ofdm_d2h(g_ctx, mh, md, cells * 8), "d2h");
-        chk(ofdm_d2h(g_ctx, ch, cd, n * 16), "d2h");
+        if (sweep_group()) chk_group(ofdm_group_sweep_mse(g_group, &lp, &sp, Ldict, mh, ch), op);
+        else {
+            double* md = (double*)devbuf(cells * 8 + 8);
+            int64_t* cd = (int64_t*)devbuf(n * 16);
+            chk(ofdm_memset(g_ctx, md, 0, cells * 8), "memset");
+            chk(ofdm_memset(g_ctx, cd, 0, n * 16), "memset");
+            chk(ofdm_sweep_mse(g_ctx, &lp, &sp, Ldict, md, cd), op);
+            chk(ofdm_d2h(g_ctx, mh, md, cells * 8), "d2h");
+            chk(ofdm_d2h(g_ctx, ch, cd, n * 16), "d2h");
+        }
         mxArray* mm = mxCreateDoubleMatrix(n, 4, mxREAL);           /* mean over the streams of each point */
         for (i = 0; i < n; ++i)
             for (e = 0; e < 4; ++e) {
@@ -728,15 +784,18 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
         const double* fl = real_data(A(N_LINK + 6));
         sp.time_desync = fl[0] != 0; sp.freq_desync = fl[1] != 0; sp.mp_desync = fl[2] != 0;
         size_t spp = (size_t)(sp.streams_per_point > 0 ? sp.streams_per_point : 0), cells = n * 9 * spp;
-        double* rd = (double*)devbuf(cells * 8 + 8);
-        int64_t* cd = (int64_t*)devbuf(n * 32);
         int64_t* ch = (int64_t*)hostbuf(n * 32);
-        chk(ofdm_memset(g_ctx, rd, 0, cells * 8), "memset");
-        chk(ofdm_memset(g_ctx, cd, 0, n * 32), "memset");
-        chk(ofdm_sweep_sync(g_ctx, &lp, &sp, rd, cd), op);
         mxArray* rm = mxCreateDoubleMatrix(spp, 9 * n, mxREAL);     /* reshape(rec, spp, 9, n_snr) in MATLAB */
-        chk(ofdm_d2h(g_ctx, real_data(rm), rd, cells * 8), "d2h");
-        chk(ofdm_d2h(g_ctx, ch, cd, n * 32), "d2h");
+        if (sweep_group()) chk_group(ofdm_group_sweep_sync(g_group, &lp, &sp, cells ? real_data(rm) : (double*)hostbuf(8), ch), op);
+        else {
+            double* rd = (double*)devbuf(cells * 8 + 8);
+            int64_t* cd = (int64_t*)devbuf(n * 32);
+            chk(ofdm_memset(g_ctx, rd, 0, cells * 8), "memset");
+            chk(ofdm_memset(g_ctx, cd, 0, n * 32), "memset");
+            chk(ofdm_sweep_sync(g_ctx, &lp, &sp, rd, cd), op);
+            chk(ofdm_d2h(g_ctx, real_data(rm), rd, cells * 8), "d2h");
+            chk(ofdm_d2h(g_ctx, ch, cd, n * 32), "d2h");
+        }
         OUT(0, rm);
         mxArray* cm = mxCreateDoubleMatrix(n, 4, mxREAL);
         for (i = 0; i < n; ++i) { int j; for (j = 0; j < 4; ++j) real_data(cm)[(size_t)j * n + i] = (double)ch[4 * i + j]; }
@@ -774,18 +833,21 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
         pp.bin_db = mxGetScalar(A(N_LINK + 4));
         pp.n_bins = (int32_t)mxGetScalar(A(N_LINK + 5));
         size_t spp = (size_t)(pp.streams_per_point > 0 ? pp.streams_per_point : 0), nb = (size_t)(pp.n_bins > 0 ? pp.n_bins : 0);
-        double* pd = (double*)devbuf(n * spp * 8 + 8);
-        int64_t* hd = (int64_t*)devbuf(n * nb * 8 + 8);
         int64_t* hh = (int64_t*)hostbuf(n * nb * 8 + 8);
-        chk(ofdm_memset(g_ctx, pd, 0, n * spp * 8), "memset");
-        chk(ofdm_memset(g_ctx, hd, 0, n * nb * 8), "memset");
-        chk(ofdm_sweep_papr(g_ctx, &lp, &pp, pd, hd), op);
+        mxArray* pm = mxCreateDoubleMatrix(spp, n, mxREAL);
+        if (sweep_group()) chk_group(ofdm_group_sweep_papr(g_group, &lp, &pp, spp ? real_data(pm) : (double*)hostbuf(8), hh), op);
+        else {
+            double* pd = (double*)devbuf(n * spp * 8 + 8);
+            int64_t* hd = (int64_t*)devbuf(n * nb * 8 + 8);
+            chk(ofdm_memset(g_ctx, pd, 0, n * spp * 8), "memset");
+            chk(ofdm_memset(g_ctx, hd, 0, n * nb * 8), "memset");
+            chk(ofdm_sweep_papr(g_ctx, &lp, &pp, pd, hd), op);
+            chk(ofdm_d2h(g_ctx, hh, hd, n * nb * 8), "d2h");
+            chk(ofdm_d2h(g_ctx, real_data(pm), pd, n * spp * 8), "d2h");
+        }
         mxArray* hm = mxCreateDoubleMatrix(nb, n, mxREAL);
-        chk(ofdm_d2h(g_ctx, hh, hd, n * nb * 8), "d2h");
         for (i = 0; i < n * nb; ++i) real_data(hm)[i] = (double)hh[i];
         OUT(0, hm);
-        mxArray* pm = mxCreateDoubleMatrix(spp, n, mxREAL);
-        chk(ofdm_d2h(g_ctx, real_data(pm), pd, n * spp * 8), "d2h");
         OUT(1, pm);
     } else if (!strcmp(op, "sweep_part2")) {   /* [NMSE (4 x n_points), BER (4 x n_points), per_run (mc_runs x 4*n_points), counts (12 x n_points),
                                                    runs (2 x n_points)] = sweep_part2(Nfft, T_Guard, N_carrier, N_symb, SpF, Constellation,
@@ -793,7 +855,7 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
                                                    offsets = [] -> pilots is a vector of combs (pilots 1:comb:N_carrier, Ldict ceil(Nfft/comb));
                                                    else pilots are the concatenated 1-based pilot vectors of the points, offsets (n_points + 1,
                                                    from 0) delimit them and Ldict defaults to Nfft.  Ldict = [] takes the defaults.  pattern: the
-                                                   two pilot values (pilot q carries pattern(mod(q-1,2)+1)).  bits: 0/1 payload.  Single GPU. */
+                                                   two pilot values (pilot q carries pattern(mod(q-1,2)+1)).  bits: 0/1 payload. */
         NEED(18);
         ofdm_link_params lp;
         ofdm_part2_params pp;
@@ -855,19 +917,22 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
         pp.seed = (uint64_t)mxGetScalar(A(15));
         pp.near_eps = mxGetScalar(A(16)); pp.tie_eps = mxGetScalar(A(17));
         size_t R = (size_t)(pp.mc_runs > 0 ? pp.mc_runs : 0), cells = P * 4 * R;
-        double* md = (double*)devbuf(cells * 8 + 8);
-        int64_t* cd = (int64_t*)devbuf(P * 96);
-        int64_t* rd = (int64_t*)devbuf(P * 16);
         double* mh = (double*)hostbuf(cells * 8 + 8);
         int64_t* ch = (int64_t*)hostbuf(P * 96);
         int64_t* rh = (int64_t*)hostbuf(P * 16);
-        chk(ofdm_memset(g_ctx, md, 0, cells * 8), "memset");
-        chk(ofdm_memset(g_ctx, cd, 0, P * 96), "memset");
-        chk(ofdm_memset(g_ctx, rd, 0, P * 16), "memset");
-        chk(ofdm_sweep_part2(g_ctx, &lp, &pp, md, cd, rd), op);
-        chk(ofdm_d2h(g_ctx, mh, md, cells * 8), "d2h");
-        chk(ofdm_d2h(g_ctx, ch, cd, P * 96), "d2h");
-        chk(ofdm_d2h(g_ctx, rh, rd, P * 16), "d2h");
+        if (sweep_group()) chk_group(ofdm_group_sweep_part2(g_group, &lp, &pp, mh, ch, rh), op);
+        else {
+            double* md = (double*)devbuf(cells * 8 + 8);
+            int64_t* cd = (int64_t*)devbuf(P * 96);
+            int64_t* rd = (int64_t*)devbuf(P * 16);
+            chk(ofdm_memset(g_ctx, md, 0, cells * 8), "memset");
+            chk(ofdm_memset(g_ctx, cd, 0, P * 96), "memset");
+            chk(ofdm_memset(g_ctx, rd, 0, P * 16), "memset");
+            chk(ofdm_sweep_part2(g_ctx, &lp, &pp, md, cd, rd), op);
+            chk(ofdm_d2h(g_ctx, mh, md, cells * 8), "d2h");
+            chk(ofdm_d2h(g_ctx, ch, cd, P * 96), "d2h");
+            chk(ofdm_d2h(g_ctx, rh, rd, P * 16), "d2h");
+        }
         mxArray* nm = mxCreateDoubleMatrix(4, P, mxREAL);              /* `Task5_part2.m:305-314`: estimators x points */
         mxArray* bm = mxCreateDoubleMatrix(4, P, mxREAL);
         for (i = 0; i < P; ++i)

@@ -9,4 +9,5 @@ from . import _cabi  # noqa: F401
 from .link import *  # noqa: F401,F403
 from .link import Context, OfdmError, default_context, pack_bits, unpack_bits, CONSTELLATIONS, DEFAULT_REGISTER  # noqa: F401
 from . import sweep  # noqa: F401,E402
+from .sweep import Group  # noqa: F401,E402
 from . import layouts  # noqa: F401,E402

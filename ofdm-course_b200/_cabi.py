@@ -128,6 +128,15 @@ SIGNATURES = {
     "ofdm_draw_sto_cfo": (i32, [vp, i64, u64, i64, i32, i32, vp, vp]),
     "ofdm_payload_bernoulli": (i32, [vp, vp, i64, i64, dbl, u64, i64]),
     "ofdm_rx_chain_t4_ex": (i32, [vp, C.POINTER(LinkParams), vp, i64, i32, i32, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, dbl, vp]),
+    "ofdm_group_create": (i32, [C.POINTER(vp), pi32, i32, i32]),
+    "ofdm_group_destroy": (None, [vp]),
+    "ofdm_group_last_error": (C.c_char_p, [vp]),
+    "ofdm_group_size": (i32, [vp]),
+    "ofdm_group_sweep_ber": (i32, [vp, C.POINTER(LinkParams), C.POINTER(SweepParams), vp]),
+    "ofdm_group_sweep_mse": (i32, [vp, C.POINTER(LinkParams), C.POINTER(SweepParams), i32, vp, vp]),
+    "ofdm_group_sweep_sync": (i32, [vp, C.POINTER(LinkParams), C.POINTER(SyncParams), vp, vp]),
+    "ofdm_group_sweep_papr": (i32, [vp, C.POINTER(LinkParams), C.POINTER(PaprParams), vp, vp]),
+    "ofdm_group_sweep_part2": (i32, [vp, C.POINTER(LinkParams), C.POINTER(Part2Params), vp, vp, vp]),
 }
 
 _lib = None

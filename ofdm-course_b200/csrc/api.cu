@@ -2,6 +2,8 @@
 #include <cmath>
 #include <cstdarg>
 #include <algorithm>
+#include <mutex>
+#include <utility>
 
 #include "common.cuh"
 
@@ -158,6 +160,21 @@ extern "C" int ofdm_host_alloc(void** host, size_t bytes) {
     return cudaMallocHost(host, bytes ? bytes : 1) == cudaSuccess ? OFDM_OK : OFDM_ERR_CUDA;
 }
 extern "C" int ofdm_host_free(void* host) { return cudaFreeHost(host) == cudaSuccess ? OFDM_OK : OFDM_ERR_CUDA; }
+
+cudaError_t func_smem_optin(const void* func, int bytes) {
+    static std::mutex mu;
+    static std::map<std::pair<int, const void*>, int> limit;   // (device, kernel) -> limit set so far
+    int dev = 0;
+    cudaError_t e = cudaGetDevice(&dev);
+    if (e != cudaSuccess) return e;
+    std::lock_guard<std::mutex> lock(mu);
+    const auto key = std::make_pair(dev, func);
+    const auto it = limit.find(key);
+    if (it != limit.end() && it->second >= bytes) return cudaSuccess;
+    e = cudaFuncSetAttribute(func, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+    if (e == cudaSuccess) limit[key] = bytes;
+    return e;
+}
 
 // ---------------------------------------------------------------- caches
 // Table uploads come from pageable host memory.  cudaMemcpy may return once the data sits in the driver's staging buffer,

@@ -343,7 +343,7 @@ extern "C" int ofdm_tx_chain_p(ofdm_ctx* ctx, const ofdm_link_params* lp, const 
         const int fw = (d.frame_bits + 31) / 32;
         const size_t smem = sizeof(float2) * 2 * TXF_XBUF + 2 * sizeof(uint32_t) * (size_t)(fw + TXF_PAD(fw));   // two bit arrays + their zero pads
         if (ok && smem <= 110 * 1024) {
-            CUDA_TRY(ctx, cudaFuncSetAttribute(tx4096_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            CUDA_TRY(ctx, func_smem_optin((const void*)tx4096_kernel, (int)smem));
             const int64_t grid = std::min<int64_t>(B, 2 * (int64_t)ctx->sm_count);
             unsigned long long* sched = nullptr;                  // per launch: launches on different streams may overlap
             if (B > grid && !getenv("OFDM_B200_STATIC_STREAMS")) {
@@ -373,7 +373,7 @@ extern "C" int ofdm_tx_chain_p(ofdm_ctx* ctx, const ofdm_link_params* lp, const 
         if (rc) return rc;
         size_t smem = 2 * sizeof(cx<T>) * d.Nfft + 2 * sizeof(uint32_t) * ((d.frame_bits + 31) / 32);
         auto k = tx_chain_kernel<T>;
-        if (smem > 48 * 1024) CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        if (smem > 48 * 1024) CUDA_TRY(ctx, func_smem_optin((const void*)k, (int)smem));
         k<<<(unsigned)B, CH_THREADS, smem, ctx->stream>>>(d, bits, B * (int64_t)d.frame_bits * d.frames, (cx<T>*)time);
     });
     LAUNCH_CHECK(ctx);
@@ -493,7 +493,7 @@ extern "C" int ofdm_rx_chain_t5(ofdm_ctx* ctx, const ofdm_link_params* lp, const
         const int fw = (d.frame_bits + 31) / 32;
         size_t smem = sizeof(cx<T>) * (2 * (size_t)d.Nfft + 2 * (size_t)pl->n_knots + d.Nc) + sizeof(uint32_t) * fw + (size_t)d.SpF * d.Nd + 16;
         auto k = rx_chain_kernel<T>;
-        if (smem > 48 * 1024) CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        if (smem > 48 * 1024) CUDA_TRY(ctx, func_smem_optin((const void*)k, (int)smem));
         k<<<(unsigned)B, CH_THREADS, smem, ctx->stream>>>(d, plan_dev<T>(pl), (const cx<T>*)rx, tx_bits, B * stream_bits, out_bits, (cx<T>*)H,
                                                            (unsigned long long*)counts, err_stream, (T)near_eps);
     });

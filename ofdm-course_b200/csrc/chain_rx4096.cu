@@ -499,7 +499,7 @@ int ofdm_rx_chain_fast4096(ofdm_ctx* ctx, const ofdm_link_params* lp, const void
     } else kern = near ? rx4096_kernel<false, true, 0, false> : rx4096_kernel<false, false, 0, false>;
     const bool use_slim = slim && q16;
     if (use_slim) smem = smem_slim;
-    CUDA_TRY(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    CUDA_TRY(ctx, func_smem_optin((const void*)kern, (int)smem));
     int grid = (int)std::min<int64_t>(B, (int64_t)ctx->sm_count * (use_slim ? 3 : 2));
     if (err_stream) CUDA_TRY(ctx, cudaMemsetAsync(err_stream, 0, sizeof(int32_t) * B, ctx->stream));
     if (out_bits && !p.aligned) CUDA_TRY(ctx, cudaMemsetAsync(out_bits, 0, sizeof(uint32_t) * OFDM_BIT_WORDS(B * (int64_t)frame_bits * p.frames), ctx->stream));

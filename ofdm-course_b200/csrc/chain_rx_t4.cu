@@ -1184,7 +1184,7 @@ int ofdm_tx1024_fast(ofdm_ctx* ctx, const ofdm_link_params* lp, const uint32_t* 
     p.pilots = (const float2*)ofdm_upload_pilots(ctx, lp->pilot_vals_host, (size_t)lp->Np * lp->S);
     p.tw_t = (const float2*)t4_twiddle_blob(ctx);
     REQUIRE(ctx, p.slot && p.pilots && p.tw_t, "device upload failed");
-    CUDA_TRY(ctx, cudaFuncSetAttribute(tx1024_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    CUDA_TRY(ctx, func_smem_optin((const void*)tx1024_kernel, (int)smem));
     const int64_t stream_bits = (int64_t)p.frame_bits * p.frames;
     double* part = nullptr;
     if (power) CUDA_TRY(ctx, cudaMallocAsync((void**)&part, sizeof(double) * (size_t)B * p.S, ctx->stream));
@@ -1254,9 +1254,9 @@ static int t4_split_run(ofdm_ctx* ctx, const ofdm_link_params* lp, const T4Param
     const int groups = (p.S + T4_THREADS / 32 - 1) / (T4_THREADS / 32);
     const size_t sym_smem = T4_TILES + sizeof(float2) * 1024, post_smem = t4_post_smem(p, pl);
     auto symk = p.Nc <= 416 ? t4_sym_kernel<13> : t4_sym_kernel<32>;
-    CUDA_TRY(ctx, cudaFuncSetAttribute(t4_ifo_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T4_TILES));
-    CUDA_TRY(ctx, cudaFuncSetAttribute(symk, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sym_smem));
-    CUDA_TRY(ctx, cudaFuncSetAttribute(post, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)post_smem));
+    CUDA_TRY(ctx, func_smem_optin((const void*)t4_ifo_kernel, (int)T4_TILES));
+    CUDA_TRY(ctx, func_smem_optin((const void*)symk, (int)sym_smem));
+    CUDA_TRY(ctx, func_smem_optin((const void*)post, (int)post_smem));
     float2* bins = nullptr;
     CUDA_TRY(ctx, cudaMallocAsync((void**)&bins, sizeof(float2) * (size_t)CH * p.S * ((size_t)p.Nd + p.Np), ctx->stream));
     float2* Yd_all = bins;
@@ -1361,7 +1361,7 @@ extern "C" int ofdm_rx_chain_t4_ex(ofdm_ctx* ctx, const ofdm_link_params* lp, co
                                       (float)near_eps, nullptr);
                     fast_done = true;
                 } else if (fx.tw_t) {
-                    cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fsmem);
+                    func_smem_optin((const void*)kern, (int)fsmem);
                     kern<<<grid, T4_THREADS, fsmem, ctx->stream>>>(p, fx, plan_dev<float>(pl), make_devconst<float>(lp->constellation), (const float2*)rx, B, L, tg_dev, fo_dev,
                                                                    (float2*)scr, tx_bits, B * stream_bits, out_bits, (unsigned long long*)counts, ifo_dev, tau_dev,
                                                                    phase_dev, (float2*)H_dev, (float)near_eps);
@@ -1374,7 +1374,7 @@ extern "C" int ofdm_rx_chain_t4_ex(ofdm_ctx* ctx, const ofdm_link_params* lp, co
         }
         if (rc == OFDM_OK && !fast_done && smem > 200 * 1024) rc = ctx_fail(ctx, OFDM_ERR_UNSUPPORTED, "stream shape needs %zu bytes of shared memory", smem);
         if (rc == OFDM_OK && !fast_done) {
-            cudaFuncSetAttribute(rx_t4_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+            func_smem_optin((const void*)rx_t4_kernel, (int)smem);
             rx_t4_kernel<<<grid, T4_THREADS, smem, ctx->stream>>>(p, plan_dev<float>(pl), make_devconst<float>(lp->constellation), (const float2*)rx, B, L, tg_dev, fo_dev,
                                                                    (float2*)scr, tx_bits, B * stream_bits, out_bits, (unsigned long long*)counts, ifo_dev, tau_dev,
                                                                    phase_dev, (float2*)H_dev, (float)near_eps);

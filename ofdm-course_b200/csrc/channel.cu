@@ -454,7 +454,7 @@ static int channel_fused_launch(ofdm_ctx* ctx, const void* tx, int64_t B, int64_
         ctx->launches++;
         const size_t smem = sizeof(cx<T>) * (size_t)(CH_TILE + 2 * D - 1) + sizeof(int) * (size_t)D;
         auto k = imp ? channel_t5_kernel<T, true> : channel_t5_kernel<T, false>;
-        if (smem > 48 * 1024) CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        if (smem > 48 * 1024) CUDA_TRY(ctx, func_smem_optin((const void*)k, (int)smem));
         k<<<dim3((unsigned)B, (unsigned)cdiv64(L, (int64_t)CH_TILE * CH_CHUNK)), 256, smem, ctx->stream>>>((const cx<T>*)tx, L, (const T*)(scr + o_sig), (const T*)normals, seed,
                                                                                          first_stream_id, (const cx<T>*)(scr + o_hv), (const int*)(scr + o_hd),
                                                                                          (const int*)(scr + o_nnz), D, (cx<T>*)rx, nsto, cfo, imp ? 1.0 / Nfft : 0.0);

@@ -178,7 +178,7 @@ extern "C" int ofdm_interpolate(ofdm_ctx* ctx, const void* Hp, int64_t B, const 
     DISPATCH_T(ctx, {
         size_t smem = 2 * sizeof(cx<T>) * pl->n_knots;
         auto k = interpolate_kernel<T>;
-        if (smem > 48 * 1024) CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        if (smem > 48 * 1024) CUDA_TRY(ctx, func_smem_optin((const void*)k, (int)smem));
         k<<<(unsigned)B, CE_THREADS, smem, ctx->stream>>>((const cx<T>*)Hp, plan_dev<T>(pl), (cx<T>*)H);
     });
     LAUNCH_CHECK(ctx);
@@ -196,7 +196,7 @@ extern "C" int ofdm_ls_ce(ofdm_ctx* ctx, const void* grid, int64_t B, int S, int
     DISPATCH_T(ctx, {
         size_t smem = 2 * sizeof(cx<T>) * pl->n_knots;
         auto k = ls_ce_kernel<T>;
-        if (smem > 48 * 1024) CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        if (smem > 48 * 1024) CUDA_TRY(ctx, func_smem_optin((const void*)k, (int)smem));
         k<<<(unsigned)B, CE_THREADS, smem, ctx->stream>>>((const cx<T>*)grid, (int64_t)S * Nfft, l0, (const cx<T>*)xp, plan_dev<T>(pl), (cx<T>*)H);
     });
     LAUNCH_CHECK(ctx);
@@ -238,7 +238,7 @@ extern "C" int ofdm_estimate_channel(ofdm_ctx* ctx, const void* grid, int64_t B,
     DISPATCH_T(ctx, {
         size_t smem = 2 * sizeof(cx<T>) * pl->n_knots;
         auto k = estimate_channel_kernel<T>;
-        if (smem > 48 * 1024) CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        if (smem > 48 * 1024) CUDA_TRY(ctx, func_smem_optin((const void*)k, (int)smem));
         k<<<(unsigned)B, CE_THREADS, smem, ctx->stream>>>((const cx<T>*)grid, S, Nfft, l0, (const cx<T>*)xp, plan_dev<T>(pl), (cx<T>*)H, (cx<T>*)Hp);
     });
     LAUNCH_CHECK(ctx);
@@ -258,7 +258,7 @@ extern "C" int ofdm_mmse_ce(ofdm_ctx* ctx, const void* grid, int64_t B, int S, i
         size_t smem = 5 * sizeof(double2) * Np + 2 * sizeof(cx<T>) * pl->n_knots;
         REQUIRE(ctx, smem <= 220 * 1024, "too many pilots for the in-SMEM Levinson solver");
         auto k = mmse_kernel<T>;
-        if (smem > 48 * 1024) CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        if (smem > 48 * 1024) CUDA_TRY(ctx, func_smem_optin((const void*)k, (int)smem));
         k<<<(unsigned)B, MM_THREADS, smem, ctx->stream>>>((const cx<T>*)grid, (int64_t)S * Nfft, l0, (const cx<T>*)xp, Np, (double)(loc[1] - loc[0]), Nc,
                                                            (const cx<T>*)h, h_len, snr_db, plan_dev<T>(pl), (cx<T>*)H);
     });
@@ -280,7 +280,7 @@ int ofdm_mmse_ce_meas(ofdm_ctx* ctx, const void* y, int64_t B, const int32_t* lo
         size_t smem = 5 * sizeof(double2) * Np + 2 * sizeof(cx<T>) * pl->n_knots;
         REQUIRE(ctx, smem <= 220 * 1024, "too many pilots for the in-SMEM Levinson solver");
         auto k = mmse_kernel<T, true>;
-        if (smem > 48 * 1024) CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        if (smem > 48 * 1024) CUDA_TRY(ctx, func_smem_optin((const void*)k, (int)smem));
         k<<<(unsigned)B, MM_THREADS, smem, ctx->stream>>>((const cx<T>*)y, (int64_t)Np, l0, nullptr, Np, (double)(loc[1] - loc[0]), Nc,
                                                            (const cx<T>*)h, h_len, snr_db, plan_dev<T>(pl), (cx<T>*)H);
     });

@@ -245,6 +245,11 @@ const void* ctx_twiddles_prec(ofdm_ctx* ctx, int N, int precision);      // same
 const InterpPlan* ctx_plan(ofdm_ctx* ctx, const int32_t* knots1, int n, int ext_to /*0=no ext*/,
                            const int32_t* queries1 /*NULL => 1..nq*/, int nq, int method);
 uint64_t fnv1a(const void* p, size_t n, uint64_t h = 1469598103934665603ull);
+// Opt-in to `bytes` of dynamic shared memory for kernel `func` on the current device.  The limit belongs to the device's copy
+// of the kernel, not to a context, so contexts driven from several host threads (ofdm_group) share it: a plain
+// cudaFuncSetAttribute by one thread could LOWER it between another thread's opt-in and launch.  This one only ever raises it,
+// under a process-wide lock.
+cudaError_t func_smem_optin(const void* func, int bytes);
 
 #define CUDA_TRY(ctx, expr)                                                                   \
     do {                                                                                      \

@@ -190,11 +190,11 @@ extern "C" int ofdm_mmse_ce_shared(ofdm_ctx* ctx, const void* grid, int64_t B, i
     mmse_stats_kernel<float><<<1, 256, 0, st>>>((const float2*)h, h_len, (double)(loc[1] - loc[0]), Nc, snr_db, stats);
     const size_t wsm = 4 * sizeof(double2) * (size_t)Np;
     int rc = OFDM_OK;
-    if (wsm > 48 * 1024) cudaFuncSetAttribute(mmse_weight_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wsm);
+    if (wsm > 48 * 1024) func_smem_optin((const void*)mmse_weight_kernel, (int)wsm);
     mmse_weight_kernel<<<Np, MS_THREADS, wsm, st>>>(stats, Np, Npad, K2, Bt);
     mmse_ls_split_kernel<<<(unsigned)Bpad, 128, 0, st>>>((const float2*)grid, (int64_t)S * Nfft, B, l0, Np, Npad, K2, (const float2*)xp, At);
     if (rc == OFDM_OK) {
-        cudaFuncSetAttribute(tc_gemm_store_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM_BYTES);
+        func_smem_optin((const void*)tc_gemm_store_kernel, TC_SMEM_BYTES);
         for (int s = 0; s < n_slices && rc == OFDM_OK; ++s) {
             const int k0 = s * Ks, kn = std::min(Ks, Kt - k0);
             CUtensorMap mapA, mapB;
@@ -210,7 +210,7 @@ extern "C" int ofdm_mmse_ce_shared(ofdm_ctx* ctx, const void* grid, int64_t B, i
     }
     if (rc == OFDM_OK) {
         const size_t ssm = 2 * sizeof(float2) * (size_t)pl->n_knots;
-        if (ssm > 48 * 1024) cudaFuncSetAttribute(mmse_spline_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ssm);
+        if (ssm > 48 * 1024) func_smem_optin((const void*)mmse_spline_kernel, (int)ssm);
         mmse_spline_kernel<<<(unsigned)B, 256, ssm, st>>>(D, 2 * Npad, Npad, n_slices, slice_stride, plan_dev<float>(pl), (float2*)H);
         ctx->launches += 4;
         cudaError_t e = cudaGetLastError();

@@ -134,7 +134,7 @@ static int launch_fft(ofdm_ctx* ctx, const void* in, void* out, int64_t n_batch,
     if (!tw) return ctx_fail(ctx, OFDM_ERR_CUDA, "twiddle table allocation failed");
     size_t smem = 2 * (size_t)N * sizeof(cx<T>);
     auto kern = fft_kernel<T, MODE, INV>;
-    if (smem > 48 * 1024) CUDA_TRY(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    if (smem > 48 * 1024) CUDA_TRY(ctx, func_smem_optin((const void*)kern, (int)smem));
     int64_t done = 0;
     while (done < n_batch) {  // gridDim.x limit is 2^31-1; chunk anyway
         int64_t nb = std::min<int64_t>(n_batch - done, 1 << 30);

@@ -123,7 +123,7 @@ extern "C" int ofdm_window_papr(ofdm_ctx* ctx, const void* x, int64_t B, int64_t
     DISPATCH_T(ctx, {
         const size_t smem = 2 * (size_t)W * (sizeof(double) + sizeof(T));
         auto k = window_papr_kernel<T>;
-        if (smem > 48 * 1024) CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        if (smem > 48 * 1024) CUDA_TRY(ctx, func_smem_optin((const void*)k, (int)smem));
         k<<<dim3((unsigned)B, (unsigned)cdiv64(n_out, W)), PAPR_THREADS, smem, ctx->stream>>>((const cx<T>*)x, L, W, n_out, (T*)paprs);
     });
     LAUNCH_CHECK(ctx);
@@ -284,7 +284,7 @@ int ofdm_papr_stats(ofdm_ctx* ctx, const void* x, int64_t B, int64_t L, int W, c
     const void* k = ctx->precision == OFDM_PREC_F64 ? papr_stats_kernel_for<double>(W) : papr_stats_kernel_for<float>(W);
     REQUIRE(ctx, k != nullptr, "no statistics kernel for this window length");
     const size_t smem = papr_stats_smem(ctx->precision, W, n_bins);
-    CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    CUDA_TRY(ctx, func_smem_optin((const void*)k, (int)smem));
     int per_sm = 0;
     CUDA_TRY(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k, PAPR_THREADS, smem));
     int64_t n_out = L - W + 1, nbw = cdiv64(n_out, W);

@@ -229,8 +229,8 @@ static int pursuit_common(ofdm_ctx* ctx, const void* y, int64_t B, int Np, const
         auto kd = pursuit_kernel<T, true, IS_OMP>;
         auto kf = pursuit_kernel<T, false, IS_OMP>;
         // static shared (Gram + Cholesky factor, ~34 KB) plus dynamic can pass 48 KB: always opt in
-        CUDA_TRY(ctx, cudaFuncSetAttribute(kd, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max<size_t>(smem, 64 * 1024)));
-        CUDA_TRY(ctx, cudaFuncSetAttribute(kf, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max<size_t>(smem, 64 * 1024)));
+        CUDA_TRY(ctx, func_smem_optin((const void*)kd, (int)std::max<size_t>(smem, 64 * 1024)));
+        CUDA_TRY(ctx, func_smem_optin((const void*)kf, (int)std::max<size_t>(smem, 64 * 1024)));
         if (A) kd<<<(unsigned)B, PU_THREADS, smem, ctx->stream>>>((const C*)y, Np, At, Ldict, nullptr, Nfft, ilog2(Nfft), (const C*)tw, norms, K, (C*)H, (C*)h, index, iters, near_ties, (T)tie_eps);
         else kf<<<(unsigned)B, PU_THREADS, smem, ctx->stream>>>((const C*)y, Np, nullptr, Ldict, p0, Nfft, ilog2(Nfft), (const C*)tw, nullptr, K, (C*)H, (C*)h, index, iters, near_ties, (T)tie_eps);
         ctx->launches++;

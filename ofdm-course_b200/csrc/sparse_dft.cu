@@ -406,7 +406,7 @@ int ofdm_omp_dft(ofdm_ctx* ctx, const void* y, int64_t B, int Np, const int32_t*
     omp_dft_gram_kernel<<<(Nfft + 63) / 64, 64, 0, ctx->stream>>>(p0_dev, Np, Nfft, tw_d, g_d, g_f);
     const size_t smem = sizeof(float2) * 2 * (size_t)Nfft;
     auto kern = Ldict <= 1024 ? omp_dft_kernel<4> : (Ldict <= 2048 ? omp_dft_kernel<8> : omp_dft_kernel<16>);
-    cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    func_smem_optin((const void*)kern, (int)smem);
     kern<<<(unsigned)B, OD_THREADS, smem, ctx->stream>>>((const float2*)y, Np, p0_dev, Ldict, Nfft, ilog2(Nfft), tw, tw_d, g_f, g_d, K, (float2*)H, (float2*)h,
                                                          index, iters, near_ties, (float)tie_eps);
     ctx->launches += 2;

@@ -327,9 +327,9 @@ int ofdm_omp_tc(ofdm_ctx* ctx, const void* y, int64_t B, int Np, const void* A, 
     if (!tc_make_kmajor_map(&mapA, Rt, (uint64_t)Bpad, (uint64_t)K2) || !tc_make_kmajor_map(&mapB, Bt, (uint64_t)2 * Lpad, (uint64_t)K2))
         rc = ctx_fail(ctx, OFDM_ERR_CUDA, "cuTensorMapEncodeTiled failed");
     if (rc == OFDM_OK) {
-        cudaFuncSetAttribute(tc_corr_top_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM_TOP_BYTES);
+        func_smem_optin((const void*)tc_corr_top_kernel, TC_SMEM_TOP_BYTES);
         const size_t smem_step = sizeof(float2) * 2 * (size_t)Np;
-        cudaFuncSetAttribute(omp_tc_step_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max<size_t>(smem_step, 64 * 1024));
+        func_smem_optin((const void*)omp_tc_step_kernel, (int)std::max<size_t>(smem_step, 64 * 1024));
         for (int it = 0; it < K; ++it) {
             tc_corr_top_kernel<<<(unsigned)(Bpad / TC_BM), TC_THREADS, TC_SMEM_TOP_BYTES, st>>>(mapA, mapB, 2 * Lpad / TC_BN, K2, Ldict, cand, score);
             omp_tc_step_kernel<<<(unsigned)B, TS_THREADS, smem_step, st>>>((const float2*)y, (const float2*)A, Np, Ldict, K2, it, cand, score, Rt, sel, nsel, xs, Gs, rhs, K, fb, near_ties, (float)tie_eps);

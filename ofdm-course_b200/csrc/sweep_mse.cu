@@ -189,8 +189,8 @@ extern "C" int ofdm_sweep_mse(ofdm_ctx* ctx, const ofdm_link_params* lp, const o
     ofdm_link_params lp_tx = *lp;                             // as ofdm_sweep_ber: the Philox words are mapped without the scrambler
     lp_tx.scramble = 0;
     if (rc == OFDM_OK && fe_smem > 48 * 1024) {
-        cudaError_t e = f64 ? cudaFuncSetAttribute(mse_front_end_kernel<double>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fe_smem)
-                            : cudaFuncSetAttribute(mse_front_end_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fe_smem);
+        cudaError_t e = f64 ? func_smem_optin((const void*)mse_front_end_kernel<double>, (int)fe_smem)
+                            : func_smem_optin((const void*)mse_front_end_kernel<float>, (int)fe_smem);
         if (e != cudaSuccess) rc = ctx_fail(ctx, OFDM_ERR_CUDA, "front-end shared-memory opt-in failed: %s", cudaGetErrorString(e));
     }
 

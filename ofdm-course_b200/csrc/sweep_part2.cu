@@ -240,10 +240,10 @@ extern "C" int ofdm_sweep_part2(ofdm_ctx* ctx, const ofdm_link_params* base, con
     const void* tw = ctx_twiddles(ctx, Nfft);
     if (rc == OFDM_OK && !tw) rc = ctx_fail(ctx, OFDM_ERR_CUDA, "twiddle table allocation failed");
     if (rc == OFDM_OK && smem > 48 * 1024) {
-        cudaError_t e1 = f64 ? cudaFuncSetAttribute(part2_front_end_kernel<double>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)
-                             : cudaFuncSetAttribute(part2_front_end_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        cudaError_t e2 = f64 ? cudaFuncSetAttribute(part2_decide_kernel<double>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)
-                             : cudaFuncSetAttribute(part2_decide_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        cudaError_t e1 = f64 ? func_smem_optin((const void*)part2_front_end_kernel<double>, (int)smem)
+                             : func_smem_optin((const void*)part2_front_end_kernel<float>, (int)smem);
+        cudaError_t e2 = f64 ? func_smem_optin((const void*)part2_decide_kernel<double>, (int)smem)
+                             : func_smem_optin((const void*)part2_decide_kernel<float>, (int)smem);
         if (e1 != cudaSuccess || e2 != cudaSuccess)
             rc = ctx_fail(ctx, OFDM_ERR_CUDA, "shared-memory opt-in failed: %s", cudaGetErrorString(e1 != cudaSuccess ? e1 : e2));
     }

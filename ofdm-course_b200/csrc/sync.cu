@@ -300,7 +300,7 @@ extern "C" int ofdm_cp_autocorr(ofdm_ctx* ctx, const void* rx, int64_t B, int64_
                                                                         second ? list : nullptr, second ? n_list : nullptr);
             } else {
                 auto k1 = (W & 15) ? autocorr_kernel<T, false> : autocorr_kernel<T, true>;
-                if (smem > 48 * 1024) CUDA_TRY(ctx, cudaFuncSetAttribute(k1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+                if (smem > 48 * 1024) CUDA_TRY(ctx, func_smem_optin((const void*)k1, (int)smem));
                 k1<<<dim3((unsigned)B, tiles), AC_THREADS, smem, ctx->stream>>>((const cx<T>*)rx, L, W, Nfft, n_scan, tile, (cx<T>*)autocorr, flags, fw, gate);
             }
             ctx->launches++;
@@ -360,7 +360,7 @@ extern "C" int ofdm_remove_ifo(ofdm_ctx* ctx, const void* rx, int64_t B, int64_t
     DISPATCH_T(ctx, {
         size_t smem = 2 * (size_t)Nfft * sizeof(cx<T>);
         auto k1 = ifo_detect_kernel<T>;
-        if (smem > 48 * 1024) CUDA_TRY(ctx, cudaFuncSetAttribute(k1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        if (smem > 48 * 1024) CUDA_TRY(ctx, func_smem_optin((const void*)k1, (int)smem));
         k1<<<(unsigned)B, fft_threads(Nfft), smem, ctx->stream>>>((const cx<T>*)rx, L, Nfft, ilog2(Nfft), (const cx<T>*)tw, ifo);
         ctx->launches++;
         ifo_derotate_kernel<T><<<(unsigned)cdiv64(B * L, 256), 256, 0, ctx->stream>>>((const cx<T>*)rx, B, L, Nfft, (const cx<T>*)tw, ifo, (cx<T>*)out);
@@ -461,7 +461,7 @@ extern "C" int ofdm_fine_sync(ofdm_ctx* ctx, const void* grid, int64_t B, int S,
     size_t smem = sizeof(double) * (size_t)(Np * S);
     DISPATCH_T(ctx, {
         auto k1 = fine_sync_est_kernel<T>;
-        if (smem > 48 * 1024) CUDA_TRY(ctx, cudaFuncSetAttribute(k1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        if (smem > 48 * 1024) CUDA_TRY(ctx, func_smem_optin((const void*)k1, (int)smem));
         k1<<<(unsigned)B, FS_THREADS, smem, ctx->stream>>>((const cx<T>*)grid, S, Nfft, pc0, Np, txp, time_desync, tau_dev, phase_dev);
         ctx->launches++;
         int64_t n = B * S * (int64_t)Nfft;

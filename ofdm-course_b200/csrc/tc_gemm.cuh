@@ -21,13 +21,16 @@
 // ---------------------------------------------------------------- host: tensor maps
 typedef CUresult (*tc_encode_fn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*, const cuuint32_t*,
                                  const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+// The lookup runs once, under the C++ guarantee for function-local statics, so contexts on several host threads
+// (ofdm_group) never race on it.
 static inline tc_encode_fn tc_get_encode() {
-    static tc_encode_fn fn = nullptr;
-    if (!fn) {
+    static const tc_encode_fn fn = [] {
         void* p = nullptr;
         cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess) fn = (tc_encode_fn)p;
-    }
+        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
+            return (tc_encode_fn)p;
+        return (tc_encode_fn) nullptr;
+    }();
     return fn;
 }
 // rows x K FP32 matrix, K contiguous; box = 128 rows x 32 floats (128 B), 128B swizzle

@@ -167,12 +167,10 @@ def reduce_part2(per_run, counts, runs):
     return NMSE, BER, per, cnt, rn
 
 
-def sweep_lib_local(ctx, combs, mc_runs, payload_bits, *, tile=0, rank=0, world=1, reg_pilot=True, random_masks=None, profile="EPA",
-                    fs_hz=4e7, snr_db=20.0, seed=1, near_eps=0.0, tie_eps=0.0, Nfft=4096, N_carrier=1024, frames=2, spf=7,
-                    constellation="16QAM", per_run=None, counts=None, runs=None):
-    """This rank's share of the experiment through ``ofdm_sweep_part2``, WITHOUT synchronising: writes its cells of ``per_run``
-    (n_points, 4, mc_runs) float64 and adds to ``counts`` (n_points, 4, 3) and ``runs`` (n_points, 2) int64; all three are
-    zero-initialised device tensors when not given.  ``payload_bits``: uint8 0/1, at least the longest stream of any point."""
+def lib_params(combs, mc_runs, payload_bits, *, tile=0, rank=0, world=1, reg_pilot=True, random_masks=None, profile="EPA", fs_hz=4e7,
+               snr_db=20.0, seed=1, near_eps=0.0, tie_eps=0.0, Nfft=4096, N_carrier=1024, frames=2, spf=7, constellation="16QAM"):
+    """(``ofdm_link_params``, ``ofdm_part2_params``) of :func:`sweep_lib_local`'s arguments (host arrays kept alive on the
+    part-2 params)."""
     from . import _cabi
     from . import link as G
     offsets, carriers, ldict = lib_layout(combs, N_carrier, Nfft, reg_pilot, random_masks)
@@ -197,6 +195,17 @@ def sweep_lib_local(ctx, combs, mc_runs, payload_bits, *, tile=0, rank=0, world=
     pp.mc_runs, pp.tile_runs = int(mc_runs), int(tile)
     pp.rank, pp.world, pp.seed = int(rank), int(world), int(seed)
     pp.near_eps, pp.tie_eps = float(near_eps), float(tie_eps)
+    pp._keep = (offsets, carriers, ldict, pattern, words)
+    return lp, pp
+
+
+def sweep_lib_local(ctx, combs, mc_runs, payload_bits, *, tile=0, rank=0, world=1, per_run=None, counts=None, runs=None, **kw):
+    """This rank's share of the experiment through ``ofdm_sweep_part2``, WITHOUT synchronising: writes its cells of ``per_run``
+    (n_points, 4, mc_runs) float64 and adds to ``counts`` (n_points, 4, 3) and ``runs`` (n_points, 2) int64; all three are
+    zero-initialised device tensors when not given.  ``payload_bits``: uint8 0/1, at least the longest stream of any point.
+    The other keywords are those of :func:`lib_params`."""
+    lp, pp = lib_params(combs, mc_runs, payload_bits, tile=tile, rank=rank, world=world, **kw)
+    n_pts = pp.n_points
     if per_run is None:
         per_run = torch.zeros((n_pts, 4, int(mc_runs)), dtype=torch.float64, device=ctx.device)
     if counts is None:

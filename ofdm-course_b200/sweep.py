@@ -78,10 +78,9 @@ def run_sweep(snrs_db, streams_per_point, tile, compute, rank=0, world=1, device
     return reduce_counts(torch.from_numpy(local), device).cpu().numpy()
 
 
-def sweep_local(ctx, lp, snrs_db, streams_per_point, taps=None, chain="task5", seed=1, rank=0, world=1, tile=0, near_eps=0.0,
-                sto_max=None, cfo_int_max=30, counts=None):
-    """This rank's share of the sweep through ``ofdm_sweep_ber``; returns the device counters (n_snr, 4) int64
-    {errors, bits, near-boundary symbols, detector failures} WITHOUT synchronising (everything is stream-ordered)."""
+def sweep_params(lp, snrs_db, streams_per_point, taps=None, chain="task5", seed=1, rank=0, world=1, tile=0, near_eps=0.0,
+                 sto_max=None, cfo_int_max=30):
+    """The ``ofdm_sweep_params`` of :func:`sweep_local`'s arguments (its host arrays are kept alive on the returned object)."""
     snr = np.ascontiguousarray(np.asarray(snrs_db, dtype=np.float64))
     sp = _cabi.SweepParams()
     sp.chain = CHAINS[chain]
@@ -99,8 +98,17 @@ def sweep_local(ctx, lp, snrs_db, streams_per_point, taps=None, chain="task5", s
     sp.near_eps = float(near_eps)
     sp.sto_max = int(lp.Nfft + lp.Tg if sto_max is None else sto_max)
     sp.cfo_int_max = int(cfo_int_max)
+    sp._keep = (snr, t)
+    return sp
+
+
+def sweep_local(ctx, lp, snrs_db, streams_per_point, taps=None, chain="task5", seed=1, rank=0, world=1, tile=0, near_eps=0.0,
+                sto_max=None, cfo_int_max=30, counts=None):
+    """This rank's share of the sweep through ``ofdm_sweep_ber``; returns the device counters (n_snr, 4) int64
+    {errors, bits, near-boundary symbols, detector failures} WITHOUT synchronising (everything is stream-ordered)."""
+    sp = sweep_params(lp, snrs_db, streams_per_point, taps, chain, seed, rank, world, tile, near_eps, sto_max, cfo_int_max)
     if counts is None:
-        counts = torch.zeros((snr.size, 4), dtype=torch.int64, device=ctx.device)
+        counts = torch.zeros((sp.n_snr, 4), dtype=torch.int64, device=ctx.device)
     ctx._chk(ctx.lib.ofdm_sweep_ber(ctx.h, C.byref(lp), C.byref(sp), ctx.p(counts)))
     return counts
 
@@ -138,11 +146,8 @@ def run_mse_sweep(snrs_db, streams_per_point, tile, compute, rank=0, world=1):
     return reduce_mse(per, counts)
 
 
-def mse_sweep_local(ctx, lp, snrs_db, streams_per_point, taps, Ldict=None, seed=1, rank=0, world=1, tile=0, tie_eps=0.0, per_stream=None, counts=None):
-    """This rank's share of the MSE sweep through ``ofdm_sweep_mse``, WITHOUT synchronising: writes its cells of
-    ``per_stream`` (n_snr, 4, streams_per_point) float64 and adds to ``counts`` (n_snr, 2) int64 {streams, OMP frames with a
-    near-tie}; both are zero-initialised device tensors when not given.  ``Ldict`` defaults to the script's
-    ceil(N_carrier / comb) (`Main_model_Task_5.m:182-190`)."""
+def mse_params(lp, snrs_db, streams_per_point, taps, Ldict=None, seed=1, rank=0, world=1, tile=0, tie_eps=0.0):
+    """(``ofdm_sweep_params``, Ldict) of :func:`mse_sweep_local`'s arguments (host arrays kept alive on the params)."""
     snr = np.ascontiguousarray(np.asarray(snrs_db, dtype=np.float64))
     pc = np.asarray(lp.pilotCarriers)
     if Ldict is None:
@@ -159,11 +164,21 @@ def mse_sweep_local(ctx, lp, snrs_db, streams_per_point, taps, Ldict=None, seed=
     sp.taps_host = t.ctypes.data_as(_cabi.pdbl)
     sp.n_taps = t.shape[0]
     sp.near_eps = float(tie_eps)
+    sp._keep = (snr, t)
+    return sp, int(Ldict)
+
+
+def mse_sweep_local(ctx, lp, snrs_db, streams_per_point, taps, Ldict=None, seed=1, rank=0, world=1, tile=0, tie_eps=0.0, per_stream=None, counts=None):
+    """This rank's share of the MSE sweep through ``ofdm_sweep_mse``, WITHOUT synchronising: writes its cells of
+    ``per_stream`` (n_snr, 4, streams_per_point) float64 and adds to ``counts`` (n_snr, 2) int64 {streams, OMP frames with a
+    near-tie}; both are zero-initialised device tensors when not given.  ``Ldict`` defaults to the script's
+    ceil(N_carrier / comb) (`Main_model_Task_5.m:182-190`)."""
+    sp, Ldict = mse_params(lp, snrs_db, streams_per_point, taps, Ldict, seed, rank, world, tile, tie_eps)
     if per_stream is None:
-        per_stream = torch.zeros((snr.size, 4, int(streams_per_point)), dtype=torch.float64, device=ctx.device)
+        per_stream = torch.zeros((sp.n_snr, 4, int(streams_per_point)), dtype=torch.float64, device=ctx.device)
     if counts is None:
-        counts = torch.zeros((snr.size, 2), dtype=torch.int64, device=ctx.device)
-    ctx._chk(ctx.lib.ofdm_sweep_mse(ctx.h, C.byref(lp), C.byref(sp), int(Ldict), ctx.p(per_stream), ctx.p(counts)))
+        counts = torch.zeros((sp.n_snr, 2), dtype=torch.int64, device=ctx.device)
+    ctx._chk(ctx.lib.ofdm_sweep_mse(ctx.h, C.byref(lp), C.byref(sp), Ldict, ctx.p(per_stream), ctx.p(counts)))
     return per_stream, counts
 
 
@@ -239,13 +254,9 @@ def run_sync_sweep(snrs_db, streams_per_point, tile, compute, rank=0, world=1, *
     return reduce_sync(rec, counts, **reduce_kw)
 
 
-def sync_sweep_local(ctx, lp, snrs_db, streams_per_point, taps=None, seed=1, rank=0, world=1, tile=0, sto=None, cfo=None, sto_max=None,
-                     cfo_int_max=30, time_desync=True, freq_desync=True, mp_desync=True, rec=None, counts=None):
-    """This rank's share of the sync sweep through ``ofdm_sweep_sync``, WITHOUT synchronising: writes its cells of ``rec``
-    (n_snr, 9, streams_per_point) float64, fields :data:`SYNC_FIELDS`, and adds to ``counts`` (n_snr, 4) int64 {bit errors,
-    bits, detector failures, IFO misses}; both are zero-initialised device tensors when not given.  With ``sto`` and ``cfo``
-    every stream gets that STO / CFO; otherwise they are drawn as :func:`sweep_local` draws them (``sto_max`` defaults to
-    Nfft + Tg)."""
+def sync_params(lp, snrs_db, streams_per_point, taps=None, seed=1, rank=0, world=1, tile=0, sto=None, cfo=None, sto_max=None,
+                cfo_int_max=30, time_desync=True, freq_desync=True, mp_desync=True):
+    """The ``ofdm_sync_params`` of :func:`sync_sweep_local`'s arguments (host arrays kept alive on the returned object)."""
     snr = np.ascontiguousarray(np.asarray(snrs_db, dtype=np.float64))
     sp = _cabi.SyncParams()
     sp.n_snr = snr.size
@@ -266,10 +277,23 @@ def sync_sweep_local(ctx, lp, snrs_db, streams_per_point, taps=None, seed=1, ran
     sp.sto_max = int(lp.Nfft + lp.Tg if sto_max is None else sto_max)
     sp.cfo_int_max = int(cfo_int_max)
     sp.time_desync, sp.freq_desync, sp.mp_desync = int(bool(time_desync)), int(bool(freq_desync)), int(bool(mp_desync))
+    sp._keep = (snr, t)
+    return sp
+
+
+def sync_sweep_local(ctx, lp, snrs_db, streams_per_point, taps=None, seed=1, rank=0, world=1, tile=0, sto=None, cfo=None, sto_max=None,
+                     cfo_int_max=30, time_desync=True, freq_desync=True, mp_desync=True, rec=None, counts=None):
+    """This rank's share of the sync sweep through ``ofdm_sweep_sync``, WITHOUT synchronising: writes its cells of ``rec``
+    (n_snr, 9, streams_per_point) float64, fields :data:`SYNC_FIELDS`, and adds to ``counts`` (n_snr, 4) int64 {bit errors,
+    bits, detector failures, IFO misses}; both are zero-initialised device tensors when not given.  With ``sto`` and ``cfo``
+    every stream gets that STO / CFO; otherwise they are drawn as :func:`sweep_local` draws them (``sto_max`` defaults to
+    Nfft + Tg)."""
+    sp = sync_params(lp, snrs_db, streams_per_point, taps, seed, rank, world, tile, sto, cfo, sto_max, cfo_int_max, time_desync, freq_desync,
+                     mp_desync)
     if rec is None:
-        rec = torch.zeros((snr.size, 9, int(streams_per_point)), dtype=torch.float64, device=ctx.device)
+        rec = torch.zeros((sp.n_snr, 9, int(streams_per_point)), dtype=torch.float64, device=ctx.device)
     if counts is None:
-        counts = torch.zeros((snr.size, 4), dtype=torch.int64, device=ctx.device)
+        counts = torch.zeros((sp.n_snr, 4), dtype=torch.int64, device=ctx.device)
     ctx._chk(ctx.lib.ofdm_sweep_sync(ctx.h, C.byref(lp), C.byref(sp), ctx.p(rec), ctx.p(counts)))
     return rec, counts
 
@@ -283,13 +307,8 @@ def sync_sweep(ctx, lp, snrs_db, streams_per_point, taps=None, seed=1, rank=0, w
     return reduce_sync(rec, cnt, h_power=channel_power(taps, lp.Nfft, lp.N_carrier), sym_len=lp.Nfft + lp.Tg, cfo_tol=cfo_tol)
 
 
-def papr_sweep_local(ctx, lp, points, streams_per_point, seed=1, rank=0, world=1, tile=0, bin_db=0.01, n_bins=4000, pool=None, pool_stride=0,
-                     hist=None, papr=None):
-    """This rank's share of the PAPR study through ``ofdm_sweep_papr``, WITHOUT synchronising.  ``points``: a list of
-    ``(scramble, p_one)``; ``p_one`` is P(bit = 1) of the Philox payload and is ignored when ``pool`` (0/1 payload bits, e.g.
-    ``realisations.file_reader``) is given: stream j then transmits pool bits (j * pool_stride + i) mod len(pool).  Writes
-    its cells of ``papr`` (n_points, streams_per_point) float64 and adds to ``hist`` (n_points, n_bins) int64, window
-    PAPR v in bin min(floor(v / bin_db), n_bins - 1); both are zero-initialised device tensors when not given."""
+def papr_params(points, streams_per_point, seed=1, rank=0, world=1, tile=0, bin_db=0.01, n_bins=4000, pool=None, pool_stride=0):
+    """The ``ofdm_papr_params`` of :func:`papr_sweep_local`'s arguments (host arrays kept alive on the returned object)."""
     pts = [(int(bool(s)), p) for s, p in points]
     scr = np.ascontiguousarray(np.array([s for s, _ in pts], dtype=np.int32))
     pone = np.ascontiguousarray(np.array([0.5 if p is None else float(p) for _, p in pts], dtype=np.float64))
@@ -311,10 +330,22 @@ def papr_sweep_local(ctx, lp, points, streams_per_point, seed=1, rank=0, world=1
     pp.seed = int(seed)
     pp.bin_db = float(bin_db)
     pp.n_bins = int(n_bins)
+    pp._keep = (scr, pone, words)
+    return pp
+
+
+def papr_sweep_local(ctx, lp, points, streams_per_point, seed=1, rank=0, world=1, tile=0, bin_db=0.01, n_bins=4000, pool=None, pool_stride=0,
+                     hist=None, papr=None):
+    """This rank's share of the PAPR study through ``ofdm_sweep_papr``, WITHOUT synchronising.  ``points``: a list of
+    ``(scramble, p_one)``; ``p_one`` is P(bit = 1) of the Philox payload and is ignored when ``pool`` (0/1 payload bits, e.g.
+    ``realisations.file_reader``) is given: stream j then transmits pool bits (j * pool_stride + i) mod len(pool).  Writes
+    its cells of ``papr`` (n_points, streams_per_point) float64 and adds to ``hist`` (n_points, n_bins) int64, window
+    PAPR v in bin min(floor(v / bin_db), n_bins - 1); both are zero-initialised device tensors when not given."""
+    pp = papr_params(points, streams_per_point, seed, rank, world, tile, bin_db, n_bins, pool, pool_stride)
     if hist is None:
-        hist = torch.zeros((len(pts), int(n_bins)), dtype=torch.int64, device=ctx.device)
+        hist = torch.zeros((pp.n_points, int(n_bins)), dtype=torch.int64, device=ctx.device)
     if papr is None:
-        papr = torch.zeros((len(pts), int(streams_per_point)), dtype=torch.float64, device=ctx.device)
+        papr = torch.zeros((pp.n_points, int(streams_per_point)), dtype=torch.float64, device=ctx.device)
     ctx._chk(ctx.lib.ofdm_sweep_papr(ctx.h, C.byref(lp), C.byref(pp), ctx.p(papr), ctx.p(hist)))
     return hist, papr
 
@@ -367,3 +398,90 @@ def papr_sweep(ctx, lp, points, streams_per_point, seed=1, rank=0, world=1, tile
     hist, papr = papr_sweep_local(ctx, lp, points, streams_per_point, seed, rank, world, tile, bin_db, n_bins, pool, pool_stride)
     ctx.sync()
     return reduce_papr(hist, papr, bin_db)
+
+
+class Group:
+    """Several GPUs of this process as ONE ``ofdm_group`` (include/ofdm_b200.h): each method runs a sweep's shares on all
+    members at once, one host thread per member inside the library, and returns the assembled host arrays as NumPy --
+    bit-identical to the single-context call with world 1, without ``torch.distributed``.  ``devices``: CUDA ordinals
+    (0-based, repeats allowed); member i is rank i.  The methods take the arguments of the matching ``*_sweep_local``
+    function without rank / world / output tensors."""
+
+    def __init__(self, devices, precision="f32"):
+        from .link import OfdmError
+        self.lib = _cabi.load()
+        ids = np.ascontiguousarray(np.asarray(list(devices), dtype=np.int32))
+        h = C.c_void_p()
+        rc = self.lib.ofdm_group_create(C.byref(h), ids.ctypes.data_as(_cabi.pi32), int(ids.size), 1 if precision in ("f64", 1, "double") else 0)
+        if rc != 0:
+            err = OfdmError(f"status {rc}: ofdm_group_create failed for devices {ids.tolist()}")
+            err.status = rc
+            raise err
+        self.h = h
+        self.devices = tuple(int(d) for d in ids)
+
+    def close(self):
+        if getattr(self, "h", None):
+            self.lib.ofdm_group_destroy(self.h)
+            self.h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def _chk(self, rc):
+        if rc != 0:
+            from .link import OfdmError
+            err = OfdmError(f"status {rc}: {self.lib.ofdm_group_last_error(self.h).decode()}")
+            err.status = rc
+            raise err
+
+    def sweep_ber(self, lp, snrs_db, streams_per_point, taps=None, chain="task5", seed=1, tile=0, near_eps=0.0, sto_max=None, cfo_int_max=30):
+        """Counters (n_snr, 4) int64 of :func:`sweep_local`."""
+        sp = sweep_params(lp, snrs_db, streams_per_point, taps, chain, seed, 0, 1, tile, near_eps, sto_max, cfo_int_max)
+        counts = np.zeros((sp.n_snr, 4), dtype=np.int64)
+        self._chk(self.lib.ofdm_group_sweep_ber(self.h, C.byref(lp), C.byref(sp), counts.ctypes.data))
+        return counts
+
+    def sweep_mse(self, lp, snrs_db, streams_per_point, taps, Ldict=None, seed=1, tile=0, tie_eps=0.0):
+        """(per_stream (n_snr, 4, streams_per_point) float64, counts (n_snr, 2) int64) of :func:`mse_sweep_local`."""
+        sp, Ldict = mse_params(lp, snrs_db, streams_per_point, taps, Ldict, seed, 0, 1, tile, tie_eps)
+        per = np.zeros((sp.n_snr, 4, int(streams_per_point)), dtype=np.float64)
+        counts = np.zeros((sp.n_snr, 2), dtype=np.int64)
+        self._chk(self.lib.ofdm_group_sweep_mse(self.h, C.byref(lp), C.byref(sp), Ldict, per.ctypes.data, counts.ctypes.data))
+        return per, counts
+
+    def sweep_sync(self, lp, snrs_db, streams_per_point, taps=None, seed=1, tile=0, **kw):
+        """(rec (n_snr, 9, streams_per_point) float64, counts (n_snr, 4) int64) of :func:`sync_sweep_local`."""
+        sp = sync_params(lp, snrs_db, streams_per_point, taps, seed, 0, 1, tile, **kw)
+        rec = np.zeros((sp.n_snr, 9, int(streams_per_point)), dtype=np.float64)
+        counts = np.zeros((sp.n_snr, 4), dtype=np.int64)
+        self._chk(self.lib.ofdm_group_sweep_sync(self.h, C.byref(lp), C.byref(sp), rec.ctypes.data, counts.ctypes.data))
+        return rec, counts
+
+    def sweep_papr(self, lp, points, streams_per_point, seed=1, tile=0, bin_db=0.01, n_bins=4000, pool=None, pool_stride=0):
+        """(hist (n_points, n_bins) int64, papr (n_points, streams_per_point) float64) of :func:`papr_sweep_local`."""
+        pp = papr_params(points, streams_per_point, seed, 0, 1, tile, bin_db, n_bins, pool, pool_stride)
+        hist = np.zeros((pp.n_points, int(n_bins)), dtype=np.int64)
+        papr = np.zeros((pp.n_points, int(streams_per_point)), dtype=np.float64)
+        self._chk(self.lib.ofdm_group_sweep_papr(self.h, C.byref(lp), C.byref(pp), papr.ctypes.data, hist.ctypes.data))
+        return hist, papr
+
+    def sweep_part2(self, combs, mc_runs, payload_bits, *, tile=0, **kw):
+        """(per_run (n_points, 4, mc_runs) float64, counts (n_points, 4, 3) int64, runs (n_points, 2) int64) of
+        ``part2.sweep_lib_local``; keywords as ``part2.lib_params``."""
+        from .part2 import lib_params
+        lp, pp = lib_params(combs, mc_runs, payload_bits, tile=tile, **kw)
+        per = np.zeros((pp.n_points, 4, int(mc_runs)), dtype=np.float64)
+        counts = np.zeros((pp.n_points, 4, 3), dtype=np.int64)
+        runs = np.zeros((pp.n_points, 2), dtype=np.int64)
+        self._chk(self.lib.ofdm_group_sweep_part2(self.h, C.byref(lp), C.byref(pp), per.ctypes.data, counts.ctypes.data, runs.ctypes.data))
+        return per, counts, runs
