@@ -312,9 +312,9 @@ OFDM_API int ofdm_rx_chain_t4_ex(ofdm_ctx*, const ofdm_link_params*, const void*
                                  double* phase_dev, void* H_dev, double near_eps, int32_t* fail_dev);
 
 /* ---- Monte-Carlo BER-vs-SNR sweep (the script loops) ------------------------------------------ */
-/* Replaces the SNR loops `Task 3/Main_model_Task_3.m:192-268` / `Task 5/Main_model_Task_5.m:303-346` (chain
- * OFDM_SWEEP_TASK5: TX chain -> Noise -> multipath -> M1 RX chain; the BER half of the Task-5 loop, ofdm_sweep_mse below
- * runs its channel-estimation half) and the impaired channel of
+/* Replaces the SNR loop `Task 5/Main_model_Task_5.m:303-346` (chain OFDM_SWEEP_TASK5: TX chain -> Noise -> multipath -> M1
+ * RX chain; the BER half of the Task-5 loop, ofdm_sweep_mse below runs its channel-estimation half; Task 3's loop, which has
+ * no channel estimate, is ofdm_sweep_mer) and the impaired channel of
  * `Task 4/Main_model_Task_4.m:95-110,252-264,277-366` swept over SNR (chain OFDM_SWEEP_TASK4: TX chain -> Noise ->
  * add_STO -> add_CFO -> multipath -> M2 RX chain with AutoCorrFunction / remove_IFO / fine_sync / estimate_channel).
  * Streams are numbered globally, g = snr_index * streams_per_point + j; payload bits, noise, STO and CFO draws are
@@ -457,6 +457,42 @@ typedef struct ofdm_papr_params {
     int32_t n_bins;                 /* 1 .. 16384; the last bin also takes everything above it */
 } ofdm_papr_params;
 OFDM_API int ofdm_sweep_papr(ofdm_ctx*, const ofdm_link_params*, const ofdm_papr_params*, double* papr_dev, int64_t* hist_dev);
+/* Task-3 BER and MER study over constellations and SNR (`Task 3/Main_model_Task_3.m:192-268`, `Task 3/README.md:53-55`): per
+ * stream TX -> Noise -> add_STO -> add_CFO -> multipath -> OFDM_demodulator -> get_payload -> demapping -> DeScrambler -> BER
+ * and MER_func.  Task 3 has no synchroniser, estimator or equaliser: the STO, CFO and multipath reach the decisions
+ * uncorrected.  Point k has its own constellation, SNR and fixed STO / CFO.  From `lp` the call reads Nfft, Tg, N_carrier,
+ * S, SpF, the carriers, reg0 and scramble; lp->constellation is ignored.  Stream g = k * streams_per_point + j; the call
+ * processes the share ofdm_sweep_share(n_points * streams_per_point, rank, world) gives, in tiles that never straddle a point.
+ * Stream g carries the first S * Nd * bps_k bits of the Philox words ofdm_payload_bits draws for it, as one contiguous
+ * bitstream: these are the scrambled frames s, the payload is p = DeScrambler(s) (p = s when lp->scramble = 0), and the
+ * transmitter maps s without scrambling.  The channel is ofdm_channel_t4_p with the point's SNR, STO and CFO, so a call whose
+ * points share one constellation transmits, with equal pilot values, the streams ofdm_sweep_sync transmits for the same SNR
+ * list, seed and taps with sto_mode 1.  The receiver decides every symbol in the pass that transforms it: its bins and
+ * decisions are those of ofdm_rx_chain_t4_ex(..., 0, 0, 0, ...).  FP32 contexts and Nfft = 1024 only (OFDM_ERR_UNSUPPORTED
+ * otherwise); streams need not be word aligned.
+ * mer_dev: n_points x 2 x streams_per_point doubles, [k][f][j]: f = 0 the sum of |ideal|^2, f = 1 the sum of |ideal - rx|^2
+ * over the stream's data symbols, so MER_func of the stream is 10 log10(f0 / f1) dB; only this call's share is written, and
+ * each cell is summed in an order that depends on the stream shape only.
+ * counts_dev: n_points x 3 int64 += {bit errors after DeScrambler, bits, symbols within near_eps of a decision boundary}.
+ * The values do not depend on the rank count or the tile size; the caller sums both arrays over ranks (each MER cell is
+ * written by one rank). */
+typedef struct ofdm_mer_params {
+    int32_t n_points;
+    const int32_t* constellation_host; /* n_points: OFDM_BPSK .. OFDM_16QAM */
+    const double* snr_db_host;         /* n_points; +INFINITY = noise-free (Noise.m's noise power is then 0); not NaN */
+    double pilot_scale;                /* > 0: every pilot of point k is pilot_scale * max|constellation_func(c_k)|, real
+                                          (Task 3's scalar broadcast, `Main_model_Task_3.m:57-59`); 0: lp->pilot_vals_host */
+    const int32_t* nsto_host;          /* n_points or NULL (= 0): fixed add_STO offset, >= 0, not corrected */
+    const double* cfo_host;            /* n_points or NULL (= 0): fixed add_CFO offset, finite, not corrected */
+    const double* taps_host;           /* n_taps x 2 doubles (delay, amplitude), delays integers in [0, Nfft); n_taps = 0: no multipath */
+    int32_t n_taps;
+    int64_t streams_per_point;
+    int64_t tile_streams;              /* streams per work item; 0 = 8192 (two signal buffers of tile x stream bytes are allocated) */
+    int32_t rank, world;
+    uint64_t seed;
+    double near_eps;                   /* symbols whose two smallest squared distances differ by less are counted; 0 = off */
+} ofdm_mer_params;
+OFDM_API int ofdm_sweep_mer(ofdm_ctx*, const ofdm_link_params*, const ofdm_mer_params*, double* mer_dev, int64_t* counts_dev);
 /* first / count of the contiguous share of `total_streams` that (rank, world) processes */
 OFDM_API int ofdm_sweep_share(int64_t total_streams, int rank, int world, int64_t* first, int64_t* count);
 /* The sweep's synthetic inputs, also usable on their own: payload words of streams first_stream_id .. +n_streams-1
@@ -507,6 +543,8 @@ OFDM_API int ofdm_group_sweep_mse(ofdm_group*, const ofdm_link_params*, const of
 OFDM_API int ofdm_group_sweep_sync(ofdm_group*, const ofdm_link_params*, const ofdm_sync_params*, double* rec_host, int64_t* counts_host);
 /* papr_host: n_points x streams_per_point doubles; hist_host: n_points x n_bins int64 */
 OFDM_API int ofdm_group_sweep_papr(ofdm_group*, const ofdm_link_params*, const ofdm_papr_params*, double* papr_host, int64_t* hist_host);
+/* mer_host: n_points x 2 x streams_per_point doubles; counts_host: n_points x 3 int64 */
+OFDM_API int ofdm_group_sweep_mer(ofdm_group*, const ofdm_link_params*, const ofdm_mer_params*, double* mer_host, int64_t* counts_host);
 /* nmse_host: n_points x 4 x mc_runs doubles; counts_host: n_points x 4 x 3 int64; runs_host: n_points x 2 int64 */
 OFDM_API int ofdm_group_sweep_part2(ofdm_group*, const ofdm_link_params* base, const ofdm_part2_params*, double* nmse_host,
                                     int64_t* counts_host, int64_t* runs_host);

@@ -12,7 +12,7 @@
  * type, 0/1 double bits -> packed words, 1-based double indices -> int32, host <-> device copies.
  * No computation happens here and there is no CPU fallback: without an sm_100 GPU every op fails
  * with ofdm:ctx:nodevice.  The matlab/<Name>.m wrappers give each op the reference's signature.
- * The five sweep ops run on the device set of ofdm_mex('devices', ids) (0-based CUDA ids, default [0]: one context on
+ * The six sweep ops run on the device set of ofdm_mex('devices', ids) (0-based CUDA ids, default [0]: one context on
  * device 0); any other set runs them through one ofdm_group, every other op stays on device 0.
  */
 #include <math.h>
@@ -31,7 +31,7 @@
 
 static ofdm_ctx* g_ctx = NULL;
 static int g_prec = OFDM_PREC_F32;
-/* the device set of the five sweep ops (ofdm_mex('devices', ids), 0-based CUDA ids): [0] runs them on g_ctx, any other set
+/* the device set of the six sweep ops (ofdm_mex('devices', ids), 0-based CUDA ids): [0] runs them on g_ctx, any other set
  * on g_group, built on first use and rebuilt after a precision switch */
 #define MAX_DEVICES 64
 static int g_devices[MAX_DEVICES] = {0};
@@ -259,7 +259,7 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
     }
     ensure_ctx();
 
-    if (!strcmp(op, "devices")) {   /* ids = ofdm_mex('devices' [, ids]): the 0-based CUDA devices of the five sweep ops */
+    if (!strcmp(op, "devices")) {   /* ids = ofdm_mex('devices' [, ids]): the 0-based CUDA devices of the six sweep ops */
         if (nrhs > 1) {
             size_t n = mxGetNumberOfElements(A(0)), i;
             int ids[MAX_DEVICES];
@@ -799,6 +799,63 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
         OUT(0, rm);
         mxArray* cm = mxCreateDoubleMatrix(n, 4, mxREAL);
         for (i = 0; i < n; ++i) { int j; for (j = 0; j < 4; ++j) real_data(cm)[(size_t)j * n + i] = (double)ch[4 * i + j]; }
+        OUT(1, cm);
+    } else if (!strcmp(op, "sweep_mer")) {    /* [mer (spp x 2*n_points), counts (n_points x 3)] =
+                                                 sweep_mer(LINK..., constellations (ids 1..4, one per point), snrs (one per point),
+                                                 streams_per_point, taps (K x 2, [] = none), seed, sto, cfo, pilot_scale, near_eps);
+                                                 sto / cfo: one value for every point or one per point */
+        NEED(N_LINK + 9);
+        ofdm_link_params lp;
+        ofdm_mer_params mp;
+        parse_link(&A(0), &lp);
+        memset(&mp, 0, sizeof mp);
+        size_t n = mxGetNumberOfElements(A(N_LINK + 1)), i;
+        int K = (int)mxGetM(A(N_LINK + 3)), k2;
+        if (!n) fail("ofdm:sweep_mer:snr", "need at least one point");
+        if (mxGetNumberOfElements(A(N_LINK)) != n) fail("ofdm:sweep_mer:points", "need one constellation per SNR point");
+        if (K && mxGetN(A(N_LINK + 3)) != 2) fail("ofdm:sweep_mer:taps", "channel_taps must be K x 2 (delay, amplitude) or []");
+        size_t ns = mxGetNumberOfElements(A(N_LINK + 5)), nc = mxGetNumberOfElements(A(N_LINK + 6));
+        if ((ns != 1 && ns != n) || (nc != 1 && nc != n)) fail("ofdm:sweep_mer:impairments", "sto and cfo take one value or one per point");
+        int32_t* cons = (int32_t*)hostbuf(n * 8);
+        int32_t* nsto = cons + n;
+        double* cfo = (double*)hostbuf(n * 8);
+        for (i = 0; i < n; ++i) {
+            cons[i] = (int32_t)real_data(A(N_LINK))[i];
+            nsto[i] = (int32_t)real_data(A(N_LINK + 5))[ns == 1 ? 0 : i];
+            cfo[i] = real_data(A(N_LINK + 6))[nc == 1 ? 0 : i];
+        }
+        mp.n_points = (int32_t)n;
+        mp.constellation_host = cons;
+        mp.snr_db_host = real_data(A(N_LINK + 1));
+        mp.streams_per_point = (int64_t)mxGetScalar(A(N_LINK + 2));
+        mp.rank = 0; mp.world = 1;
+        mp.seed = (uint64_t)mxGetScalar(A(N_LINK + 4));
+        if (K) {
+            double* tp = real_data(A(N_LINK + 3));
+            double* taps = (double*)hostbuf((size_t)K * 16);
+            for (k2 = 0; k2 < K; ++k2) { taps[2 * k2] = tp[k2]; taps[2 * k2 + 1] = tp[K + k2]; }
+            mp.taps_host = taps; mp.n_taps = K;
+        }
+        mp.nsto_host = nsto;
+        mp.cfo_host = cfo;
+        mp.pilot_scale = mxGetScalar(A(N_LINK + 7));
+        mp.near_eps = mxGetScalar(A(N_LINK + 8));
+        size_t spp = (size_t)(mp.streams_per_point > 0 ? mp.streams_per_point : 0), cells = n * 2 * spp;
+        int64_t* ch = (int64_t*)hostbuf(n * 24);
+        mxArray* mm = mxCreateDoubleMatrix(spp, 2 * n, mxREAL);     /* reshape(mer, spp, 2, n_points) in MATLAB */
+        if (sweep_group()) chk_group(ofdm_group_sweep_mer(g_group, &lp, &mp, cells ? real_data(mm) : (double*)hostbuf(8), ch), op);
+        else {
+            double* md = (double*)devbuf(cells * 8 + 8);
+            int64_t* cd = (int64_t*)devbuf(n * 24);
+            chk(ofdm_memset(g_ctx, md, 0, cells * 8), "memset");
+            chk(ofdm_memset(g_ctx, cd, 0, n * 24), "memset");
+            chk(ofdm_sweep_mer(g_ctx, &lp, &mp, md, cd), op);
+            chk(ofdm_d2h(g_ctx, real_data(mm), md, cells * 8), "d2h");
+            chk(ofdm_d2h(g_ctx, ch, cd, n * 24), "d2h");
+        }
+        OUT(0, mm);
+        mxArray* cm = mxCreateDoubleMatrix(n, 3, mxREAL);
+        for (i = 0; i < n; ++i) { int j; for (j = 0; j < 3; ++j) real_data(cm)[(size_t)j * n + i] = (double)ch[3 * i + j]; }
         OUT(1, cm);
     } else if (!strcmp(op, "sweep_papr")) {   /* [hist (n_bins x n_points), PAPR (spp x n_points)] =
                                                  sweep_papr(LINK..., scramble, p_one, streams_per_point, seed, bin_db, n_bins, pool, pool_stride):

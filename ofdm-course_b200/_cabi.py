@@ -56,6 +56,14 @@ class PaprParams(C.Structure):
                 ("rank", C.c_int32), ("world", C.c_int32), ("seed", C.c_uint64), ("bin_db", C.c_double), ("n_bins", C.c_int32)]
 
 
+class MerParams(C.Structure):
+    """``ofdm_mer_params`` of include/ofdm_b200.h."""
+    _fields_ = [("n_points", C.c_int32), ("constellation_host", pi32), ("snr_db_host", pdbl), ("pilot_scale", C.c_double),
+                ("nsto_host", pi32), ("cfo_host", pdbl), ("taps_host", pdbl), ("n_taps", C.c_int32),
+                ("streams_per_point", C.c_int64), ("tile_streams", C.c_int64), ("rank", C.c_int32), ("world", C.c_int32),
+                ("seed", C.c_uint64), ("near_eps", C.c_double)]
+
+
 # name -> (restype, argtypes); every symbol declared in include/ofdm_b200.h
 SIGNATURES = {
     "ofdm_ctx_create": (i32, [C.POINTER(vp), i32, i32]),
@@ -123,6 +131,7 @@ SIGNATURES = {
     "ofdm_sweep_part2": (i32, [vp, C.POINTER(LinkParams), C.POINTER(Part2Params), vp, vp, vp]),
     "ofdm_sweep_sync": (i32, [vp, C.POINTER(LinkParams), C.POINTER(SyncParams), vp, vp]),
     "ofdm_sweep_papr": (i32, [vp, C.POINTER(LinkParams), C.POINTER(PaprParams), vp, vp]),
+    "ofdm_sweep_mer": (i32, [vp, C.POINTER(LinkParams), C.POINTER(MerParams), vp, vp]),
     "ofdm_sweep_share": (i32, [i64, i32, i32, C.POINTER(i64), C.POINTER(i64)]),
     "ofdm_payload_bits": (i32, [vp, vp, i64, i64, u64, i64]),
     "ofdm_draw_sto_cfo": (i32, [vp, i64, u64, i64, i32, i32, vp, vp]),
@@ -136,6 +145,7 @@ SIGNATURES = {
     "ofdm_group_sweep_mse": (i32, [vp, C.POINTER(LinkParams), C.POINTER(SweepParams), i32, vp, vp]),
     "ofdm_group_sweep_sync": (i32, [vp, C.POINTER(LinkParams), C.POINTER(SyncParams), vp, vp]),
     "ofdm_group_sweep_papr": (i32, [vp, C.POINTER(LinkParams), C.POINTER(PaprParams), vp, vp]),
+    "ofdm_group_sweep_mer": (i32, [vp, C.POINTER(LinkParams), C.POINTER(MerParams), vp, vp]),
     "ofdm_group_sweep_part2": (i32, [vp, C.POINTER(LinkParams), C.POINTER(Part2Params), vp, vp, vp]),
 }
 

@@ -10,7 +10,7 @@
 // FFT phase and the decision phase, because fine_sync's estimates need all symbols before any of them is corrected.
 #include "fft.cuh"
 #include "interp.cuh"
-#include "fft_reg.cuh"
+#include "rx1024.cuh"
 
 const void* ofdm_upload_pilots(ofdm_ctx* ctx, const double* pv, size_t n_complex);
 uint32_t ofdm_reg_to_prev(const uint8_t* reg);
@@ -248,16 +248,6 @@ __global__ void __launch_bounds__(T4_THREADS) rx_t4_kernel(T4Params p, PlanDev<f
 //     per-sample part exp(-2j*pi*c*i/Nfft) comes from a per-stream shared table;
 //   * 16QAM decisions use the separable rule and the frame's bits are packed eight symbols per word.
 // Estimators (fine_sync) and the channel estimate are the code of the generic kernel above.
-#define T4F_EROW 33
-__device__ __forceinline__ float2 ldg_stream(const float2* p) {   // the sample stream is read once here: keep it out of L1 (tables live there)
-    float2 r;
-    asm("ld.global.nc.L1::no_allocate.v2.f32 {%0, %1}, [%2];" : "=f"(r.x), "=f"(r.y) : "l"(p));
-    return r;
-}
-struct T4FastExtra {
-    const float2* tw_t;        // [k1][n2] = W1024^{n2*k1}: transposed twiddles, coalesced across lanes
-    float two_a;
-};
 
 template <int K2N, bool QAM16, bool NEAR>
 __global__ void __launch_bounds__(T4_THREADS, 2) rx_t4_fast_kernel(T4Params p, T4FastExtra fx, PlanDev<float> plan, DevConst<float> con,
@@ -618,36 +608,6 @@ __global__ void __launch_bounds__(T4_THREADS, 2) rx_t4_fast_kernel(T4Params p, T
 //                    rotation table; writes the N_carrier kept bins and the pilots of every symbol
 //   t4_post_kernel   one CTA per stream, few registers: fine_sync estimators, channel estimate, decisions, DeScrambler, BER
 // The kept bins travel through global memory (N_carrier x S complex per stream) instead of a per-CTA L2 parking area.
-__device__ __forceinline__ void t4_load_window(const float2* __restrict__ r, int64_t L, int SL, int64_t n0, int tg, bool tshift, int lane, float2* v) {
-    constexpr int N = 1024;
-    const int64_t m0 = tshift ? n0 - SL + tg : n0;          // sample n of the corrected stream is r[n - SL + tg] for n >= SL, else 0 (`add_STO.m:5-9`)
-    const bool all_in = (m0 >= 0 && m0 + N <= L && (!tshift || n0 >= SL));
-    if (all_in) {
-        const float2* q = r + m0 + lane;
-#pragma unroll
-        for (int n1 = 0; n1 < 32; ++n1) v[n1] = ldg_stream(q + 32 * n1);
-    } else {
-#pragma unroll
-        for (int n1 = 0; n1 < 32; ++n1) {
-            const int64_t m = m0 + 32 * n1 + lane;
-            const bool ok = m >= 0 && m < L && (!tshift || n0 + 32 * n1 + lane >= SL);
-            v[n1] = ok ? ldg_stream(r + m) : make_float2(0.f, 0.f);
-        }
-    }
-}
-__device__ __forceinline__ void t4_pass_a(float2* v, float2* E, const float2* __restrict__ tw_t, int lane) {   // DFT over n1, twiddle, transpose
-    fft32<32>(v);
-#pragma unroll
-    for (int k1 = 0; k1 < 32; ++k1) {
-        float2 x = v[k1];
-        if (k1) x = cmul(x, __ldg(tw_t + 32 * k1 + lane));
-        E[k1 * T4F_EROW + lane] = x;
-    }
-    __syncwarp();
-#pragma unroll
-    for (int n2 = 0; n2 < 32; ++n2) v[n2] = E[lane * T4F_EROW + n2];
-    __syncwarp();
-}
 
 __global__ void __launch_bounds__(T4_THREADS) t4_ifo_kernel(T4FastExtra fx, const float2* __restrict__ rx, int64_t B, int64_t L, int Tg, int time_desync,
                                                             const int32_t* __restrict__ tg_pos, const double* __restrict__ freq_off,
@@ -742,14 +702,6 @@ struct T4Stats {
     const double* cfo;
     float a_in, a_out;         // 16QAM: |levels| of the inner and outer points per axis
 };
-// 16QAM point nearest to e, per axis (the separable rule of demap16_nib), accumulated as `MER_func.m:7-25` does.  It is the
-// point MER_func's abs() search returns except for exact ties on a decision boundary, where either point is equally near.
-__device__ __forceinline__ void t4_mer16(float2 e, float two_a, float a_in, float a_out, double& s1, double& s2) {
-    const float ix = copysignf(fabsf(e.x) < two_a ? a_in : a_out, e.x), iy = copysignf(fabsf(e.y) < two_a ? a_in : a_out, e.y);
-    const double er = (double)ix - (double)e.x, ei = (double)iy - (double)e.y;
-    s1 += (double)ix * ix + (double)iy * iy;
-    s2 += er * er + ei * ei;
-}
 
 // STATS (ofdm_sweep_sync, NEAR false): the same chain and arithmetic without output bits, tau / phase, H or near-boundary
 // count, and the same CTA also

@@ -254,6 +254,19 @@ extern "C" int ofdm_group_sweep_papr(ofdm_group* g, const ofdm_link_params* lp, 
                      });
 }
 
+extern "C" int ofdm_group_sweep_mer(ofdm_group* g, const ofdm_link_params* lp, const ofdm_mer_params* mp, double* mer_host, int64_t* counts_host) {
+    if (!g) return OFDM_ERR_INVALID;
+    if (!lp || !mp || !mer_host || !counts_host) return group_fail(g, OFDM_ERR_INVALID, "ofdm_group_sweep_mer: bad argument");
+    const int64_t n = dim(mp->n_points), spp = dim(mp->streams_per_point);
+    return group_run(g, n * spp, std::max<int64_t>(spp, 1), {{mer_host, n * 2 * spp, 2}, {counts_host, n * 3, 0}},
+                     [&](ofdm_ctx* ctx, int rank, int world, void* const* dev) {
+                         ofdm_mer_params p = *mp;
+                         p.rank = rank;
+                         p.world = world;
+                         return ofdm_sweep_mer(ctx, lp, &p, (double*)dev[0], (int64_t*)dev[1]);
+                     });
+}
+
 extern "C" int ofdm_group_sweep_part2(ofdm_group* g, const ofdm_link_params* base, const ofdm_part2_params* pp, double* nmse_host,
                                       int64_t* counts_host, int64_t* runs_host) {
     if (!g) return OFDM_ERR_INVALID;

@@ -8,6 +8,10 @@
 
 // The payload of streams g .. g + n - 1 as ofdm_sweep_ber draws it (sweep.cu)
 int ofdm_sweep_tile_payload(ofdm_ctx* ctx, const ofdm_link_params* lp, uint32_t* sbits, uint32_t* bits, int64_t n, int64_t words, uint64_t seed, int64_t g);
+// Per stream of a tile of n: the SNR the channel reads and, when `fixed`, the STO and CFO (sweep_sync.cu)
+void ofdm_sweep_fill(ofdm_ctx* ctx, int64_t n, double snr_db, int fixed, int32_t sto, double cfo, double* snr, int32_t* nsto, double* cfo_out);
+// n streams of stream_bits bits, each the first bits of wpad padded words of `raw`, as one contiguous bitstream (sweep_sync.cu)
+void ofdm_sweep_pack_bits(ofdm_ctx* ctx, const uint32_t* raw, int64_t n, int64_t wpad, int64_t stream_bits, uint32_t* out);
 
 // Rank `rank` of `world` takes the contiguous share [first, first + count) of the n_points x per_point global streams
 // g = point * per_point + j (ofdm_sweep_share).  tile = min(tile_streams > 0 ? tile_streams : tile_default, per_point).

@@ -43,6 +43,16 @@ __global__ void sync_pack_kernel(const uint32_t* __restrict__ in, int64_t wpad, 
     out[W] = v;
 }
 
+void ofdm_sweep_fill(ofdm_ctx* ctx, int64_t n, double snr_db, int fixed, int32_t sto, double cfo, double* snr, int32_t* nsto, double* cfo_out) {
+    sync_fill_kernel<<<(unsigned)cdiv64(n, 256), 256, 0, ctx->stream>>>(n, snr_db, snr, fixed, sto, cfo, nsto, cfo_out);
+    ctx->launches++;
+}
+
+void ofdm_sweep_pack_bits(ofdm_ctx* ctx, const uint32_t* raw, int64_t n, int64_t wpad, int64_t stream_bits, uint32_t* out) {
+    sync_pack_kernel<<<(unsigned)cdiv64(n * wpad, 256), 256, 0, ctx->stream>>>(raw, wpad, stream_bits, n * stream_bits, out);
+    ctx->launches++;
+}
+
 extern "C" int ofdm_sweep_sync(ofdm_ctx* ctx, const ofdm_link_params* lp, const ofdm_sync_params* sp, double* rec_dev, int64_t* counts_dev) {
     if (!ctx) return OFDM_ERR_INVALID;
     REQUIRE(ctx, lp, "ofdm_sweep_sync: link parameters are NULL");
@@ -127,15 +137,11 @@ extern "C" int ofdm_sweep_sync(ofdm_ctx* ctx, const ofdm_link_params* lp, const 
         if (aligned) rc = ofdm_sweep_tile_payload(ctx, lp, sbits, bits, n, words, sp->seed, g);
         else {
             rc = ofdm_payload_bits(ctx, raw, n, words, sp->seed, g);
-            if (rc == OFDM_OK) {
-                sync_pack_kernel<<<(unsigned)cdiv64(n * words, 256), 256, 0, ctx->stream>>>(raw, words, stream_bits, n * stream_bits, sbits);
-                ctx->launches++;
-            }
+            if (rc == OFDM_OK) ofdm_sweep_pack_bits(ctx, raw, n, words, stream_bits, sbits);
             if (rc == OFDM_OK && lp->scramble) rc = ofdm_descramble(ctx, sbits, bits, n * (lp->S / lp->SpF), stream_bits / (lp->S / lp->SpF), lp->reg0_host, nullptr);
         }
         if (rc) return rc;
-        sync_fill_kernel<<<(unsigned)cdiv64(n, 256), 256, 0, ctx->stream>>>(n, sp->snr_db_host[i], snr_d, sp->sto_mode, sp->sto_fixed, sp->cfo_fixed, sto_d, cfo_d);
-        ctx->launches++;
+        ofdm_sweep_fill(ctx, n, sp->snr_db_host[i], sp->sto_mode, sp->sto_fixed, sp->cfo_fixed, snr_d, sto_d, cfo_d);
         // Task 4 order: Noise -> add_STO -> add_CFO -> multipath (`Main_model_Task_4.m:95,103,110,263-264`), one pass
         rc = ofdm_tx_chain_p(ctx, &lp_tx, sbits, n, tx, psum);
         if (rc == OFDM_OK && sp->sto_mode == 0) rc = ofdm_draw_sto_cfo(ctx, n, sp->seed, g, sp->sto_max, sp->cfo_int_max, sto_d, cfo_d);

@@ -16,6 +16,10 @@ which is exact because every cell is written by exactly one rank.
 ``sync_sweep`` is Task 4's own study (``ofdm_sweep_sync`` in csrc/sweep_sync.cu): the synchroniser's estimates, the
 channel-estimate error and the MER of every stream of the Task-4 chain, one record per stream, reduced the same way.
 
+``mer_sweep`` is Task 3's study (``ofdm_sweep_mer`` in csrc/sweep_mer.cu): the BER and MER of the receiver without
+synchroniser or estimator, over points that each have their own constellation and SNR, one all-reduce each of the per-stream
+MER sums and the counters.
+
 ``papr_sweep`` is Task 2's study (``ofdm_sweep_papr`` in csrc/sweep_papr.cu): the PAPR of every transmitted stream and an
 integer histogram of the PAPR of all its Nfft-sample windows, plain against scrambled, one all-reduce each.
 """
@@ -307,6 +311,112 @@ def sync_sweep(ctx, lp, snrs_db, streams_per_point, taps=None, seed=1, rank=0, w
     return reduce_sync(rec, cnt, h_power=channel_power(taps, lp.Nfft, lp.N_carrier), sym_len=lp.Nfft + lp.Tg, cfo_tol=cfo_tol)
 
 
+MER_FIELDS = ("ideal_power", "error_power")
+
+
+def reduce_mer(mer, counts):
+    """Sum the per-stream MER sums (n_points, 2, streams_per_point) float64 -- field 0 the sum of |ideal|^2, field 1 the sum
+    of |ideal - rx|^2 over the stream's data symbols -- and the counters (n_points, 3) int64 {bit errors, bits, near-boundary
+    symbols} over all ranks: one all-reduce each, exact because every MER cell is written by one rank (no-op without an
+    initialised process group).  Returns a dict of NumPy arrays over the points, identical on every rank:
+      ber; mer_db, the pooled MER_func 10 log10(sum f0 / sum f1) with both sums taken in stream order; mer_stream_db, the
+      mean of the finite per-stream MER values in dB (``per_stream_db``); near, the near-boundary symbol count;
+    plus ``mer`` and ``counts`` themselves."""
+    all_reduce_sum(mer, counts)
+    m = mer.cpu().numpy()
+    c = counts.cpu().numpy()
+    pooled = np.cumsum(m, axis=2)[:, :, -1]
+    with np.errstate(divide="ignore", invalid="ignore"):
+        per_db = 10 * np.log10(m[:, 0, :] / m[:, 1, :])
+        mer_db = 10 * np.log10(pooled[:, 0] / pooled[:, 1])
+    fin = np.isfinite(per_db)
+    n_fin = fin.sum(axis=1)
+    mean_db = np.where(n_fin > 0, np.where(fin, per_db, 0.0).sum(axis=1) / np.maximum(n_fin, 1), np.nan)
+    return {"ber": c[:, 0] / np.maximum(c[:, 1], 1), "mer_db": mer_db, "mer_stream_db": mean_db, "near": c[:, 2],
+            "per_stream_db": per_db, "mer": m, "counts": c}
+
+
+def run_mer_sweep(points, streams_per_point, tile, compute, rank=0, world=1):
+    """Generic host driver of the MER study (used with a stand-in ``compute`` in the gloo tests).
+    ``compute(point_index, point, first_stream, n_streams) -> (mer[2, n_streams], counts[3])`` processes one tile on this
+    rank; the result is that of :func:`reduce_mer`."""
+    points = list(points)
+    mer = torch.zeros((len(points), 2, int(streams_per_point)), dtype=torch.float64)
+    counts = torch.zeros((len(points), 3), dtype=torch.int64)
+    for (k, s0, n) in tiles(len(points), streams_per_point, tile, rank, world):
+        m, c = compute(k, points[k], s0, n)
+        mer[k, :, s0:s0 + n] = torch.as_tensor(np.asarray(m, dtype=np.float64))
+        counts[k] += torch.as_tensor(np.asarray(c, dtype=np.int64))
+    return reduce_mer(mer, counts)
+
+
+def _per_point(v, n, dtype):
+    """None, a scalar or n values, as a contiguous array of n (None stays None)."""
+    if v is None:
+        return None
+    a = np.asarray(v, dtype=dtype)
+    return np.ascontiguousarray(np.full(n, a, dtype=dtype) if a.ndim == 0 else a.reshape(n))
+
+
+def mer_params(constellations, snrs_db, streams_per_point, taps=None, seed=1, rank=0, world=1, tile=0, pilot_scale=0.0, sto=None, cfo=None,
+               near_eps=0.0):
+    """The ``ofdm_mer_params`` of :func:`mer_sweep_local`'s arguments (host arrays kept alive on the returned object)."""
+    from .link import CONSTELLATIONS
+    snr = np.ascontiguousarray(np.asarray(snrs_db, dtype=np.float64).ravel())
+    n = snr.size
+    names = [constellations] * n if isinstance(constellations, str) else list(constellations)
+    if len(names) != n:
+        raise ValueError(f"{len(names)} constellations for {n} SNR points")
+    cons = np.ascontiguousarray(np.array([CONSTELLATIONS[str(c)] if str(c) in CONSTELLATIONS else int(c) for c in names], dtype=np.int32))
+    mp = _cabi.MerParams()
+    mp.n_points = n
+    mp.constellation_host = cons.ctypes.data_as(_cabi.pi32)
+    mp.snr_db_host = snr.ctypes.data_as(_cabi.pdbl)
+    mp.pilot_scale = float(pilot_scale)
+    nsto, cf = _per_point(sto, n, np.int32), _per_point(cfo, n, np.float64)
+    if nsto is not None:
+        mp.nsto_host = nsto.ctypes.data_as(_cabi.pi32)
+    if cf is not None:
+        mp.cfo_host = cf.ctypes.data_as(_cabi.pdbl)
+    t = None
+    if taps is not None and len(taps):
+        t = np.ascontiguousarray(np.asarray(taps, dtype=np.float64).reshape(-1, 2))
+        mp.taps_host = t.ctypes.data_as(_cabi.pdbl)
+        mp.n_taps = t.shape[0]
+    mp.streams_per_point = int(streams_per_point)
+    mp.tile_streams = int(tile)
+    mp.rank, mp.world = int(rank), int(world)
+    mp.seed = int(seed)
+    mp.near_eps = float(near_eps)
+    mp._keep = (snr, cons, nsto, cf, t)
+    return mp
+
+
+def mer_sweep_local(ctx, lp, constellations, snrs_db, streams_per_point, taps=None, seed=1, rank=0, world=1, tile=0, pilot_scale=0.0, sto=None,
+                    cfo=None, near_eps=0.0, mer=None, counts=None):
+    """This rank's share of the Task-3 study through ``ofdm_sweep_mer``, WITHOUT synchronising.  Point k is
+    (``constellations[k]``, ``snrs_db[k]``; a single name applies to every point), with the fixed STO / CFO ``sto`` / ``cfo``
+    (None, one value, or one per point; not corrected by the receiver).  ``pilot_scale`` > 0 makes every pilot of point k the
+    real value pilot_scale * max|constellation| (Task 3's scalar pilots); 0 keeps ``lp``'s pilots.  Writes its cells of ``mer``
+    (n_points, 2, streams_per_point) float64, fields :data:`MER_FIELDS`, and adds to ``counts`` (n_points, 3) int64 {bit errors,
+    bits, near-boundary symbols}; both are zero-initialised device tensors when not given."""
+    mp = mer_params(constellations, snrs_db, streams_per_point, taps, seed, rank, world, tile, pilot_scale, sto, cfo, near_eps)
+    if mer is None:
+        mer = torch.zeros((mp.n_points, 2, int(streams_per_point)), dtype=torch.float64, device=ctx.device)
+    if counts is None:
+        counts = torch.zeros((mp.n_points, 3), dtype=torch.int64, device=ctx.device)
+    ctx._chk(ctx.lib.ofdm_sweep_mer(ctx.h, C.byref(lp), C.byref(mp), ctx.p(mer), ctx.p(counts)))
+    return mer, counts
+
+
+def mer_sweep(ctx, lp, constellations, snrs_db, streams_per_point, taps=None, seed=1, rank=0, world=1, tile=0, **kw):
+    """Whole Task-3 study: this rank's call, then :func:`reduce_mer` (one all-reduce each of the per-stream MER sums and the
+    counters); identical on every rank and for every world size and tile."""
+    mer, cnt = mer_sweep_local(ctx, lp, constellations, snrs_db, streams_per_point, taps, seed, rank, world, tile, **kw)
+    ctx.sync()
+    return reduce_mer(mer, cnt)
+
+
 def papr_params(points, streams_per_point, seed=1, rank=0, world=1, tile=0, bin_db=0.01, n_bins=4000, pool=None, pool_stride=0):
     """The ``ofdm_papr_params`` of :func:`papr_sweep_local`'s arguments (host arrays kept alive on the returned object)."""
     pts = [(int(bool(s)), p) for s, p in points]
@@ -474,6 +584,14 @@ class Group:
         papr = np.zeros((pp.n_points, int(streams_per_point)), dtype=np.float64)
         self._chk(self.lib.ofdm_group_sweep_papr(self.h, C.byref(lp), C.byref(pp), papr.ctypes.data, hist.ctypes.data))
         return hist, papr
+
+    def sweep_mer(self, lp, constellations, snrs_db, streams_per_point, taps=None, seed=1, tile=0, **kw):
+        """(mer (n_points, 2, streams_per_point) float64, counts (n_points, 3) int64) of :func:`mer_sweep_local`."""
+        mp = mer_params(constellations, snrs_db, streams_per_point, taps, seed, 0, 1, tile, **kw)
+        mer = np.zeros((mp.n_points, 2, int(streams_per_point)), dtype=np.float64)
+        counts = np.zeros((mp.n_points, 3), dtype=np.int64)
+        self._chk(self.lib.ofdm_group_sweep_mer(self.h, C.byref(lp), C.byref(mp), mer.ctypes.data, counts.ctypes.data))
+        return mer, counts
 
     def sweep_part2(self, combs, mc_runs, payload_bits, *, tile=0, **kw):
         """(per_run (n_points, 4, mc_runs) float64, counts (n_points, 4, 3) int64, runs (n_points, 2) int64) of
