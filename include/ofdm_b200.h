@@ -299,7 +299,8 @@ OFDM_API int ofdm_rx_chain_t5_host_eps(ofdm_ctx*, const ofdm_link_params*, const
  * (`Task 4/Main_model_Task_4.m:277-366`), one pass for the autocorrelation plus one persistent kernel.
  * rx_dev B x S x (Nfft+Tg).  Optional outputs: out_bits_dev, counts_dev {errors, bits, near} += , and the
  * per-stream estimates tg_dev (int32), fo_dev (double), ifo_dev (int32, -1 = no bin above 0.77), tau_dev,
- * phase_dev (double), H_dev (B x N_carrier). */
+ * phase_dev (double), H_dev (B x N_carrier).  A data carrier past N_carrier is decided from 0 (equalize_signal.m zeroes it);
+ * with mp_desync = 0 such a layout returns OFDM_ERR_UNSUPPORTED, since the chain keeps only the N_carrier first bins. */
 OFDM_API int ofdm_rx_chain_t4(ofdm_ctx*, const ofdm_link_params*, const void* rx_dev, int64_t B, int time_desync,
                               int freq_desync, int mp_desync, const uint32_t* tx_bits_dev, uint32_t* out_bits_dev,
                               int64_t* counts_dev, int32_t* tg_dev, double* fo_dev, int32_t* ifo_dev, double* tau_dev,
@@ -468,8 +469,9 @@ OFDM_API int ofdm_sweep_papr(ofdm_ctx*, const ofdm_link_params*, const ofdm_papr
  * transmitter maps s without scrambling.  The channel is ofdm_channel_t4_p with the point's SNR, STO and CFO, so a call whose
  * points share one constellation transmits, with equal pilot values, the streams ofdm_sweep_sync transmits for the same SNR
  * list, seed and taps with sto_mode 1.  The receiver decides every symbol in the pass that transforms it: its bins and
- * decisions are those of ofdm_rx_chain_t4_ex(..., 0, 0, 0, ...).  FP32 contexts and Nfft = 1024 only (OFDM_ERR_UNSUPPORTED
- * otherwise); streams need not be word aligned.
+ * decisions are those of ofdm_rx_chain_t4_ex(..., 0, 0, 0, ...) when that call runs its split chain (>= 512 streams of a
+ * shape whose fused kernel fits; its other kernels round differently).  FP32 contexts and Nfft = 1024 only, data carriers
+ * within N_carrier (OFDM_ERR_UNSUPPORTED otherwise); streams need not be word aligned.
  * mer_dev: n_points x 2 x streams_per_point doubles, [k][f][j]: f = 0 the sum of |ideal|^2, f = 1 the sum of |ideal - rx|^2
  * over the stream's data symbols, so MER_func of the stream is 10 log10(f0 / f1) dB; only this call's share is written, and
  * each cell is summed in an order that depends on the stream shape only.

@@ -1164,6 +1164,10 @@ static int t4_setup(ofdm_ctx* ctx, const char* fn, const ofdm_link_params* lp, i
     std::vector<int32_t> d0(lp->Nd), p0(lp->Np);
     for (int i = 0; i < lp->Nd; ++i) {
         if (lp->data_carriers_host[i] < 1 || lp->data_carriers_host[i] > lp->Nfft) return ctx_fail(ctx, OFDM_ERR_INVALID, "%s: data carrier out of range", fn);
+        // The kernels keep the N_carrier first bins only.  With the equaliser a data carrier past N_carrier is 0 in the reference
+        // too (`equalize_signal.m:6`); without it the reference decides the carrier from its demodulated bin.
+        if (!mp_desync && lp->data_carriers_host[i] > lp->N_carrier)
+            return ctx_fail(ctx, OFDM_ERR_UNSUPPORTED, "%s: a data carrier past N_carrier needs mp_desync (the chain keeps N_carrier bins)", fn);
         d0[i] = lp->data_carriers_host[i] - 1;
     }
     for (int i = 0; i < lp->Np; ++i) {

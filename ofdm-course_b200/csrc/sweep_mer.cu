@@ -10,7 +10,8 @@
 //   * one CTA per stream, one warp per OFDM symbol (warp w takes symbols w, w + 8, ...): the 1024 samples after the cyclic
 //     prefix (the prefix is never read), the split Task-4 chain's 1024-point transform (t4_load_window / t4_pass_a / fft32
 //     of rx1024.cuh, as t4_sym_kernel runs it with every desync flag off), so bins and decisions are bit-identical to
-//     ofdm_rx_chain_t4_ex(..., 0, 0, 0, ...);
+//     those of ofdm_rx_chain_t4_ex(..., 0, 0, 0, ...) when that call takes its split chain (from 512 streams on, for shapes
+//     whose fused kernel fits in 111 KB of shared memory; its fused and generic kernels round differently);
 //   * the data carriers of the symbol are decided by its warp (16QAM: the separable rule of demap16_nib; BPSK / QPSK / 8PSK:
 //     the first-minimum table rule of nearest_idx), with the near-boundary count of ofdm_demap and the two MER_func sums
 //     `MER_func.m:7-25` in double;
@@ -160,6 +161,9 @@ extern "C" int ofdm_sweep_mer(ofdm_ctx* ctx, const ofdm_link_params* lp, const o
     std::vector<int32_t> d0(lp->Nd);
     for (int i = 0; i < lp->Nd; ++i) {
         if (lp->data_carriers_host[i] < 1 || lp->data_carriers_host[i] > Nfft) return ctx_fail(ctx, OFDM_ERR_INVALID, "ofdm_sweep_mer: data carrier out of range");
+        // the receiver keeps the N_carrier first bins; Task 3 has no equaliser and decides a carrier past N_carrier from its bin
+        if (lp->data_carriers_host[i] > lp->N_carrier)
+            return ctx_fail(ctx, OFDM_ERR_UNSUPPORTED, "ofdm_sweep_mer: a data carrier past N_carrier needs its bin, which the receiver does not keep");
         d0[i] = lp->data_carriers_host[i] - 1;
     }
     const int64_t sym_bits_max = (int64_t)lp->S * lp->Nd * bps_max;

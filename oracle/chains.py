@@ -152,10 +152,13 @@ def impair_task4(p: LinkParams, tx, SNR_dB=None, Time_Delay=None, Freq_Shift=Non
     return rx
 
 
-def rx_chain_task4(p: LinkParams, rx_stream, input_bits, time_desync=True, freq_desync=True, mp_desync=True):
+def rx_chain_task4(p: LinkParams, rx_stream, input_bits, time_desync=True, freq_desync=True, mp_desync=True, descramble=True,
+                   ifo_passthrough=False):
     """M2 chain (`Task 4/Main_model_Task_4.m:277-366`): AutoCorrFunction -> add_STO x2 -> add_CFO ->
     remove_IFO -> reshape -> OFDM_demodulator -> fine_sync -> estimate_channel -> equalize_signal ->
-    get_payload -> demapping -> DeScrambler -> BER."""
+    get_payload -> demapping -> DeScrambler -> BER.  remove_IFO raises like MATLAB when no spectrum bin
+    exceeds 0.77; with ``ifo_passthrough`` the stream passes unchanged with IFO = -1 instead, as the
+    device library does (`ofdm_remove_ifo`).  ``raw_bits`` are the decisions before DeScrambler."""
     rx = np.asarray(rx_stream).ravel()
     info = {}
     if time_desync or freq_desync:
@@ -166,7 +169,12 @@ def rx_chain_task4(p: LinkParams, rx_stream, input_bits, time_desync=True, freq_
             rx = F.add_STO(rx, -(p.Nfft + p.T_Guard))
     if freq_desync:
         rx = F.add_CFO(rx, -fo, p.Nfft)
-        rx, ifo = F.remove_IFO(rx, p.Nfft)
+        try:
+            rx, ifo = F.remove_IFO(rx, p.Nfft)
+        except IndexError:
+            if not ifo_passthrough:
+                raise
+            ifo = -1
         info.update(IFO=ifo)
     X = rx.reshape((p.Nfft + p.T_Guard, p.N_symb), order="F")
     Y = F.OFDM_demodulator(X, p.T_Guard)
@@ -179,9 +187,9 @@ def rx_chain_task4(p: LinkParams, rx_stream, input_bits, time_desync=True, freq_
         Y = F.equalize_signal(Y, H, p.N_carrier)
     rx_iq = F.get_payload(Y, p.dataCarriers).ravel(order="F")
     out_bits = F.demapping(-1, rx_iq, p.Constellation)
-    dsc = scramble_frames(p, out_bits, descramble=True)
+    dsc = scramble_frames(p, out_bits, descramble=True) if descramble else out_bits
     tx_bits = np.asarray(input_bits).ravel()
-    info.update(Y=Y, rx_iq=rx_iq, bits=dsc, errors=int(np.sum(tx_bits != dsc)), n_bits=tx_bits.size)
+    info.update(Y=Y, rx_iq=rx_iq, bits=dsc, raw_bits=out_bits, errors=int(np.sum(tx_bits != dsc)), n_bits=tx_bits.size)
     return info
 
 

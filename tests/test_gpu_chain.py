@@ -436,9 +436,12 @@ def test_rx_chain_task4_fused_matches_oracle_and_composed(G):
 @pytest.mark.parametrize("ncar,con,near_eps", [(800, "16QAM", 1e-3), (400, "8PSK", 1e-3), (400, "QPSK", 0.0), (416, "16QAM", 0.0)])
 def test_rx_chain_task4_fast_kernel_variants(G, monkeypatch, ncar, con, near_eps):
     """Template variants of the warp-per-symbol Task-4 kernel (unpruned second DFT for N_carrier > 416, generic
-    constellations, near-boundary counting off) against the oracle and against the generic block-FFT kernel."""
+    constellations, near-boundary counting off) against the oracle and against the generic block-FFT kernel.  At N_carrier
+    800 the stream has 5 frames: 10 need more shared memory than the fused kernel may take, and the generic one would run."""
+    from kernel_witness import witness
     TAPS4 = [[0, 1], [4, .6], [10, .3]]
-    p = OC.LinkParams(Nfft=1024, N_carrier=ncar, T_Guard=128, Amount_OFDM_Frames=10, Amount_ODFM_SpF=5, Constellation=con)
+    frames = 5 if ncar > 416 else 10
+    p = OC.LinkParams(Nfft=1024, N_carrier=ncar, T_Guard=128, Amount_OFDM_Frames=frames, Amount_ODFM_SpF=5, Constellation=con)
     p.pilotCarriers, p.dataCarriers = O.pilot_layout_percent(ncar, 15, 1024, last_gap=2)
     p.pilotValues, _ = OC.make_pilot_values(len(p.pilotCarriers), p.N_symb, con, 4.0 / 3.0, True)
     ctx = G.default_context("f32")
@@ -455,11 +458,14 @@ def test_rx_chain_task4_fast_kernel_variants(G, monkeypatch, ncar, con, near_eps
         refs.append(OC.rx_chain_task4(p, rx, bits[b]))
     rx_d = ctx.cplx(np.stack(rxs))
     bd = ctx.bits(bits.ravel())
-    fast = ctx.rx_chain_t4_fused(lp, rx_d, tx_bits_dev=bd, near_eps=near_eps, want_H=True)
+    fast, kf = witness(lambda: ctx.rx_chain_t4_fused(lp, rx_d, tx_bits_dev=bd, near_eps=near_eps, want_H=True))
     got = ctx.host_bits(fast["bits"], B * p.stream_bits).reshape(B, -1)
     monkeypatch.setenv("OFDM_B200_NO_FAST", "1")
-    slow = ctx.rx_chain_t4_fused(lp, rx_d, tx_bits_dev=bd, near_eps=1e-3, want_H=True)
+    slow, ks = witness(lambda: ctx.rx_chain_t4_fused(lp, rx_d, tx_bits_dev=bd, near_eps=1e-3, want_H=True))
     monkeypatch.delenv("OFDM_B200_NO_FAST")
+    if kf is not None:             # None: no CUPTI, kernel identities are not observable
+        rx = [k for k in kf + ks if k[0] in ("rx_t4_fast_kernel", "rx_t4_kernel")]
+        assert rx == [("rx_t4_fast_kernel", (32 if ncar > 416 else 13, con == "16QAM", near_eps > 0)), ("rx_t4_kernel", ())], rx
     got_s = ctx.host_bits(slow["bits"], B * p.stream_bits).reshape(B, -1)
     near = max(int(slow["counts"].cpu().numpy()[2]), 1)
     checked = 0

@@ -6,13 +6,13 @@ outputs, per-symbol pilot columns and scrambler registers whose cells 13 and 14 
 Which kernel ran is read from the CUDA activity of `torch.profiler` (one launch of `rx4096_kernel` and one of `rx_chain_kernel`
 look alike to a launch counter); a box without CUPTI skips those asserts and still runs the parity ones."""
 import ctypes as C
-import re
 
 import numpy as np
 import pytest
 
 import oracle as O
 from oracle import chains as OC
+from kernel_witness import Registry, t4_phase_bounds as _t4_phase_bounds, witness as _witness
 
 pytestmark = pytest.mark.gpu
 TAPS5 = [[0, 1], [4, .8], [10, .6], [15, .4], [21, .2], [25, .1]]
@@ -78,90 +78,8 @@ def _streams(p, B, seed, scramble=True):
     return bits, rx
 
 
-def _t4_phase_bounds(p, rx, ref):
-    """Interval of fine_sync's phase_shift (`fine_sync.m:47-52`, the mean of the pilot angles above 1e-3) over the signs of exact
-    zeros.  The pilots of a symbol that add_STO zero-filled give tx * conj(rx) = +-0 +-0j, whose angle is 0, +pi or -pi depending
-    only on the signs of the zeros (the order of the arithmetic, not its accuracy): such a pilot is left out of the mean or
-    counted at +pi or -pi, and each one moves the mean by about pi / n.  Returns (lo, hi) over every choice; the oracle's own value
-    is one of them."""
-    x = np.asarray(rx, dtype=np.complex128).ravel()
-    # the oracle's receiver up to fine_sync (OC.rx_chain_task4), with its own integer and frequency estimates
-    x = O.add_STO(O.add_STO(x, ref["TgPosition"]), -(p.Nfft + p.T_Guard))
-    x, _ = O.remove_IFO(O.add_CFO(x, -ref["FreqOffset"], p.Nfft), p.Nfft)
-    Y = O.OFDM_demodulator(x.reshape((p.Nfft + p.T_Guard, p.N_symb), order="F"), p.T_Guard)
-    pc = np.asarray(p.pilotCarriers)
-    rxp = Y[pc - 1, :] * np.exp(2j * np.pi * ref["tau"] * (pc - 1))[:, None]        # time_desync correction (`fine_sync.m:39-42`)
-    prod = p.pilotValues.ravel(order="F") * np.conj(rxp.ravel(order="F"))
-    zero = prod == 0
-    a = np.angle(prod[~zero])
-    a = a[np.abs(a) > 1e-3]
-    z = int(zero.sum())
-    means = [(a.sum() + np.pi * (kp - km)) / (a.size + kp + km) for kp in range(z + 1) for km in range(z + 1 - kp)]
-    return min(means), max(means)
-
-
 # ------------------------------------------------------------------------------------------------------------- kernel witness
-_SEEN = {}                       # (kernel, template arguments) -> ids of the cases that launched it
-_WITNESS = {"available": None}   # False once a profiled call recorded no CUDA activity at all
-_RAN = set()                     # RX matrix cases that ran in this session
-
-
-def _targ(x):
-    x = re.sub(r"^\((?:unsigned\s+)?(?:int|long|short|char|bool)\)\s*", "", x.strip())
-    if x in ("true", "false"):
-        return x == "true"
-    m = re.fullmatch(r"(-?(?:0x[0-9a-fA-F]+|\d+))[uUlL]*", x)
-    return int(m.group(1), 0) if m else x
-
-
-def parse_kernel(name):
-    """'void rx4096_kernel<true, false, (int)257, true>(Fast4096Params, ...)' -> ('rx4096_kernel', (True, False, 257, True));
-    None for activity that is not a kernel (memsets, copies)."""
-    s = name.strip()
-    if s.startswith("void "):
-        s = s[5:]
-    m = re.match(r"[A-Za-z_][\w:]*", s)
-    if not m:
-        return None
-    ident, i, args = m.group(0).split("::")[-1], m.end(), ()
-    if i < len(s) and s[i] == "<":
-        depth, parts, cur = 0, [], ""
-        for j in range(i, len(s)):
-            ch = s[j]
-            if ch in "<(":
-                depth += 1
-                if depth == 1 and ch == "<":
-                    continue
-            elif ch in ">)":
-                depth -= 1
-                if depth == 0:
-                    break
-            if ch == "," and depth == 1:
-                parts.append(cur)
-                cur = ""
-            else:
-                cur += ch
-        parts.append(cur)
-        args, i = tuple(_targ(x) for x in parts), j + 1
-    if i >= len(s) or s[i] != "(":
-        return None
-    return ident, args
-
-
-def _witness(fn):
-    """Run fn() under torch.profiler (CUDA activity only); returns (fn's result, parsed kernels in launch order) -- kernels is
-    None when the profiler recorded no CUDA activity (no CUPTI on this box)."""
-    import torch
-    from torch.autograd import DeviceType
-    from torch.profiler import ProfilerActivity, profile
-    torch.cuda.synchronize()
-    with profile(activities=[ProfilerActivity.CUDA]) as prof:
-        out = fn()
-        torch.cuda.synchronize()
-    names = [e.name for e in prof.events() if e.device_type == DeviceType.CUDA]
-    if not names:
-        return out, None
-    return out, [k for k in map(parse_kernel, names) if k is not None]
+_W = Registry()                  # kernels seen, RX matrix cases that ran
 
 
 CHAIN_KERNELS = ("rx4096_kernel", "rx_chain_kernel", "tx4096_kernel", "tx_chain_kernel", "tx1024_kernel")
@@ -169,13 +87,8 @@ CHAIN_KERNELS = ("rx4096_kernel", "rx_chain_kernel", "tx4096_kernel", "tx_chain_
 
 def _expect(kernels, want, case):
     """The chain kernel that ran must be exactly `want` (one launch); records what was seen for the coverage test."""
-    if kernels is None:
-        _WITNESS["available"] = False
+    if not _W.record(kernels, case):
         return
-    if _WITNESS["available"] is None:
-        _WITNESS["available"] = True
-    for k in kernels:
-        _SEEN.setdefault(k, set()).add(case)
     chain = [k for k in kernels if k[0] in CHAIN_KERNELS]
     assert chain == [want], f"{case}: expected {want}, the profiler saw {kernels}"
 
@@ -293,7 +206,7 @@ def test_rx_matrix_against_oracle(G, monkeypatch, case):
     res, kernels = _witness(lambda: ctx.rx_chain_t5(lp, rx_d, B, tx_bits_dev=tx_d, near_eps=near_eps, want_err_per_stream=True))
     _expect(kernels, want, case)
     _check_rx(ctx, p, res, refs, bits, near_eps, scramble)
-    _RAN.add(case)
+    _W.ran.add(case)
 
 
 # ------------------------------------------------------------------------------------------------------------- batch geometry
@@ -569,15 +482,15 @@ def test_per_symbol_pilots_rx_t4(G, monkeypatch, path):
 def test_witness_covered_every_instantiation():
     """The cases above together launched all 14 rx4096_kernel instantiations, tx4096_kernel, and the generic receiver for each
     fallback (odd guard, misaligned rx, N_carrier > 1024, shared memory over the limit)."""
-    if _WITNESS["available"] is False:
+    if _W.available is False:
         pytest.skip("the profiler recorded no CUDA activity (no CUPTI): kernel identities are not observable here")
-    if _WITNESS["available"] is None or set(RX_CASES) - _RAN:
+    if _W.available is None or set(RX_CASES) - _W.ran:
         pytest.skip("kernel coverage needs every RX case of this module in the same session")
     want = {K(True, n, m, s) for n in (False, True) for m in (0x1111, 0x0101, 0) for s in (False, True)}
     want |= {K(False, n, 0, False) for n in (False, True)}
-    seen = {k for k in _SEEN if k[0] == "rx4096_kernel"}
+    seen = {k for k in _W.seen if k[0] == "rx4096_kernel"}
     print("rx4096_kernel instantiations observed:", sorted(k[1] for k in seen))
-    print("generic receiver observed for:", sorted(_SEEN.get(GEN_RX, ())))
+    print("generic receiver observed for:", sorted(_W.seen.get(GEN_RX, ())))
     assert len(want) == 14 and want <= seen, sorted(want - seen)
-    assert TX4096 in _SEEN
-    assert set(FALLBACKS) <= _SEEN.get(GEN_RX, set())
+    assert TX4096 in _W.seen
+    assert set(FALLBACKS) <= _W.seen.get(GEN_RX, set())
